@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the population-generation hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload: BASELINE.json configs[1] (README 8-core scenario): 10 000 cases + 10 000 controls, -f 0.01,
@@ -19,6 +19,7 @@ Extra keys of the N = 1 line: value_sustained (>= 1 s of back-to-back device-onl
 value, e2e on the C5 sample shape), cli_to_file (the drop-in CLI writing population.vcf.gz), allele_chi_square
 (dna_factory_b200/allele_stats.py), cpu_baseline (the UNMODIFIED reference CLI from oracle/_ref, `-n <cores-1>`),
 cpu_baseline_c1_full (BASELINE config 1 in full) and cpu_baseline_port (the C port).  N > 1: multi_gpu_parity.
+--dump-outputs DIR: rank 0 writes what the last timed step of `value` and of `e2e` returned to DIR/*.npy (dump_outputs).
 """
 import argparse
 import json
@@ -170,6 +171,51 @@ def _inflate_bgzf(blob):
     return allele_stats.inflate_bgzf(blob)
 
 
+DUMP_STATS = ("rows", "calls", "text_bytes", "bgzf_bytes", "bgzf_blocks", "crc_xor")
+DUMP_SEED = 20260101
+DUMP_WINDOW = 1 << 16
+
+
+def _sample_windows(n_bytes, n, rng):
+    """Sorted offsets of n windows of min(DUMP_WINDOW, n_bytes) bytes inside n_bytes bytes, and that width."""
+    width = min(DUMP_WINDOW, n_bytes)
+    return np.sort(rng.integers(0, n_bytes - width + 1, n)), width
+
+
+def dump_outputs(out_dir, value_stats, e2e_stats, blob):
+    """What the last timed step handed its caller, as .npy files for comparing two builds output for output (~50 MB).
+
+    value_stats / e2e_stats   float64[6]: rows, calls, text_bytes, bgzf_bytes, bgzf_blocks, crc_xor of the last step
+                              of the `value` pass (dnaf_generate_device returns nothing else) and of the `e2e` pass
+    e2e_bgzf_blocks           float32[blocks, 2]: compressed and text size of every BGZF block of the e2e step's stream
+    e2e_bgzf, e2e_text        float32[windows, 64 KiB]: bytes of that stream and of its decompressed VCF text in
+                              windows at seeded offsets (e2e_bgzf_offsets, e2e_text_offsets: float64)
+    The text is inflated only around the windows; every block inflated is checked against its CRC32 and ISIZE.
+    """
+    from dna_factory_b200 import _native, allele_stats
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(DUMP_SEED)
+    csize, usize = _native.bgzf_scan(blob)
+    coff = np.concatenate(([0], np.cumsum(csize, dtype=np.int64)))
+    uoff = np.concatenate(([0], np.cumsum(usize, dtype=np.int64)))
+    b_off, b_w = _sample_windows(len(blob), 64, rng)
+    t_off, t_w = _sample_windows(int(uoff[-1]), 128, rng)
+    text = []
+    for o in t_off:
+        b0, b1 = np.searchsorted(uoff, o, "right") - 1, np.searchsorted(uoff, o + t_w, "left")
+        t = allele_stats.inflate_bgzf(blob[coff[b0]:coff[max(b0 + 1, b1)]])
+        text.append(np.frombuffer(t, np.uint8)[o - uoff[b0]:o - uoff[b0] + t_w])
+    arrays = {"value_stats": np.array([value_stats[k] for k in DUMP_STATS], np.float64),
+              "e2e_stats": np.array([e2e_stats[k] for k in DUMP_STATS], np.float64),
+              "e2e_bgzf_blocks": np.stack([csize, usize], axis=1).astype(np.float32),
+              "e2e_bgzf_offsets": b_off.astype(np.float64),
+              "e2e_bgzf": np.stack([blob[o:o + b_w] for o in b_off]).astype(np.float32),
+              "e2e_text_offsets": t_off.astype(np.float64),
+              "e2e_text": np.stack(text).astype(np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _lap(what, t0=[time.perf_counter()]):
     """Phase timing on stderr (the JSON line on stdout stays alone)."""
     now = time.perf_counter()
@@ -298,7 +344,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip level_sweep / value_sustained / cli_to_file / chi-square")
     ap.add_argument("--level", type=int, default=LEVEL, help="-z of the timed steps (default: the workload's 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     # debugging aid: DNAF_BENCH_ONE_GPU=1 runs all ranks of a torchrun launch on GPU 0 over gloo, so that the N > 1
@@ -501,6 +550,8 @@ def main():
     torch.cuda.synchronize()
     e2e_s = max_over_ranks(time.perf_counter() - t0)
     barrier()
+    # the last step's stream, taken before the -z runs below reuse the output buffers
+    last_blob = outs[(args.steps - 1) % n_ctx][:e2e_stats[-1]["bgzf_bytes"]].copy() if args.dump_outputs else None
     e2e_calls = sum_over_ranks(sum(s["calls"] for s in e2e_stats))
     h2d = int(np.mean([sum(v.nbytes for v in b[0].values()) + b[1].nbytes + b[2].nbytes for b in
                        batches[warmup:]]))
@@ -614,6 +665,8 @@ def main():
         if multi_gpu_parity is not None:
             line["multi_gpu_parity"] = multi_gpu_parity
         line.update(extras)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, stats[-1], e2e_stats[-1], last_blob)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -25,13 +25,17 @@ def test_library_loads_and_exports_every_declared_symbol():
 
 
 def test_missing_gpu_fails_loudly():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    from dna_factory_b200 import _native
-    with pytest.raises(_native.DnafError) as e:
-        _native.Engine(0)
-    assert "no CPU fallback" in str(e.value)
+    """No visible CUDA device: creating a context raises.  The devices are hidden from a child process, so that the
+    check runs on a machine with a GPU as well."""
+    import subprocess
+    import sys
+    code = ("from dna_factory_b200 import _native\n"
+            "try:\n    _native.Engine(0)\nexcept _native.DnafError as e:\n    print(e)\n"
+            "else:\n    raise SystemExit('a context was created without a visible device')\n")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True,
+                       cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0 and "no CPU fallback" in r.stdout, r.stdout + r.stderr
 
 
 def test_arg_parser_matches_reference_surface():
@@ -348,6 +352,36 @@ def test_bench_population_windows_do_not_depend_on_what_follows():
     r1, s1 = host.slice_overrides(one[3], one[4], 0, 64)
     r3, s3 = host.slice_overrides(three[3], three[4], 0, 64)
     assert np.array_equal(r1, r3) and np.array_equal(s1, s3) and len(r1) >= 2
+
+
+def test_bench_dump_outputs_hold_the_stream_and_its_text(tmp_path):
+    """bench.py --dump-outputs: float .npy files of at most 64 MB in all; the sampled windows are the bytes of the BGZF
+    stream and of its text at the stored offsets, the block table covers the text, and the same stream gives the same
+    files."""
+    import bench
+    from dna_factory_b200 import _native
+    from oracle import oracle
+    from tests.cases import synth_case
+    case = synth_case(2000, 300, seed=4)
+    text, _ = oracle.rows(case.samples, case.snps, case.seed, n_threads=4)
+    blob = np.frombuffer(oracle.bgzf(text, level=2, with_eof=False), np.uint8)
+    assert len(blob) > 2 * bench.DUMP_WINDOW
+    st = {"rows": 300, "calls": 600000, "text_bytes": len(text), "bgzf_bytes": len(blob),
+          "bgzf_blocks": len(_native.bgzf_scan(blob)[0]), "crc_xor": 0xDEADBEEF, "ms_total": 1.5}
+    bench.dump_outputs(str(tmp_path / "a"), st, st, blob)
+    got = {p.stem: np.load(p) for p in (tmp_path / "a").glob("*.npy")}
+    assert {a.dtype for a in got.values()} <= {np.dtype(np.float32), np.dtype(np.float64)}
+    assert sum(a.nbytes for a in got.values()) <= 64 << 20
+    assert list(got["e2e_stats"]) == [300, 600000, len(text), len(blob), st["bgzf_blocks"], 0xDEADBEEF]
+    assert got["e2e_bgzf_blocks"].shape == (st["bgzf_blocks"], 2) and got["e2e_bgzf_blocks"][:, 1].sum() == len(text)
+    assert got["e2e_text"].shape == (128, bench.DUMP_WINDOW) and got["e2e_bgzf"].shape == (64, bench.DUMP_WINDOW)
+    for o, w in zip(got["e2e_text_offsets"].astype(np.int64), got["e2e_text"]):
+        assert w.astype(np.uint8).tobytes() == text[o:o + bench.DUMP_WINDOW]
+    for o, w in zip(got["e2e_bgzf_offsets"].astype(np.int64), got["e2e_bgzf"]):
+        assert w.astype(np.uint8).tobytes() == blob[o:o + bench.DUMP_WINDOW].tobytes()
+    bench.dump_outputs(str(tmp_path / "b"), st, st, blob.copy())
+    for name, a in got.items():
+        assert np.array_equal(np.load(tmp_path / "b" / (name + ".npy")), a), name
 
 
 def test_header_is_plain_c_and_links(tmp_path):
