@@ -41,7 +41,8 @@ EXPORTS = ["dnaf_abi_version", "dnaf_device_count", "dnaf_last_error", "dnaf_cre
            "dnaf_plan", "dnaf_row_offsets", "dnaf_generate", "dnaf_generate_stream", "dnaf_generate_fd", "dnaf_generate_fd_at", "dnaf_generate_device", "dnaf_genotypes",
            "dnaf_text", "dnaf_bgzf_compress", "dnaf_bgzf_bound", "dnaf_bgzf_eof", "dnaf_bgzf_scan", "dnaf_block_log",
            "dnaf_block_log_get", "dnaf_select_snps", "dnaf_parse_snps_jsonl", "dnaf_format_prefixes",
-           "dnaf_format_snps_jsonl", "dnaf_debug_lz_block"]
+           "dnaf_format_snps_jsonl", "dnaf_debug_lz_block", "dnaf_generate_bed", "dnaf_generate_bed_fd_at",
+           "dnaf_generate_bed_device"]
 
 _lib = None
 
@@ -80,6 +81,9 @@ def load():
         "dnaf_generate_fd": (i32, [vp, u64, u64, u64, i32, i32, sp]),
         "dnaf_generate_fd_at": (i32, [vp, u64, u64, u64, i32, i32, u64, sp]),
         "dnaf_generate_device": (i32, [vp, u64, u64, u64, i32, sp]),
+        "dnaf_generate_bed": (i32, [vp, u64, u64, u64, u8p, u64, sp]),
+        "dnaf_generate_bed_fd_at": (i32, [vp, u64, u64, u64, i32, u64, sp]),
+        "dnaf_generate_bed_device": (i32, [vp, u64, u64, u64, sp]),
         "dnaf_genotypes": (i32, [vp, u64, u64, u64, u8p, u64]),
         "dnaf_text": (i32, [vp, u64, u64, u64, u8p, u64, u64p]),
         "dnaf_bgzf_compress": (i32, [vp, u8p, u64, u8p, u64, sp]),
@@ -290,6 +294,36 @@ class Engine:
         st = Stats()
         self._check(self._lib.dnaf_generate_device(self._h, row_begin, row_end, seed, level,
                                                    ctypes.byref(st)))
+        return st.as_dict()
+
+    # -- PLINK 1 .bed rows (payload only: the caller writes the magic bytes, pop_factory.BED_MAGIC, first)
+    def bed_pitch(self):
+        """Bytes per .bed row: ceil(samples / 4)."""
+        return (self.n_samples + 3) // 4
+
+    def generate_bed(self, row_begin, row_end, seed):
+        """.bed bytes of rows [row_begin,row_end) -> (bytes, stats dict)."""
+        out = np.empty(max((row_end - row_begin) * self.bed_pitch(), 1), dtype=np.uint8)
+        st = Stats()
+        self._check(self._lib.dnaf_generate_bed(self._h, row_begin, row_end, seed, _u8(out), out.nbytes, ctypes.byref(st)))
+        return out[:(row_end - row_begin) * self.bed_pitch()].tobytes(), st.as_dict()
+
+    def generate_bed_into(self, row_begin, row_end, seed, out):
+        """Same, into a caller-owned uint8 numpy buffer (page-locked memory is written by DMA); returns stats dict."""
+        st = Stats()
+        self._check(self._lib.dnaf_generate_bed(self._h, row_begin, row_end, seed, _u8(out), out.nbytes, ctypes.byref(st)))
+        return st.as_dict()
+
+    def generate_bed_fd_at(self, row_begin, row_end, seed, fd, file_offset):
+        """Same bytes, written with pwrite() at `file_offset` of an open file descriptor; returns stats dict."""
+        st = Stats()
+        self._check(self._lib.dnaf_generate_bed_fd_at(self._h, row_begin, row_end, seed, fd, int(file_offset), ctypes.byref(st)))
+        return st.as_dict()
+
+    def generate_bed_device(self, row_begin, row_end, seed):
+        """Same work, output left on the device; returns stats dict."""
+        st = Stats()
+        self._check(self._lib.dnaf_generate_bed_device(self._h, row_begin, row_end, seed, ctypes.byref(st)))
         return st.as_dict()
 
     # -- parity gates

@@ -6,7 +6,8 @@
 //   Bio.bgzf.BgzfWriter.write          call site pop_factory.py:449
 // Work is cut into passes of at most `chunk_bytes` of uncompressed text; each pass is
 //   sample -> (overrides) -> format -> BGZF encode -> scan -> compact -> D2H -> sink      (generic path)
-// or the fused kernel (k_fused.cuh) followed by scan -> compact -> D2H -> sink.
+// or the fused kernel (k_fused.cuh) followed by scan -> compact -> D2H -> sink.  The PLINK 1 .bed writer
+// (dnaf_generate_bed*) is one kernel per pass, k_bed -> D2H -> sink (host_bed.h).
 #include <unistd.h>
 
 #include <algorithm>
@@ -23,6 +24,7 @@
 #include "../../include/dnaf_b200.h"
 #include "dnaf_device.cuh"
 #include "fused_host.h"
+#include "k_bed.cuh"
 #include "k_deflate.cuh"
 #include "k_fused.cuh"
 #include "k_fused_text.cuh"
@@ -40,6 +42,7 @@ using namespace dnaf;
 #include "host_plan.h"
 #include "host_sink.h"
 #include "host_passes.h"
+#include "host_bed.h"
 
 
 // ================================================================================================ C ABI
@@ -101,6 +104,8 @@ int dnaf_create(int device_ordinal, dnaf_ctx** out) {
     if ((e = cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
     if ((e = cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
     if ((e = cudaEventCreateWithFlags(&c->ev_join2, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
+    for (auto& ev : c->ev_bed)
+        if ((e = cudaEventCreate(&ev)) != cudaSuccess) return bail("cudaEventCreate", e);
     // CRC tables: byte table and x^(8k) mod P for k = 0..kBlk
     std::vector<uint32_t> tab(256), xp(kBlk + 1);
     for (uint32_t i = 0; i < 256; ++i) {
@@ -141,6 +146,8 @@ void dnaf_destroy(dnaf_ctx* c) {
     }
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev_join) cudaEventDestroy(c->ev_join);
+    for (auto& ev : c->ev_bed)
+        if (ev) cudaEventDestroy(ev);
     if (c->own_stream && c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }
@@ -211,6 +218,11 @@ int dnaf_set_samples(dnaf_ctx* c, uint32_t n, const uint8_t* sex, const uint8_t*
     c->h_xspans = hosttab::build_xspans(sex, n, xoff.data());
     rc = upload(c, c->d_xspans, c->h_xspans.data(), c->h_xspans.size());
     if (rc) return rc;
+    {   // k_bed: which cells of a 16-sample group are male / female (haploid on X and Y, missing on Y)
+        const std::vector<uint32_t> m = bed_sex_masks(sex, n);
+        rc = upload(c, c->d_sexmask, m.data(), m.size());
+        if (rc) return rc;
+    }
     {   // X rows: the sample that holds body byte 256*k (for k_fused_text)
         std::vector<uint32_t> xspan((size_t)acc / 256 + 2, 0);
         uint32_t i = 0;
@@ -550,6 +562,34 @@ int dnaf_generate_device(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint
     Sink s;
     s.device_only = true;
     return generate_impl(c, row_begin, row_end, seed, level, s, stats);
+}
+
+int dnaf_generate_bed(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out, uint64_t out_cap,
+                      dnaf_stats* stats) {
+    if (!c) return DNAF_E_ARG;
+    if (!out && out_cap) return fail(c, DNAF_E_ARG, "out is NULL");
+    Sink s;
+    s.buf = out;
+    s.cap = out_cap;
+    return bed_impl(c, row_begin, row_end, seed, s, stats);
+}
+
+int dnaf_generate_bed_fd_at(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, int fd, uint64_t file_offset,
+                            dnaf_stats* stats) {
+    if (!c) return DNAF_E_ARG;
+    if (fd < 0) return fail(c, DNAF_E_ARG, "bad file descriptor");
+    if (file_offset > (uint64_t)INT64_MAX) return fail(c, DNAF_E_ARG, "file offset out of range");
+    Sink s;
+    s.fd = fd;
+    s.fd_off = (int64_t)file_offset;
+    return bed_impl(c, row_begin, row_end, seed, s, stats);
+}
+
+int dnaf_generate_bed_device(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, dnaf_stats* stats) {
+    if (!c) return DNAF_E_ARG;
+    Sink s;
+    s.device_only = true;
+    return bed_impl(c, row_begin, row_end, seed, s, stats);
 }
 
 int dnaf_genotypes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out, uint64_t cap) {

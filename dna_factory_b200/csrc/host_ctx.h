@@ -1,6 +1,6 @@
 // Host-side state of one GPU context (struct dnaf_ctx), error / trace helpers, uploads and the row layout.
 // Part of the single translation unit dnaf_api.cu (included there, in order: host_ctx.h, host_tables.h,
-// host_plan.h, host_sink.h, host_passes.h).
+// host_plan.h, host_sink.h, host_passes.h, host_bed.h).
 #pragma once
 
 namespace {
@@ -137,6 +137,7 @@ struct dnaf_ctx {
         int copy_mode = 0;                   // 0 nothing in flight, 1 DMA into the caller's pinned buffer, 2 via h_out
         uint64_t copy_bytes = 0;
         const uint8_t* copy_dst = nullptr;   // mode 1: where in the caller's buffer the pass lands
+        bool bed_timed = false;              // a k_bed launch (ev[0] -> ev[1]) whose time is not counted yet
     } ob[3];
     // optional record of every BGZF block handed to a host sink by dnaf_generate* (dnaf_block_log)
     bool log_blocks = false;
@@ -195,6 +196,8 @@ struct dnaf_ctx {
     bool seg_tabs_dirty = false;
     std::vector<uint8_t> h_pfx_tab;        // per row: prefix ends with '\t' (k_auto's first match may reach into it)
     std::vector<XSpan> h_xspans;
+    DevBuf d_sexmask;                      // k_bed: per 16-sample group, bit pairs of the males (x) and females (y)
+    cudaEvent_t ev_bed[2] = {};            // k_bed calls: first launch, last kernel end
     std::vector<uint32_t> h_seg_crc_x;     // L(template body) per X segment
     std::vector<uint32_t> h_xoff;
     std::vector<FusedDesc> xplan;

@@ -75,17 +75,19 @@ int generate_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t 
 // The pass pipeline keeps up to three passes in flight.  When a call fails half way (sink error, caller's buffer
 // too small, CUDA error) nothing of it may still be running when the error is returned: a copy could be landing in a
 // caller buffer that is about to be freed, and the next call must find an idle pipeline.
+void quiesce(dnaf_ctx* c) {
+    cudaSetDevice(c->dev);
+    cudaStreamSynchronize(c->stream);   // may be the caller's stream (dnaf_set_stream), NULL = the default stream
+    for (cudaStream_t s : {c->side, c->side2, c->comp, c->copy})
+        if (s) cudaStreamSynchronize(s);
+    cudaGetLastError();
+    for (auto& b : c->ob) b.copy_mode = 0;
+}
+
 int generate_impl(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, int level,
                   Sink& sink, dnaf_stats* st) {
     const int rc = generate_passes(c, row_begin, row_end, seed, level, sink, st);
-    if (rc && c) {
-        cudaSetDevice(c->dev);
-        cudaStreamSynchronize(c->stream);   // may be the caller's stream (dnaf_set_stream), NULL = the default stream
-        for (cudaStream_t s : {c->side, c->side2, c->comp, c->copy})
-            if (s) cudaStreamSynchronize(s);
-        cudaGetLastError();
-        for (auto& b : c->ob) b.copy_mode = 0;
-    }
+    if (rc && c) quiesce(c);
     return rc;
 }
 

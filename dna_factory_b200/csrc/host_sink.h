@@ -153,6 +153,8 @@ int close_pass(dnaf_ctx* c, dnaf_ctx::OutBuf& B, uint32_t nb, dnaf_stats* st) {
     return DNAF_OK;
 }
 
+int queue_copy(dnaf_ctx* c, dnaf_ctx::OutBuf& B, Sink& sink, uint64_t bytes);
+
 // A closed pass: wait for its kernels and totals, account it, and START moving its bytes to the host (straight
 // into a page-locked caller buffer when there is one).  finish_copy() completes the move.
 int start_copy(dnaf_ctx* c, dnaf_ctx::OutBuf& B, Sink& sink, dnaf_stats* st) {
@@ -188,6 +190,12 @@ int start_copy(dnaf_ctx* c, dnaf_ctx::OutBuf& B, Sink& sink, dnaf_stats* st) {
         st->rows += B.rows;
         st->text_bytes += B.text;
     }
+    return queue_copy(c, B, sink, bytes);
+}
+
+// Queues the D2H copy of `bytes` bytes of B.d_out on the copy stream: straight into a page-locked caller buffer, else into
+// the page-locked staging buffer that finish_copy() delivers from.  Device-only sinks only count the bytes.
+int queue_copy(dnaf_ctx* c, dnaf_ctx::OutBuf& B, Sink& sink, uint64_t bytes) {
     B.copy_mode = 0;
     B.copy_bytes = bytes;
     if (sink.device_only || !bytes) {

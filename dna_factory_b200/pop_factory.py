@@ -35,6 +35,18 @@ from .snp import (CHROMOSOME_LIST, CHROMOSOME_MAX_POSITION, CHROMOSOME_PROB, SNP
 MIN_SNP_FREQ = 0.005
 MIN_TOTAL_COUNT = 1000
 OUTPUT_DIR = os.path.join(os.getcwd(), "populations")
+BED_MAGIC = b"\x6c\x1b\x01"     # PLINK 1 .bed, SNP-major
+
+
+def validate_bed_table(table):
+    """--bed needs a column-form SNP table (SnpTable) without rows of more than 2 alleles: checked before the VCF is
+    written, so a table PLINK 1 cannot hold fails at once instead of after the whole generation."""
+    if not isinstance(table, SnpTable):
+        raise ValueError("--bed needs SNP records that fit the column form (integer ids, one-letter alleles)")
+    bad = numpy.nonzero(table.n_alleles > 2)[0]
+    if len(bad):
+        raise ValueError("--bed: SNP rs%d (row %d) has %d alleles; PLINK 1 .bed / .bim hold biallelic SNPs only" % (
+            int(table.ids[bad[0]]), int(bad[0]), int(table.n_alleles[bad[0]])))
 
 
 def gen_vcf_header(fam_data):
@@ -179,7 +191,7 @@ class DeleteriousGroup:
 class PopulationFactory:
     def __init__(self, num_processes=1, generate_snps=False, male_odds=0.5, deleterious_config=None,
                  deleterious_list_path=None, sample_id_offset=0, snps_path=None, output_path=None, seed=None,
-                 gpus=1, gpu_select=False, tbi=False):
+                 gpus=1, gpu_select=False, tbi=False, bed=False):
         self.deleterious = {}
         self.ordered_snps = []
         self.snp_table = None
@@ -199,7 +211,9 @@ class PopulationFactory:
         self.gpus = max(1, gpus or 1)
         self.gpu_select = bool(gpu_select)
         self.tbi = bool(tbi)
+        self.bed = bool(bed)
         self.stats = []
+        self.bed_stats = []      # dnaf_stats of the .bed calls (--bed)
 
     # ------------------------------------------------------------------------------------------ orchestration
     def generate_population(self, control_size, test_size, min_freq, max_snps, compression_level=6):
@@ -296,33 +310,46 @@ class PopulationFactory:
     def output_vcf_population(self, control_size, test_size, male_odds, compression_level):
         if not self._n_snps():
             raise Exception("No SNPs to Process! Exiting.")
+        snps = self.snp_table if self.snp_table is not None else self.ordered_snps
+        if self.bed:
+            validate_bed_table(snps)
         groups = PopulationFactory.pick_deleterious_groups(list(self.deleterious.values()), test_size)
         fam_data = self.generate_fam_file(control_size, test_size, male_odds, groups)
         main_file = self.population_dir + "population.vcf.gz"
         self._level = compression_level
         engine = _native.Engine(0)
+        bed_fd = None
         try:
+            if self.bed:
+                # population.bed / .bim beside population.fam: `plink --bfile population` reads the same population
+                bed_fd = os.open(self.population_dir + "population.bed", os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o644)
+                os.write(bed_fd, BED_MAGIC)
             with BgzfSink(main_file, engine, compresslevel=compression_level, index=self.tbi) as f:
                 f.write(gen_vcf_header(fam_data))
                 print("Outputing VCF lines", flush=True)
-                snps = self.snp_table if self.snp_table is not None else self.ordered_snps
                 # the reference cuts the list into ~1 M-SNP chunks to bound its memory (pop_factory.py:402-413);
                 # the GPU path streams, so one call covers the whole list
-                self.write_vcf_snps(fam_data, snps, f, engine=engine)
+                self.write_vcf_snps(fam_data, snps, f, engine=engine, bed_fd=bed_fd)
                 print("%s Finished work chunk 1 of 1." % datetime.now().strftime("%Y-%m-%d %H:%M"), flush=True)
             if self.tbi:
                 # what `bcftools index -t` (README.md:98-99) would derive by inflating the file again
                 blob, _ = engine.bgzf_compress(f.index.payload())
                 with open(main_file + ".tbi", "wb") as t:
                     t.write(blob + _native.bgzf_eof())
+            if self.bed:
+                with open(self.population_dir + "population.bim", "wb") as b:
+                    b.write(snps.bim_bytes())
         finally:
             engine.close()
+            if bed_fd is not None:
+                os.close(bed_fd)
         print("Finished VCF file output.", flush=True)
 
     # ------------------------------------------------------------------------------------------ the GPU seam
-    def write_vcf_snps(self, fam_data, snps, file, engine=None):
+    def write_vcf_snps(self, fam_data, snps, file, engine=None, bed_fd=None):
         """Rows of `snps` (in order) for `fam_data`, appended to `file` -- the reference's seam
-        (pop_factory.py:417-469).  `snps` is a list of SNPTuples or a SnpTable; `file` a BgzfSink."""
+        (pop_factory.py:417-469).  `snps` is a list of SNPTuples or a SnpTable; `file` a BgzfSink.  With `bed_fd`
+        (an open population.bed that holds the 3 magic bytes) the same rows also go there as PLINK 1 .bed rows."""
         t0 = time.time()
         level = getattr(file, "compresslevel", getattr(self, "_level", 6))
         seed = self.seed if self.seed is not None else int(datetime.now().strftime("%H%M%S"))
@@ -357,21 +384,24 @@ class PopulationFactory:
                 if index is not None:
                     index.add_blocks(*eng.block_log_get())
                     eng.block_log(False)
+                if bed_fd is not None:
+                    self.bed_stats.append(eng.generate_bed_fd_at(0, n_rows, seed, bed_fd, len(BED_MAGIC)))
             finally:
                 if own:
                     eng.close()
         else:
             self._write_multi_gpu(sex, ctl, arrays, orow, osamp, n_rows, seed, level, file, gpus,
-                                  index_rows if index is not None else None)
+                                  index_rows if index is not None else None, bed_fd)
         print("Finished write_vcf_snps chunk Elapsed time: {:0.4f} seconds".format(time.time() - t0))
 
-    def _write_multi_gpu(self, sex, ctl, arrays, orow, osamp, n_rows, seed, level, file, gpus, index_rows=None):
+    def _write_multi_gpu(self, sex, ctl, arrays, orow, osamp, n_rows, seed, level, file, gpus, index_rows=None, bed_fd=None):
         """Contiguous SNP ranges per GPU, no collective (SURVEY 8e; the reference stripes SNPs over its workers the
         same way, pop_factory.py:426).  BGZF blocks concatenate and the kernels are deterministic, so every rank
         first SIZES its stream on the device (dnaf_generate_device: no host traffic), the exclusive sum of the sizes
         gives every rank its offset in population.vcf.gz, and then all ranks pwrite() their streams side by side --
         nothing is spooled or copied twice.  Every rank holds only its own slice of the SNP table; the Philox row
-        counter of its local row r is bounds[g] + r (dnaf_set_row_base)."""
+        counter of its local row r is bounds[g] + r (dnaf_set_row_base).  .bed rows have a fixed size, so rank g
+        pwrite()s its rows at 3 + bounds[g] * ceil(N/4) of population.bed without a sizing pass."""
         bounds = partition.row_bounds(n_rows, gpus)
         n_dev = max(1, _native.device_count())      # more ranks than devices: ranks share devices round-robin
         errors = []
@@ -410,6 +440,8 @@ class PopulationFactory:
                 if st["bgzf_bytes"] != sizes[g]:
                     raise RuntimeError("rank %d: stream is %d bytes, its sizing pass said %d" % (g, st["bgzf_bytes"], sizes[g]))
                 self.stats.append(st)
+                if bed_fd is not None:
+                    self.bed_stats.append(eng.generate_bed_fd_at(0, hi - lo, seed, bed_fd, len(BED_MAGIC) + lo * eng.bed_pitch()))
                 if index is not None:
                     blocks[g] = eng.block_log_get()
             except BaseException as e:  # noqa
@@ -492,6 +524,9 @@ def parse_cmd_args(args):
                     help="draw and sort the simulated SNPs on the GPU from the --seed stream instead of numpy's global state")
     ap.add_argument("--tbi", action="store_true",
                     help="also write population.vcf.gz.tbi (tabix index) from the row and block sizes the writer already knows")
+    ap.add_argument("--bed", action="store_true",
+                    help="also write population.bed / population.bim (PLINK 1 binary fileset beside population.fam, "
+                         "A1 = ALT); every SNP must be biallelic")
     return ap.parse_args(args)
 
 
@@ -504,7 +539,7 @@ def main(sys_args):
                                 deleterious_list_path=args.deleterious_file, sample_id_offset=args.offset,
                                 male_odds=args.male_odds, deleterious_config=args.deleterious_config,
                                 snps_path=args.snps_file, output_path=args.outdir, seed=args.seed, gpus=args.gpus,
-                                gpu_select=args.gpu_select, tbi=args.tbi)
+                                gpu_select=args.gpu_select, tbi=args.tbi, bed=args.bed)
     factory.generate_population(args.control_size, args.size, args.min_freq, args.max_snps, args.compression_level)
 
 

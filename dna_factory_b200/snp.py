@@ -106,6 +106,39 @@ class SNPTuples:
         return snp
 
 
+def _label_matrix(labels):
+    """Chromosome labels as a zero-padded uint8 matrix, one row per label."""
+    lab = np.zeros((len(labels), max(len(c.encode("latin-1")) for c in labels)), np.uint8)
+    for i, c in enumerate(labels):
+        b = c.encode("latin-1")
+        lab[i, :len(b)] = np.frombuffer(b, np.uint8)
+    return lab
+
+
+def _digits(v):
+    """Decimal digits of non-negative ints, right-aligned in a fixed width, with the mask of the printed ones."""
+    width = max(1, len(str(int(v.max()))))
+    p = 10 ** np.arange(width - 1, -1, -1, dtype=np.int64)
+    d = (v[:, None] // p[None, :]) % 10
+    nd = 1 + (v[:, None] >= p[None, :-1]).sum(axis=1) if width > 1 else np.ones(len(v), np.int64)
+    ok = np.arange(width)[None, :] >= (width - nd)[:, None]
+    return (d + 48).astype(np.uint8), ok
+
+
+def _const(b, rows):
+    a = np.frombuffer(b, np.uint8)
+    return np.broadcast_to(a, (rows, len(a))), np.ones((rows, len(a)), bool)
+
+
+def _join_fields(fields, rows):
+    """Row-major concatenation of (bytes, mask) field matrices -> (flat bytes, row offsets[rows + 1])."""
+    data = np.concatenate([f[0] for f in fields], axis=1)
+    mask = np.concatenate([f[1] for f in fields], axis=1)
+    off = np.zeros(rows + 1, np.uint64)
+    off[1:] = np.cumsum(mask.sum(axis=1))
+    return data[mask], off
+
+
 class SnpTable:
     """Column form of a SNP list (biallelic fast path + generic K <= 4)."""
 
@@ -216,23 +249,9 @@ class SnpTable:
             return np.zeros(1, np.uint8), np.zeros(1, np.uint64)
         if np.any(self.position < 0) or np.any(self.ids < 0):
             raise ValueError("negative position / id")
-        lab_w = max(len(c) for c in self.chrom_labels)
-        lab = np.zeros((len(self.chrom_labels), lab_w), np.uint8)
-        for i, c in enumerate(self.chrom_labels):
-            b = c.encode("latin-1")
-            lab[i, :len(b)] = np.frombuffer(b, np.uint8)
-
-        def digits(v, width):
-            p = 10 ** np.arange(width - 1, -1, -1, dtype=np.int64)
-            d = (v[:, None] // p[None, :]) % 10
-            nd = 1 + (v[:, None] >= p[None, :-1]).sum(axis=1) if width > 1 else np.ones(len(v), np.int64)
-            ok = np.arange(width)[None, :] >= (width - nd)[:, None]
-            return (d + 48).astype(np.uint8), ok
-
-        pw = max(1, len(str(int(self.position.max()))))
-        iw = max(1, len(str(int(self.ids.max()))))
-        pd, pok = digits(self.position, pw)
-        idd, iok = digits(self.ids, iw)
+        lab = _label_matrix(self.chrom_labels)
+        pd, pok = _digits(self.position)
+        idd, iok = _digits(self.ids)
         alt_w = 2 * (_native.KMAX - 1) - 1
         alt = np.zeros((S, alt_w), np.uint8)
         aok = np.zeros((S, alt_w), bool)
@@ -246,21 +265,32 @@ class SnpTable:
             aok[:, 2 * (j - 1) - 1] = k > j
             aok[:, 2 * (j - 1)] = k > j
         tail = np.frombuffer(b"\t40\tPASS\t.\tGT\t", np.uint8)
-
-        def const(b):
-            a = np.frombuffer(b, np.uint8)
-            return np.broadcast_to(a, (S, len(a))), np.ones((S, len(a)), bool)
-
         cl = lab[self.chrom_idx]
-        fields = [(cl, cl != 0), const(b"\t"), (pd, pok), const(b"\trs"), (idd, iok), const(b"\t"),
-                  (self.nts[:, :1], np.ones((S, 1), bool)), const(b"\t"), (alt, aok), (np.broadcast_to(tail, (S, len(tail))),
-                                                                                       np.ones((S, len(tail)), bool))]
-        data = np.concatenate([f[0] for f in fields], axis=1)
-        mask = np.concatenate([f[1] for f in fields], axis=1)
-        off = np.zeros(S + 1, np.uint64)
-        off[1:] = np.cumsum(mask.sum(axis=1))
-        flat = data[mask]
+        fields = [(cl, cl != 0), _const(b"\t", S), (pd, pok), _const(b"\trs", S), (idd, iok), _const(b"\t", S),
+                  (self.nts[:, :1], np.ones((S, 1), bool)), _const(b"\t", S), (alt, aok), (np.broadcast_to(tail, (S, len(tail))),
+                                                                                          np.ones((S, len(tail)), bool))]
+        flat, off = _join_fields(fields, S)
         return np.concatenate([flat, np.zeros(1, np.uint8)]), off
+
+    def bim_bytes(self):
+        """PLINK .bim text, one line per row: "chrom\trs<id>\t0\tposition\tA1\tA2\n" with A1 = ALT ('0' for K == 1)
+        and A2 = REF, the allele order of the .bed codes (dnaf_generate_bed).  Rows with K > 2 have no .bim form."""
+        S = len(self)
+        if S == 0:
+            return b""
+        if np.any(self.n_alleles > 2):
+            raise ValueError("SNP %d has %d alleles: PLINK 1 filesets hold biallelic rows only" % (
+                int(self.ids[np.argmax(self.n_alleles > 2)]), int(self.n_alleles[np.argmax(self.n_alleles > 2)])))
+        if np.any(self.position < 0) or np.any(self.ids < 0):
+            raise ValueError("negative position / id")
+        cl = _label_matrix(self.chrom_labels)[self.chrom_idx]
+        pd, pok = _digits(self.position)
+        idd, iok = _digits(self.ids)
+        a1 = np.where(self.n_alleles == 1, ord("0"), self.nts[:, 1]).astype(np.uint8)[:, None]
+        one = np.ones((S, 1), bool)
+        fields = [(cl, cl != 0), _const(b"\trs", S), (idd, iok), _const(b"\t0\t", S), (pd, pok), _const(b"\t", S),
+                  (a1, one), _const(b"\t", S), (self.nts[:, :1], one), _const(b"\n", S)]
+        return _join_fields(fields, S)[0].tobytes()
 
     def device_arrays(self):
         pre, off = self.prefix_bytes()

@@ -191,6 +191,23 @@ int dnaf_generate_fd_at(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uin
 int dnaf_generate_device(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, int level,
                          dnaf_stats* stats);
 
+/*
+ * PLINK 1 binary genotypes (.bed) of rows [row_begin,row_end): the same draws, forced minors and ploidy rules as the
+ * VCF rows of the same seed (pop_factory.py:481-499), so population.bed and population.vcf.gz describe one population.
+ * Payload only: ceil(n_samples/4) bytes per row, SNP-major, no magic bytes (the caller writes 6C 1B 01 first, like it
+ * writes the VCF header).  Sample i sits in byte i/4 at bits 2(i%4), 2(i%4)+1; padding bits are 0.  Values count ALT
+ * copies with .bim A1 = ALT, A2 = REF: 2 copies -> 0, 1 -> 2, 0 -> 3, missing ('.', females on Y) -> 1; haploid cells
+ * are written homozygous.  Rows with more than 2 alleles cannot be written: DNAF_E_INPUT before any GPU work, naming
+ * the row.  stats: rows, calls, kernel_launches, ms_sample (the .bed kernel), ms_total; the other fields are 0.
+ */
+int dnaf_generate_bed(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out, uint64_t out_cap,
+                      dnaf_stats* stats);
+/* Same bytes written with pwrite() at file_offset (3 + first row * ceil(n_samples/4) in population.bed). */
+int dnaf_generate_bed_fd_at(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, int fd,
+                            uint64_t file_offset, dnaf_stats* stats);
+/* Same work, output left in device memory: kernel-only timing. */
+int dnaf_generate_bed_device(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, dnaf_stats* stats);
+
 /* Parity gates. genotypes: out[(r*n_samples+i)*2+s] = allele index, 0xFF where the cell has no such
  * allele (second slot of a haploid cell, both slots of '.').  text: the uncompressed rows. */
 int dnaf_genotypes(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out,
