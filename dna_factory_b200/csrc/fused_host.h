@@ -415,7 +415,7 @@ inline XTable make_x_table(double p_minor, const std::vector<XSpan>& xspans, int
             c[k >> 5] = (c[k >> 5] & ~(1u << (k & 31))) | (v << (k & 31));
         }
         const bool first = (sp % (size_t)std::max(1, per_block)) == 0;
-        xspan_tokens_ref(c, first ? (c[0] & 3u) : carry, xs, first, false, false, hs);
+        xspan_tokens_ref(c, first ? (c[0] & 3u) : carry, xs, (int)xs.L, first, false, false, hs);
         carry = L >= 2 ? ((bit128(c, (int)L - 1) << 1) | bit128(c, (int)L - 2)) : 0u;
     }
     const uint64_t blocks = std::max<uint64_t>(1, ns / (size_t)std::max(1, per_block));

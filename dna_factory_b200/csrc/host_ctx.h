@@ -129,6 +129,8 @@ struct dnaf_ctx {
         size_t stage_used = 0;
         cudaEvent_t ev[6] = {};
         cudaEvent_t ev_auto[2] = {};         // around the k_auto launch
+        cudaEvent_t auto_from = nullptr, auto_to = nullptr;   // what k_auto's time is read between: ev_auto[0/1], or
+                                                              // ev[3] / ev[4] when nothing else is queued in between
         uint64_t auto_text = 0;              // text bytes of the pass's k_auto blocks (0: no k_auto launch)
         cudaEvent_t ev_copied = nullptr;
         uint32_t nb = 0;
@@ -175,9 +177,9 @@ struct dnaf_ctx {
     // k_auto (k_auto.cuh): code tables + byte LUTs per (bucket, starts-row), CRC move tables, per-row prefix CRCs
     DevBuf d_atables, d_etab2, d_mtab, d_mtail, d_mpre, d_xinit, d_pre_crc;
     DevBuf d_xtables, d_mspan, d_mpre_x;   // k_x (k_x.cuh)
-    DevBuf d_bucket, d_ovr_first, d_seginfo;   // implicit block descriptors of all-autosome passes (k_auto.cuh)
+    DevBuf d_bucket, d_ovr_first, d_seginfo;   // implicit block descriptors of autosome runs (k_auto.cuh)
     std::vector<uint32_t> h_other;          // [S+1]: rows before r that do NOT take k_auto
-    bool implicit_pass = false;
+    uint64_t implicit_rows = 0;             // leading rows of the pass whose k_auto blocks derive their own descriptors
     std::map<std::pair<uint64_t, uint64_t>, XTable>& xtable_cache = g_xtable_cache;
     std::vector<uint32_t> h_mspan, h_mpre_x;
     std::map<std::pair<uint64_t, uint64_t>, AutoTable>& atable_cache = g_atable_cache;

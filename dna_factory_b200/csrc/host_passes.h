@@ -120,6 +120,9 @@ int generate_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t 
     for (auto& b : c->ob) b.copy_mode = 0;
     int npass = 0;
     if (g_trace) { g_t0 = std::chrono::steady_clock::now(); trace("generate begins", 0); }
+    // the side streams of k_fused_text / k_x start after what the main stream holds when the call begins (tables,
+    // prefix CRCs, implicit descriptors); within the call they wait only for their pass's slot set
+    CU(c, cudaEventRecord(c->ev_fork, c->stream));
     while (r0 < row_end) {
         const int cur = npass % 3;
         rc = finish_copy(c, c->ob[cur], sink);
@@ -132,20 +135,7 @@ int generate_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t 
         const uint64_t r1 = next_chunk_end(c, r0, row_end, std::max<uint64_t>(c->chunk_bytes >> std::max(0, ramp - npass), 4096));
         dnaf_ctx::OutBuf& B = c->ob[cur];
         const auto t_plan0 = std::chrono::steady_clock::now();
-        c->implicit_pass = c->fused_ok && c->h_other[r1] == c->h_other[r0] && !c->h_seg_crc.empty();
-        if (c->implicit_pass) {   // autosome rows only: k_auto derives its descriptors, the host plans nothing
-            c->fplan.clear(); c->xplan.clear(); c->tplan.clear(); c->plan.clear(); c->gslot.clear(); c->grow.clear();
-            c->goff.clear(); c->olocal.clear(); c->osub.clear();
-            c->gen_text_bytes = 0;
-            const uint32_t nseg = (uint32_t)c->h_seg_crc.size();
-            c->pass_blocks = (uint32_t)(r1 - r0) * nseg;
-            uint32_t longest = 0;
-            for (uint32_t sg = 0; sg < nseg; ++sg) longest = std::max(longest, 4u * (c->h_seg_cell0[sg + 1] - c->h_seg_cell0[sg]) + 66u);
-            c->slot_stride = std::min<uint32_t>(kSlot, (longest + 128u + 255u) & ~255u);
-            c->pass_text = c->h_row_off[r1] - c->h_row_off[r0];
-        } else {
-            plan_pass(c, r0, r1, c->h_k.data());
-        }
+        plan_pass(c, r0, r1, implicit_end(c, r0, r1), c->h_k.data());
         const auto t_plan1 = std::chrono::steady_clock::now();
         c->cur_ob = cur;
         rc = reserve_outputs(c, B, c->pass_blocks, c->pass_text);
@@ -162,26 +152,35 @@ int generate_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t 
                                      c->d_olocal.as<uint32_t>(), c->d_osub.as<uint32_t>(), &local);
             if (rc) return rc;
         }
-        CU(c, cudaEventRecord(B.ev[1], c->stream));
+        // A timed event between two kernels of the main stream is not free on the GPU: record only the marks whose
+        // intervals are read (start_copy), and let k_auto's interval share ev[3] / ev[4] when nothing else is queued
+        // between them.  ev[1], ev[2] time the generic path (grows != 0 whenever a pass has generic blocks).
         if (grows) {
+            CU(c, cudaEventRecord(B.ev[1], c->stream));
             rc = run_format(c, r0, grows, c->d_grow.as<uint32_t>(), c->d_goff.as<uint64_t>(), c->gen_text_bytes, &local);
             if (rc) return rc;
+            CU(c, cudaEventRecord(B.ev[2], c->stream));
         }
-        CU(c, cudaEventRecord(B.ev[2], c->stream));
         rc = launch_generic(c, &local);
         if (rc) return rc;
         CU(c, cudaEventRecord(B.ev[3], c->stream));
-        // descriptors of the three fused kernels go up first; the few, long blocks of k_fused_text / k_fused_x then start
-        // on the high-priority side stream and k_auto fills the rest of the chip from the main stream
-        if (!c->tplan.empty()) rc = upload_async(c, c->d_tdesc, c->tplan);
-        if (!rc && !c->xplan.empty()) rc = upload_async(c, c->d_xdesc, c->xplan);
-        if (!rc && !c->fplan.empty()) rc = upload_async(c, c->d_fdesc, c->fplan);
+        // k_fused_text and k_x write only their own slots of this pass's slot set and read descriptors that go up on
+        // their own high-priority streams, so they do not queue behind the previous pass's k_auto: they start as soon as
+        // the slot set is free (the compaction two passes ago is done) and finish under that k_auto, and the upload of
+        // their descriptors stays off the main stream.  k_auto's own descriptors (if any) go up on the main stream.
+        if (!c->fplan.empty()) rc = upload_async(c, c->d_fdesc, c->fplan);
         if (rc) return rc;
-        const bool side_work = !c->tplan.empty() || !c->xplan.empty();
-        if (side_work) {
-            CU(c, cudaEventRecord(c->ev_fork, c->stream));
-            if (!c->tplan.empty()) CU(c, cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-            if (!c->xplan.empty()) CU(c, cudaStreamWaitEvent(c->side2, c->ev_fork, 0));
+        if (!c->tplan.empty()) {
+            CU(c, cudaStreamWaitEvent(c->side, c->ev_fork, 0));
+            CU(c, cudaStreamWaitEvent(c->side, c->sbuf[c->sb].ev_free, 0));
+            rc = upload_async(c, c->d_tdesc, c->tplan, c->side);
+            if (rc) return rc;
+        }
+        if (!c->xplan.empty()) {
+            CU(c, cudaStreamWaitEvent(c->side2, c->ev_fork, 0));
+            CU(c, cudaStreamWaitEvent(c->side2, c->sbuf[c->sb].ev_free, 0));
+            rc = upload_async(c, c->d_xdesc, c->xplan, c->side2);
+            if (rc) return rc;
         }
         if (!c->tplan.empty()) {
             if (!c->text_attr_done) {
@@ -235,11 +234,13 @@ int generate_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t 
         }
         if (!c->tplan.empty()) CU(c, cudaEventRecord(c->ev_join, c->side));
         if (!c->xplan.empty()) CU(c, cudaEventRecord(c->ev_join2, c->side2));
-        if (!c->fplan.empty() || c->implicit_pass) {
+        // one k_auto launch: the implicit opening run of the pass, or else the planned blocks (implicit_end never leaves
+        // k_auto rows to plan after an implicit run)
+        if (!c->fplan.empty() || c->implicit_rows) {
             AutoArgs fa;
             fa.sv = sample_view(c);
             fa.nv = snp_view(c);
-            fa.desc = c->implicit_pass ? nullptr : c->d_fdesc.as<FusedDesc>();
+            fa.desc = c->implicit_rows ? nullptr : c->d_fdesc.as<FusedDesc>();
             fa.row0 = r0;
             fa.nseg = (uint32_t)c->h_seg_crc.size();
             fa.nseg_magic = fa.nseg > 1 ? (uint32_t)(((1ull << 32) + fa.nseg - 1) / fa.nseg) : 0u;
@@ -263,8 +264,9 @@ int generate_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t 
             fa.slot_stride = c->slot_stride;
             fa.sizes = c->sbuf[c->sb].sizes.as<uint32_t>();
             fa.crcs = c->sbuf[c->sb].crcs.as<uint32_t>();
-            CU(c, cudaEventRecord(B.ev_auto[0], c->stream));
-            const uint32_t ablocks = c->implicit_pass ? c->pass_blocks : (uint32_t)c->fplan.size();
+            B.auto_from = c->fplan.empty() ? B.ev[3] : B.ev_auto[0];   // k_auto's descriptors went up after ev[3]
+            if (!c->fplan.empty()) CU(c, cudaEventRecord(B.ev_auto[0], c->stream));
+            const uint32_t ablocks = c->implicit_rows ? (uint32_t)c->implicit_rows * fa.nseg : (uint32_t)c->fplan.size();
             if (use_lz) {
                 const LzCfg cfg = lz_cfg(level, kLzMaxKey);
                 const uint32_t smem = lz_smem_bytes(c->fused_threads, kLzMaxKey + 1u, cfg.chain != 0u);
@@ -279,9 +281,11 @@ int generate_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t 
             } else {
                 k_auto<<<ablocks, c->fused_threads, auto_smem_bytes(c->fused_threads), c->stream>>>(fa);
             }
-            CU(c, cudaEventRecord(B.ev_auto[1], c->stream));
-            if (c->implicit_pass) {
-                B.auto_text = c->pass_text;
+            const bool joins = !c->tplan.empty() || !c->xplan.empty();
+            B.auto_to = joins ? B.ev_auto[1] : B.ev[4];
+            if (joins) CU(c, cudaEventRecord(B.ev_auto[1], c->stream));
+            if (c->implicit_rows) {
+                B.auto_text = c->h_row_off[r0 + c->implicit_rows] - c->h_row_off[r0];
             } else {   // text of the planned k_auto blocks: prefix on a row's first block, cells, '\n' for '\t' at the row's end
                 uint64_t t = 0;
                 for (const FusedDesc& d : c->fplan) t += 4ull * d.ncells + ((d.flags & 1u) ? c->h_plen[d.row] : 0u);
@@ -293,17 +297,19 @@ int generate_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t 
         if (!c->tplan.empty()) CU(c, cudaStreamWaitEvent(c->stream, c->ev_join, 0));
         if (!c->xplan.empty()) CU(c, cudaStreamWaitEvent(c->stream, c->ev_join2, 0));
         CU(c, cudaEventRecord(B.ev[4], c->stream));
-        if (c->fplan.empty() && !c->implicit_pass) B.auto_text = 0;
+        if (c->fplan.empty() && !c->implicit_rows) B.auto_text = 0;
         B.rows = r1 - r0;
         B.text = c->h_row_off[r1] - c->h_row_off[r0];
         B.gen = grows != 0;
         B.generic_blocks = !c->plan.empty();
-        B.fused = c->implicit_pass || !c->fplan.empty() || !c->tplan.empty() || !c->xplan.empty();
+        B.fused = c->implicit_rows || !c->fplan.empty() || !c->tplan.empty() || !c->xplan.empty();
         rc = close_pass(c, B, c->pass_blocks, &local);
         if (rc) return rc;
         if (g_trace) {
             const auto t_l = std::chrono::steady_clock::now();
-            fprintf(stderr, "[dnaf] pass rows %llu: plan %.0f us, launch %.0f us\n", (unsigned long long)(r1 - r0),
+            fprintf(stderr, "[dnaf] pass rows %llu implicit %llu blocks %u auto %zu x %zu text %zu generic %zu: plan %.0f us, launch %.0f us\n",
+                    (unsigned long long)(r1 - r0), (unsigned long long)c->implicit_rows, c->pass_blocks,
+                    c->implicit_rows * c->h_seg_crc.size() + c->fplan.size(), c->xplan.size(), c->tplan.size(), c->plan.size(),
                     std::chrono::duration<double, std::micro>(t_plan1 - t_plan0).count(),
                     std::chrono::duration<double, std::micro>(t_l - t_plan1).count());
             trace("launched pass", npass);

@@ -1,4 +1,4 @@
-// The planner: which kernel takes which row, the implicit block descriptors of all-autosome passes and the BGZF block
+// The planner: which kernel takes which row, the implicit block descriptors of autosome runs and the BGZF block
 // plan of one pass.  Included by dnaf_api.cu after host_tables.h.
 #pragma once
 
@@ -14,8 +14,8 @@ inline int row_kind(const dnaf_ctx* c, uint64_t r, const uint8_t* hk) {
 }
 inline bool row_is_fused(const dnaf_ctx* c, uint64_t r, const uint8_t* hk) { return row_kind(c, r, hk) != 0; }
 
-// What k_auto needs to derive its block descriptors itself when a pass holds autosome rows only: which rows those
-// are (host: prefix count of the others), the bucket and first override of every row, the segment table.
+// What k_auto needs to derive its block descriptors itself over a run of autosome rows: which rows those are (host:
+// prefix count of the others), the bucket and first override of every row, the segment table.
 int ensure_implicit(dnaf_ctx* c) {
     c->h_other.assign(c->S + 1, 0);
     uint32_t others = 0;
@@ -43,8 +43,26 @@ int ensure_implicit(dnaf_ctx* c) {
     return rc;
 }
 
-// BGZF block plan of one pass (rows [r0,r1)): fused segments and generic blocks, slots in row order.
-void plan_pass(dnaf_ctx* c, uint64_t r0, uint64_t r1, const uint8_t* hk) {
+// End of the run of rows that opens the pass [r0,r1) and whose k_auto blocks derive their descriptors themselves.
+// All-autosome passes run implicitly whole.  A pass that opens with autosome rows and holds none after its first
+// other row (a sorted step window ends with its MT, X and Y rows) runs that opening run implicitly and plans only the
+// rest, so that one k_auto launch covers the pass either way.  Any other pass is planned whole (r0), as is every mixed
+// pass when DNAF_FULL_PLAN is set (the reference for tests of the split).
+uint64_t implicit_end(const dnaf_ctx* c, uint64_t r0, uint64_t r1) {
+    if (!c->fused_ok || c->h_seg_crc.empty()) return r0;
+    const uint32_t o0 = c->h_other[r0];
+    if (c->h_other[r1] == o0) return r1;
+    static const bool full_plan = getenv("DNAF_FULL_PLAN") != nullptr;
+    if (full_plan) return r0;
+    // the first row that does not take k_auto: h_other first exceeds o0 one row after it
+    const uint64_t rx = std::upper_bound(c->h_other.begin() + r0, c->h_other.begin() + r1 + 1, o0) - c->h_other.begin() - 1;
+    return c->h_other[r1] - c->h_other[rx] == r1 - rx ? rx : r0;
+}
+
+// BGZF block plan of one pass (rows [r0,r1)): fused segments and generic blocks, slots in row order.  The k_auto blocks
+// of rows [r0,rx) (implicit_end) take slots 0 .. (rx-r0)*nseg-1 without descriptors; rows [rx,r1) are planned.
+void plan_pass(dnaf_ctx* c, uint64_t r0, uint64_t r1, uint64_t rx, const uint8_t* hk) {
+    c->implicit_rows = rx - r0;
     c->fplan.clear();
     c->xplan.clear();
     c->tplan.clear();
@@ -55,9 +73,10 @@ void plan_pass(dnaf_ctx* c, uint64_t r0, uint64_t r1, const uint8_t* hk) {
     c->olocal.clear();
     c->osub.clear();
     uint64_t gtext = 0;
-    uint32_t slot = 0;
-    size_t o = std::lower_bound(c->h_orow.begin(), c->h_orow.end(), r0) - c->h_orow.begin();
-    uint64_t r = r0;
+    const uint32_t nseg_auto = (uint32_t)c->h_seg_crc.size();
+    uint32_t slot = (uint32_t)(rx - r0) * nseg_auto;
+    size_t o = std::lower_bound(c->h_orow.begin(), c->h_orow.end(), rx) - c->h_orow.begin();
+    uint64_t r = rx;
     while (r < r1) {
         while (o < c->h_orow.size() && c->h_orow[o] < r) ++o;
         const int kind = row_kind(c, r, hk);
@@ -162,6 +181,8 @@ void plan_pass(dnaf_ctx* c, uint64_t r0, uint64_t r1, const uint8_t* hk) {
     // Slot stride of the pass: the longest block's text (a stored block is the worst case: text + 5) plus the slot
     // lead, BGZF framing, the zero-fill / copy overrun of the kernels (< 64 bytes), rounded up to 256.
     uint32_t longest = 0;
+    if (rx > r0)
+        for (uint32_t sg = 0; sg < nseg_auto; ++sg) longest = std::max(longest, 4u * (c->h_seg_cell0[sg + 1] - c->h_seg_cell0[sg]) + 66u);
     for (const FusedDesc& d : c->fplan) longest = std::max(longest, 4u * d.ncells + 66u);           // prefix <= 64, +1 lead, +1
     for (const FusedDesc& d : c->xplan) longest = std::max(longest, 4u * d.ncells + 66u);
     for (const TextDesc& d : c->tplan) longest = std::max(longest, d.nbytes + 66u);

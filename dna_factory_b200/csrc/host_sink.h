@@ -70,19 +70,20 @@ int deliver(dnaf_ctx* c, Sink& s, const uint8_t* data, uint64_t n) {
 // Uploads a host vector through the pass's page-locked staging arena, so the copy is asynchronous and the
 // host can go on planning while the previous pass still runs.  reserve_stage() sizes the arena up front.
 template <class T>
-int upload_async(dnaf_ctx* c, DevBuf& b, const std::vector<T>& v) {
+int upload_async(dnaf_ctx* c, DevBuf& b, const std::vector<T>& v, cudaStream_t s = 0) {
     CU(c, b.reserve(std::max<size_t>(v.size(), 1) * sizeof(T)));
     if (v.empty()) return DNAF_OK;
+    if (!s) s = c->stream;
     dnaf_ctx::OutBuf& B = c->ob[c->cur_ob];
     const size_t bytes = v.size() * sizeof(T);
     const size_t at = (B.stage_used + 63) & ~size_t(63);
     if (at + bytes > B.h_stage.cap) {  // not planned for: fall back to a pageable (synchronising) copy
-        CU(c, cudaMemcpyAsync(b.p, v.data(), bytes, cudaMemcpyHostToDevice, c->stream));
+        CU(c, cudaMemcpyAsync(b.p, v.data(), bytes, cudaMemcpyHostToDevice, s));
         return DNAF_OK;
     }
     memcpy(B.h_stage.as<uint8_t>() + at, v.data(), bytes);
     B.stage_used = at + bytes;
-    CU(c, cudaMemcpyAsync(b.p, B.h_stage.as<uint8_t>() + at, bytes, cudaMemcpyHostToDevice, c->stream));
+    CU(c, cudaMemcpyAsync(b.p, B.h_stage.as<uint8_t>() + at, bytes, cudaMemcpyHostToDevice, s));
     return DNAF_OK;
 }
 
@@ -166,23 +167,27 @@ int start_copy(dnaf_ctx* c, dnaf_ctx::OutBuf& B, Sink& sink, dnaf_stats* st) {
         st->bgzf_bytes += bytes;
         st->bgzf_blocks += B.nb;
         if (B.nb) st->crc_xor ^= (uint32_t)reinterpret_cast<volatile uint64_t*>(B.h_totals.p)[1];
+        // only the intervals that count: each query costs a few us of host time, and after a call's last pass they
+        // sit between the GPU going idle and the caller's next call
         float t01 = 0, t12 = 0, t23 = 0, t34 = 0, t45 = 0, t05 = 0;
-        cudaEventElapsedTime(&t01, B.ev[0], B.ev[1]);
-        cudaEventElapsedTime(&t12, B.ev[1], B.ev[2]);
-        cudaEventElapsedTime(&t23, B.ev[2], B.ev[3]);
-        cudaEventElapsedTime(&t34, B.ev[3], B.ev[4]);
-        cudaEventElapsedTime(&t45, B.ev[4], B.ev[5]);
-        cudaEventElapsedTime(&t05, B.ev[0], B.ev[5]);
         if (B.gen) {
+            cudaEventElapsedTime(&t01, B.ev[0], B.ev[1]);
+            cudaEventElapsedTime(&t12, B.ev[1], B.ev[2]);
             st->ms_sample += t01;
             st->ms_format += t12;
         }
-        st->ms_deflate += (B.generic_blocks ? t23 : 0.f) + t45;
-        if (B.fused) st->ms_fused += t34;
+        if (B.generic_blocks) cudaEventElapsedTime(&t23, B.ev[2], B.ev[3]);
+        cudaEventElapsedTime(&t45, B.ev[4], B.ev[5]);
+        cudaEventElapsedTime(&t05, B.ev[0], B.ev[5]);
+        st->ms_deflate += t23 + t45;
+        if (B.fused) {
+            cudaEventElapsedTime(&t34, B.ev[3], B.ev[4]);
+            st->ms_fused += t34;
+        }
         st->ms_total += t05;
         if (B.auto_text) {
             float ta = 0;
-            cudaEventElapsedTime(&ta, B.ev_auto[0], B.ev_auto[1]);
+            cudaEventElapsedTime(&ta, B.auto_from, B.auto_to);
             st->ms_auto += ta;
             st->auto_launches += 1;
             st->auto_text_bytes += B.auto_text;

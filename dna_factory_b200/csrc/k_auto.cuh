@@ -47,8 +47,8 @@ static_assert(kATabWords % 4 == 0 && sizeof(AutoTable) % 16 == 0, "AutoTable mus
 struct AutoArgs {
     SampleView sv;
     SnpView nv;
-    const FusedDesc* desc;     // one per block, or NULL: every row of the pass is an autosome row and block b is
-                               // segment b % nseg of row row0 + b / nseg (no host planning, nothing to upload)
+    const FusedDesc* desc;     // one per block, or NULL: the launch covers a run of autosome rows opening the pass and
+                               // block b is segment b % nseg of row row0 + b / nseg, at slot b (no host planning, nothing to upload)
     uint64_t row0;
     uint32_t nseg;
     uint32_t nseg_magic;       // ceil(2^32 / nseg): block / nseg == umulhi(block, magic) while block * nseg < 2^32

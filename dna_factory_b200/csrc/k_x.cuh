@@ -31,6 +31,7 @@ struct XSpan {          // static per population, one per 64 samples
     uint32_t byte_off;  // body byte offset of the span's first sample
     uint8_t sk6[32];    // per unit u: separator kinds of positions 4u-2 .. 4u+3 (positions past L repeat, no mismatch)
 };
+static_assert(offsetof(XSpan, sk6) % 16 == 0 && sizeof(XSpan) % 16 == 0, "k_x loads XSpan::sk6 as two 16-byte words");
 
 // compacted allele bits of one span (4 words -> 128-bit little-endian sequence of total length L)
 __host__ __device__ __forceinline__ uint32_t compact_span(const uint32_t m[4], const XSpan& xs, uint32_t c[4]) {
@@ -127,14 +128,13 @@ __host__ __device__ __forceinline__ uint32_t win6(const uint32_t v[4], uint32_t 
     return r;
 }
 
-// ---- the span grammar (host statistics + device slow path).  c: compacted alleles, positions past L repeat. ----
+// ---- the span grammar (host statistics + device slow path).  c: compacted alleles, L of them; positions past L repeat. ----
 //   first span of a block: unit 0 as eight literals
 //   whole units (nfull = (L - row_end) / 4): xunit_tokens, bridged by matches of 0 or >= 3 bytes
 //   the rest, event by event; ['\n' when the span ends the row]; [EOB when it ends the block]
 template <class Sink>
-__host__ __device__ inline void xspan_tokens_ref(const uint32_t c[4], uint32_t carry, const XSpan& xs, bool first_in_block,
-                                                 bool ends_row, bool ends_block, Sink& sink) {
-    const int L = (int)xs.L;
+__host__ __device__ inline void xspan_tokens_ref(const uint32_t c[4], uint32_t carry, const XSpan& xs, int L,
+                                                 bool first_in_block, bool ends_row, bool ends_block, Sink& sink) {
     const int nfull = (L - (ends_row ? 1 : 0)) / 4;
     const int nb = 2 * L - (ends_row ? 1 : 0);
     int prev_end = 0;
@@ -215,7 +215,7 @@ struct XArgs {
 
 constexpr int kXStage = 24;   // staged words per span: X spans carry the static separator mismatches on top of the data
 __host__ __device__ inline uint32_t x_smem_bytes(uint32_t nthr) {
-    return kATabWords * 4u + ((uint32_t)(kXStage + 2) * nthr + nthr + 24u) * 4u + 20u * nthr + 16u;
+    return kATabWords * 4u + ((uint32_t)(kXStage + 2) * nthr + nthr + 24u) * 4u + 20u * nthr + 32u * nthr + 16u;
 }
 
 // 32-bit mask of the non-zero nibbles of four words
@@ -234,7 +234,10 @@ __device__ __forceinline__ uint32_t nonzero_nibbles(const uint32_t x[4]) {
     return nz;
 }
 
-__global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
+#ifndef DNAF_X_REGS
+#define DNAF_X_REGS 56   // as k_auto: 7 blocks of 160 threads per SM, no spills
+#endif
+__global__ void __maxnreg__(DNAF_X_REGS) k_x(const XArgs a) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const uint32_t tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31u, wid = tid >> 5;
     uint32_t* s_len = reinterpret_cast<uint32_t*>(smem_raw);   // len_tok | lit | eob | hdr_bits | hdr
@@ -242,6 +245,7 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
     uint32_t* s_last2 = s_stage + (kXStage + 2) * nthr;
     uint32_t* s_misc = s_last2 + nthr;
     uint8_t* s_cp = reinterpret_cast<uint8_t*>(s_misc + 24);
+    uint32_t* s_sk6 = reinterpret_cast<uint32_t*>(s_cp + 20u * nthr);   // [8][nthr]: the span's XSpan::sk6, word-interleaved
     const uint32_t* s_lits = s_len + 264;
     const uint32_t* s_hdr = s_len + 274;
 
@@ -258,11 +262,6 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
         bulk_g2s(s_len, tb->len_tok, kATabWords * 4u, mbar);
     }
     if (tid == 6) { s_misc[16] = 0; s_misc[17] = 0; }
-    const bool starts_row = d.flags & 1u, ends_row = (d.flags >> 1) & 1u;
-    const uint64_t pb = a.nv.pre_off[d.row];
-    const uint32_t plen = starts_row ? (uint32_t)(a.nv.pre_off[d.row + 1] - pb) : 0u;
-    const uint32_t body0 = a.sv.xoff[d.cell0];
-    const uint32_t n = plen + (a.sv.xoff[d.cell0 + d.ncells] - body0);  // text bytes of this block
     const uint32_t nspans = (d.ncells + 63u) / 64u;
 
     // ---- draw this span's 128 slots (as k_auto), force the overrides, compact to the printed alleles
@@ -275,14 +274,14 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
         const uint64_t prow = a.row_base + d.row;
         const uint32_t r_lo = (uint32_t)prow, r_hi = (uint32_t)(prow >> 32);
         const uint32_t g0 = cs >> 4;
-        uint32_t eq[4], lt[4], valid[4];
+        uint32_t eq[4], lt[4];
 #pragma unroll
         for (int w = 0; w < 4; ++w) {
+            // slots beyond the last sample start out decided ("U <= T": reference allele, mask bit 0)
             const uint32_t g = g0 + w;
             const uint32_t slots = 32u * g < 2u * a.sv.n ? 2u * a.sv.n - 32u * g : 0u;
-            valid[w] = slots >= 32u ? 0xFFFFFFFFu : ((1u << slots) - 1u);
-            eq[w] = valid[w];
-            lt[w] = 0;
+            eq[w] = slots >= 32u ? 0xFFFFFFFFu : ((1u << slots) - 1u);
+            lt[w] = ~eq[w];
         }
 #pragma unroll
         for (uint32_t q = 0; q < 2; ++q)
@@ -305,7 +304,7 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
                 if (k == w) { eq[k] = e; lt[k] = l; }
         }
 #pragma unroll
-        for (int w = 0; w < 4; ++w) m[w] = ~(lt[w] | eq[w]) & valid[w];
+        for (int w = 0; w < 4; ++w) m[w] = ~(lt[w] | eq[w]);
     }
     if (nc > 0) {
         for (uint32_t o = 0; o < d.ovr_count; ++o) {
@@ -313,9 +312,9 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
             if (i >= cs && i < cs + (uint32_t)nc) {
                 const uint32_t j = 2u * (i - cs);
                 const uint32_t bit = 3u << (j & 31u);
+                // selects, not m[j >> 5]: an indexed m lives in local memory for the whole kernel
 #pragma unroll
-                for (int w = 0; w < 4; ++w)
-                    if ((j >> 5) == (uint32_t)w) m[w] |= bit;
+                for (int w = 0; w < 4; ++w) m[w] |= (j >> 5) == (uint32_t)w ? bit : 0u;
             }
         }
     }
@@ -346,6 +345,12 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
             for (int k = 0; k < 4; ++k) sp ^= __ldg(&a.etab[(4 * w + k) * 256 + ((mm[w] >> (8 * k)) & 0xFFu)]);
         crc = mul_tab(a.mspan + (size_t)(cs >> 6) * 1024u, sp);
     }
+    // the block's prefix and text length, needed from here on (loaded after the draws: fewer live registers there)
+    const bool starts_row = d.flags & 1u, ends_row = (d.flags >> 1) & 1u;
+    const uint64_t pb = a.nv.pre_off[d.row];
+    const uint32_t plen = starts_row ? (uint32_t)(a.nv.pre_off[d.row + 1] - pb) : 0u;
+    const uint32_t body0 = a.sv.xoff[d.cell0];
+    const uint32_t n = plen + (a.sv.xoff[d.cell0 + d.ncells] - body0);  // text bytes of this block
     uint32_t pre_tok = 0;
     if (tid < plen) pre_tok = __ldg(&tb->pre_lit[a.nv.prefix[pb + tid]]);
     if (tid == 0) {
@@ -389,6 +394,12 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
         uint32_t* dst = reinterpret_cast<uint32_t*>(s_cp + 20u * tid);
 #pragma unroll
         for (int k = 0; k < 5; ++k) dst[k] = q[k];
+        // the unit loop's separator keys come from shared memory: one global round trip here instead of one per unit
+        // in front of the dependent LUT load
+        const uint4* sk = reinterpret_cast<const uint4*>(xs->sk6);
+        const uint4 k0 = sk[0], k1 = sk[1];
+        s_sk6[0 * nthr + tid] = k0.x; s_sk6[1 * nthr + tid] = k0.y; s_sk6[2 * nthr + tid] = k0.z; s_sk6[3 * nthr + tid] = k0.w;
+        s_sk6[4 * nthr + tid] = k1.x; s_sk6[5 * nthr + tid] = k1.y; s_sk6[6 * nthr + tid] = k1.z; s_sk6[7 * nthr + tid] = k1.w;
         const uint32_t x[4] = {cpad[0] ^ q[0], cpad[1] ^ q[1], cpad[2] ^ q[2], cpad[3] ^ q[3]};
         nz = (nonzero_nibbles(x) | xs->snz) & (nfull >= 32 ? 0xFFFFFFFFu : ((1u << nfull) - 1u));
     }
@@ -398,6 +409,7 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
     ATokSink<AStageT<kXStage>> ts{st, s_len, s_lits, eob};
     if (worker) {
         const uint8_t* cpb = s_cp + 20u * tid;
+        auto sk6_at = [&](int u) { return (s_sk6[(u >> 2) * nthr + tid] >> (8 * (u & 3))) & 0xFFu; };
         const uint2* __restrict__ lut = tb->lut;
         int prev_end = 0;
         if (tid == 0) {   // first span of the block: unit 0 as eight literals
@@ -418,7 +430,8 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
             nz &= nz - 1u;
             const uint32_t v = (uint32_t)cpb[u >> 1] | ((uint32_t)cpb[(u >> 1) + 1] << 8);
             const uint32_t c6 = (v >> (4 * (u & 1))) & 63u;
-            const uint32_t key = c6 | ((uint32_t)xs->sk6[u] << 6);
+            const uint32_t s6 = sk6_at(u);
+            const uint32_t key = c6 | (s6 << 6);
             const uint2 e = __ldg(&lut[key]);
             const uint32_t nb = (e.y >> 11) & 63u;
             const int pos = 8 * u;
@@ -429,7 +442,7 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
             } else {
                 st.put64(t1 & 0xFFFFFFu, 0u, t1 >> 24);
                 int lead, lastp;
-                xunit_tokens(c6, (uint32_t)xs->sk6[u], ts, lead, lastp);
+                xunit_tokens(c6, s6, ts, lead, lastp);
             }
             prev_end = pos + (int)(e.y >> 28);
         }
@@ -439,7 +452,7 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
             const int k0 = 4 * nfull;
             const uint32_t vt = (uint32_t)cpb[nfull >> 1] | ((uint32_t)cpb[(nfull >> 1) + 1] << 8);
             const uint32_t c6 = (vt >> (4 * (nfull & 1))) & 63u;
-            const uint32_t s6 = nfull < 32 ? (uint32_t)xs->sk6[nfull] : (xs->sk[3] >> 30);
+            const uint32_t s6 = nfull < 32 ? sk6_at(nfull) : (xs->sk[3] >> 30);
             auto lit_at = [&](int q) {
                 const int j = (q >> 1) - k0 + 2;
                 if (q & 1) return s_lits[((s6 >> j) & 1u) ? kLitSlash : kLitTab];
@@ -561,9 +574,7 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
                 // some span overflowed its staging words: every span re-emits straight into the output words
                 AEmit em{words, dst};
                 ATokSink<AEmit> te{em, s_len, s_lits, eob};
-                XSpan xl = *xs;
-                xl.L = L;
-                xspan_tokens_ref(cpad, carry, xl, tid == 0, p_end, p_last, te);
+                xspan_tokens_ref(cpad, carry, *xs, (int)L, tid == 0, p_end, p_last, te);
             }
         }
         out_payload = payload;
@@ -588,9 +599,9 @@ __global__ void __launch_bounds__(kFusedMaxThreads, 4) k_x(const XArgs a) {
     if (tid < 26) {
         const uint32_t crc32 = ~s_misc[16];
         const uint32_t bsize = out_payload + 25u;
-        if (tid < 16) {
-            const uint8_t head[16] = {0x1f, 0x8b, 0x08, 0x04, 0, 0, 0, 0, 0, 0xff, 0x06, 0x00, 0x42, 0x43, 0x02, 0x00};
-            blk[tid] = head[tid];
+        if (tid < 16) {   // 1f 8b 08 04 | 00 00 00 00 | 00 ff 06 00 | 42 43 02 00, from words (an indexed byte array is local memory)
+            const uint32_t hw = tid < 4u ? 0x04088b1fu : (tid < 8u ? 0u : (tid < 12u ? 0x0006ff00u : 0x00024342u));
+            blk[tid] = (uint8_t)(hw >> (8u * (tid & 3u)));
         } else if (tid < 18) {
             blk[tid] = (uint8_t)(bsize >> (8 * (tid - 16)));
         } else if (tid < 22) {
