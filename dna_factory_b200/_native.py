@@ -42,7 +42,7 @@ EXPORTS = ["dnaf_abi_version", "dnaf_device_count", "dnaf_last_error", "dnaf_cre
            "dnaf_text", "dnaf_bgzf_compress", "dnaf_bgzf_bound", "dnaf_bgzf_eof", "dnaf_bgzf_scan", "dnaf_block_log",
            "dnaf_block_log_get", "dnaf_select_snps", "dnaf_parse_snps_jsonl", "dnaf_format_prefixes",
            "dnaf_format_snps_jsonl", "dnaf_debug_lz_block", "dnaf_generate_bed", "dnaf_generate_bed_fd_at",
-           "dnaf_generate_bed_device"]
+           "dnaf_generate_bed_device", "dnaf_allele_counts", "dnaf_allele_counts_device", "dnaf_format_assoc"]
 
 _lib = None
 
@@ -84,6 +84,10 @@ def load():
         "dnaf_generate_bed": (i32, [vp, u64, u64, u64, u8p, u64, sp]),
         "dnaf_generate_bed_fd_at": (i32, [vp, u64, u64, u64, i32, u64, sp]),
         "dnaf_generate_bed_device": (i32, [vp, u64, u64, u64, sp]),
+        "dnaf_allele_counts": (i32, [vp, u64, u64, u64, u32p, sp]),
+        "dnaf_allele_counts_device": (i32, [vp, u64, u64, u64, sp]),
+        "dnaf_format_assoc": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64),
+                                    ctypes.POINTER(ctypes.c_int64), u8p, u8p, u32p, u8p]),
         "dnaf_genotypes": (i32, [vp, u64, u64, u64, u8p, u64]),
         "dnaf_text": (i32, [vp, u64, u64, u64, u8p, u64, u64p]),
         "dnaf_bgzf_compress": (i32, [vp, u8p, u64, u8p, u64, sp]),
@@ -326,6 +330,26 @@ class Engine:
         self._check(self._lib.dnaf_generate_bed_device(self._h, row_begin, row_end, seed, ctypes.byref(st)))
         return st.as_dict()
 
+    # -- case/control allele counts (the allelic association test, pop_factory --assoc)
+    def allele_counts(self, row_begin, row_end, seed):
+        """uint32[rows, 4] of rows [row_begin,row_end): ALT in cases, observed in cases, ALT in controls, observed in
+        controls (counting rule: include/dnaf_b200.h, dnaf_allele_counts)."""
+        return self.allele_counts_stats(row_begin, row_end, seed)[0]
+
+    def allele_counts_stats(self, row_begin, row_end, seed):
+        """Same counts -> (counts, stats dict)."""
+        out = np.zeros((max(row_end - row_begin, 0), 4), np.uint32)
+        st = Stats()
+        self._check(self._lib.dnaf_allele_counts(self._h, row_begin, row_end, seed,
+                                                 out.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)), ctypes.byref(st)))
+        return out, st.as_dict()
+
+    def allele_counts_device(self, row_begin, row_end, seed):
+        """Same work, counts left on the device; returns stats dict."""
+        st = Stats()
+        self._check(self._lib.dnaf_allele_counts_device(self._h, row_begin, row_end, seed, ctypes.byref(st)))
+        return st.as_dict()
+
     # -- parity gates
     def genotypes(self, row_begin, row_end, seed):
         rows = row_end - row_begin
@@ -438,6 +462,27 @@ def format_snps_jsonl(ids, chrom_idx, labels, position, n_alleles, nts, cum):
     used = lib.dnaf_format_snps_jsonl(n, ci.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), _label_block(labels),
                                       pos.ctypes.data_as(i64p), ids.ctypes.data_as(i64p), _u8(k), _u8(nt),
                                       ridx.ctypes.data_as(u32p), b"".join(strs), roff.ctypes.data_as(u32p), _u8(out))
+    return out[:used].tobytes()
+
+
+def format_assoc(ids, chrom_idx, labels, position, n_alleles, nts, counts):
+    """.assoc body lines (dnaf_format_assoc: F_A, F_U, CHISQ, P, OR in double, "%.4g", NA rules) of a column-form SNP
+    table and its uint32[rows, 4] allele counts -> bytes."""
+    lib = load()
+    n = len(ids)
+    if n == 0:
+        return b""
+    ids = np.ascontiguousarray(ids, np.int64)
+    pos = np.ascontiguousarray(position, np.int64)
+    ci = np.ascontiguousarray(chrom_idx, np.int32)
+    k = np.ascontiguousarray(n_alleles, np.uint8)
+    nt = np.ascontiguousarray(nts, np.uint8).reshape(n, KMAX)
+    cnt = np.ascontiguousarray(counts, np.uint32).reshape(n, 4)
+    out = np.empty(n * 192 + 16, np.uint8)
+    i64p = ctypes.POINTER(ctypes.c_int64)
+    used = lib.dnaf_format_assoc(n, ci.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), _label_block(labels),
+                                 ids.ctypes.data_as(i64p), pos.ctypes.data_as(i64p), _u8(nt), _u8(k),
+                                 cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)), _u8(out))
     return out[:used].tobytes()
 
 

@@ -7,7 +7,8 @@
 // Work is cut into passes of at most `chunk_bytes` of uncompressed text; each pass is
 //   sample -> (overrides) -> format -> BGZF encode -> scan -> compact -> D2H -> sink      (generic path)
 // or the fused kernel (k_fused.cuh) followed by scan -> compact -> D2H -> sink.  The PLINK 1 .bed writer
-// (dnaf_generate_bed*) is one kernel per pass, k_bed -> D2H -> sink (host_bed.h).
+// (dnaf_generate_bed*) is one kernel per pass, k_bed -> D2H -> sink (host_bed.h); the case/control allele counts
+// (dnaf_allele_counts*) are one kernel per pass too, k_assoc -> D2H (host_assoc.h).
 #include <unistd.h>
 
 #include <algorithm>
@@ -24,6 +25,7 @@
 #include "../../include/dnaf_b200.h"
 #include "dnaf_device.cuh"
 #include "fused_host.h"
+#include "k_assoc.cuh"
 #include "k_bed.cuh"
 #include "k_deflate.cuh"
 #include "k_fused.cuh"
@@ -43,6 +45,7 @@ using namespace dnaf;
 #include "host_sink.h"
 #include "host_passes.h"
 #include "host_bed.h"
+#include "host_assoc.h"
 
 
 // ================================================================================================ C ABI
@@ -221,6 +224,11 @@ int dnaf_set_samples(dnaf_ctx* c, uint32_t n, const uint8_t* sex, const uint8_t*
     {   // k_bed: which cells of a 16-sample group are male / female (haploid on X and Y, missing on Y)
         const std::vector<uint32_t> m = bed_sex_masks(sex, n);
         rc = upload(c, c->d_sexmask, m.data(), m.size());
+        if (rc) return rc;
+    }
+    {   // k_assoc: which cells of a 16-sample group are cases
+        const std::vector<uint32_t> m = assoc_case_masks(is_control, n);
+        rc = upload(c, c->d_casemask, m.data(), m.size());
         if (rc) return rc;
     }
     {   // X rows: the sample that holds body byte 256*k (for k_fused_text)
@@ -590,6 +598,22 @@ int dnaf_generate_bed_device(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, 
     Sink s;
     s.device_only = true;
     return bed_impl(c, row_begin, row_end, seed, s, stats);
+}
+
+int dnaf_allele_counts(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* counts, dnaf_stats* stats) {
+    if (!c) return DNAF_E_ARG;
+    if (!counts && row_end > row_begin) return fail(c, DNAF_E_ARG, "counts is NULL");
+    return assoc_impl(c, row_begin, row_end, seed, counts, stats);
+}
+
+int dnaf_allele_counts_device(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, dnaf_stats* stats) {
+    return assoc_impl(c, row_begin, row_end, seed, nullptr, stats);
+}
+
+uint64_t dnaf_format_assoc(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const int64_t* position,
+                           const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, char* out) {
+    if (!n || !chrom_idx || !labels || !ids || !position || !nts || !n_alleles || !counts || !out) return 0;
+    return assocfmt::lines(n, chrom_idx, labels, ids, position, nts, n_alleles, counts, out);
 }
 
 int dnaf_genotypes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out, uint64_t cap) {

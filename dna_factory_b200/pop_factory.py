@@ -26,7 +26,7 @@ from datetime import datetime
 
 import numpy
 
-from . import _native, partition, host
+from . import _native, assoc, partition, host
 from . import tabix
 from .tabix import TabixBuilder
 from .snp import (CHROMOSOME_LIST, CHROMOSOME_MAX_POSITION, CHROMOSOME_PROB, SNPTuples, SnpFactory, SnpTable,  # noqa: F401
@@ -38,15 +38,29 @@ OUTPUT_DIR = os.path.join(os.getcwd(), "populations")
 BED_MAGIC = b"\x6c\x1b\x01"     # PLINK 1 .bed, SNP-major
 
 
-def validate_bed_table(table):
-    """--bed needs a column-form SNP table (SnpTable) without rows of more than 2 alleles: checked before the VCF is
-    written, so a table PLINK 1 cannot hold fails at once instead of after the whole generation."""
+def validate_biallelic_table(table, flag, what):
+    """`flag` needs a column-form SNP table (SnpTable) without rows of more than 2 alleles: checked before the VCF is
+    written, so a table the output cannot hold fails at once instead of after the whole generation."""
     if not isinstance(table, SnpTable):
-        raise ValueError("--bed needs SNP records that fit the column form (integer ids, one-letter alleles)")
+        raise ValueError("%s needs SNP records that fit the column form (integer ids, one-letter alleles)" % flag)
     bad = numpy.nonzero(table.n_alleles > 2)[0]
     if len(bad):
-        raise ValueError("--bed: SNP rs%d (row %d) has %d alleles; PLINK 1 .bed / .bim hold biallelic SNPs only" % (
-            int(table.ids[bad[0]]), int(bad[0]), int(table.n_alleles[bad[0]])))
+        raise ValueError("%s: SNP rs%d (row %d) has %d alleles; %s" % (
+            flag, int(table.ids[bad[0]]), int(bad[0]), int(table.n_alleles[bad[0]]), what))
+
+
+def validate_bed_table(table):
+    validate_biallelic_table(table, "--bed", "PLINK 1 .bed / .bim hold biallelic SNPs only")
+
+
+def validate_assoc_table(table):
+    validate_biallelic_table(table, "--assoc", "the allelic test counts biallelic SNPs only")
+
+
+def validate_assoc_population(control_size, test_size):
+    """--assoc compares cases with controls: both groups must be non-empty."""
+    if control_size <= 0 or test_size <= 0:
+        raise ValueError("--assoc needs cases and controls (-s %d, -c %d)" % (test_size, control_size))
 
 
 def gen_vcf_header(fam_data):
@@ -191,7 +205,7 @@ class DeleteriousGroup:
 class PopulationFactory:
     def __init__(self, num_processes=1, generate_snps=False, male_odds=0.5, deleterious_config=None,
                  deleterious_list_path=None, sample_id_offset=0, snps_path=None, output_path=None, seed=None,
-                 gpus=1, gpu_select=False, tbi=False, bed=False):
+                 gpus=1, gpu_select=False, tbi=False, bed=False, assoc=False):
         self.deleterious = {}
         self.ordered_snps = []
         self.snp_table = None
@@ -214,10 +228,15 @@ class PopulationFactory:
         self.bed = bool(bed)
         self.stats = []
         self.bed_stats = []      # dnaf_stats of the .bed calls (--bed)
+        self.assoc = bool(assoc)
+        self.assoc_counts = None     # uint32[rows, 4] allele counts of the last write_vcf_snps (--assoc)
+        self.override_rows = None    # global row of every override pair of the last write_vcf_snps
 
     # ------------------------------------------------------------------------------------------ orchestration
     def generate_population(self, control_size, test_size, min_freq, max_snps, compression_level=6):
         t0 = time.time()
+        if self.assoc:
+            validate_assoc_population(control_size, test_size)
         clock_seed = int(datetime.now().strftime("%H%M%S"))
         numpy.random.seed(clock_seed)
         if self.seed is None:
@@ -313,6 +332,8 @@ class PopulationFactory:
         snps = self.snp_table if self.snp_table is not None else self.ordered_snps
         if self.bed:
             validate_bed_table(snps)
+        if self.assoc:
+            validate_assoc_table(snps)
         groups = PopulationFactory.pick_deleterious_groups(list(self.deleterious.values()), test_size)
         fam_data = self.generate_fam_file(control_size, test_size, male_odds, groups)
         main_file = self.population_dir + "population.vcf.gz"
@@ -339,17 +360,30 @@ class PopulationFactory:
             if self.bed:
                 with open(self.population_dir + "population.bim", "wb") as b:
                     b.write(snps.bim_bytes())
+            if self.assoc:
+                self.output_assoc(snps)
         finally:
             engine.close()
             if bed_fd is not None:
                 os.close(bed_fd)
         print("Finished VCF file output.", flush=True)
 
+    def output_assoc(self, table):
+        """population.assoc (the allelic test of every SNP) and deleterious_assoc.txt (how the planted SNPs fare) from
+        the allele counts write_vcf_snps took on the GPU."""
+        with open(self.population_dir + "population.assoc", "wb") as f:
+            f.write(assoc.assoc_bytes(table, self.assoc_counts))
+        text, summary = assoc.deleterious_report(table, self.deleterious, self.assoc_counts, self.override_rows)
+        with open(self.population_dir + "deleterious_assoc.txt", "wb") as f:
+            f.write(text)
+        print(summary, flush=True)
+
     # ------------------------------------------------------------------------------------------ the GPU seam
     def write_vcf_snps(self, fam_data, snps, file, engine=None, bed_fd=None):
         """Rows of `snps` (in order) for `fam_data`, appended to `file` -- the reference's seam
         (pop_factory.py:417-469).  `snps` is a list of SNPTuples or a SnpTable; `file` a BgzfSink.  With `bed_fd`
-        (an open population.bed that holds the 3 magic bytes) the same rows also go there as PLINK 1 .bed rows."""
+        (an open population.bed that holds the 3 magic bytes) the same rows also go there as PLINK 1 .bed rows.  With
+        --assoc the case/control allele counts of the same rows land in self.assoc_counts."""
         t0 = time.time()
         level = getattr(file, "compresslevel", getattr(self, "_level", 6))
         seed = self.seed if self.seed is not None else int(datetime.now().strftime("%H%M%S"))
@@ -362,6 +396,7 @@ class PopulationFactory:
             orow, osamp = host.override_pairs_table(fam_data, snps)
         else:
             orow, osamp = host.override_pairs(fam_data, snps)
+        self.override_rows = orow
         gpus = min(self.gpus, max(1, n_rows))
         index = getattr(file, "index", None)
         if index is not None:
@@ -386,6 +421,8 @@ class PopulationFactory:
                     eng.block_log(False)
                 if bed_fd is not None:
                     self.bed_stats.append(eng.generate_bed_fd_at(0, n_rows, seed, bed_fd, len(BED_MAGIC)))
+                if self.assoc:
+                    self.assoc_counts = eng.allele_counts(0, n_rows, seed)
             finally:
                 if own:
                     eng.close()
@@ -401,12 +438,14 @@ class PopulationFactory:
         gives every rank its offset in population.vcf.gz, and then all ranks pwrite() their streams side by side --
         nothing is spooled or copied twice.  Every rank holds only its own slice of the SNP table; the Philox row
         counter of its local row r is bounds[g] + r (dnaf_set_row_base).  .bed rows have a fixed size, so rank g
-        pwrite()s its rows at 3 + bounds[g] * ceil(N/4) of population.bed without a sizing pass."""
+        pwrite()s its rows at 3 + bounds[g] * ceil(N/4) of population.bed without a sizing pass.  With --assoc every
+        rank counts its own rows after its VCF write; the slices are joined in rank order."""
         bounds = partition.row_bounds(n_rows, gpus)
         n_dev = max(1, _native.device_count())      # more ranks than devices: ranks share devices round-robin
         errors = []
         index = getattr(file, "index", None)
         blocks, row_off, sizes, engines = [None] * gpus, [None] * gpus, [0] * gpus, [None] * gpus
+        counts = [None] * gpus
         barrier = threading.Barrier(gpus)
         file.flush()   # the header blocks must be in the file: the ranks write behind them
         base = file._handle.tell()
@@ -444,6 +483,8 @@ class PopulationFactory:
                     self.bed_stats.append(eng.generate_bed_fd_at(0, hi - lo, seed, bed_fd, len(BED_MAGIC) + lo * eng.bed_pitch()))
                 if index is not None:
                     blocks[g] = eng.block_log_get()
+                if self.assoc:
+                    counts[g] = eng.allele_counts(0, hi - lo, seed)
             except BaseException as e:  # noqa
                 errors.append(e)
 
@@ -458,6 +499,8 @@ class PopulationFactory:
         if errors:
             raise errors[0]
         file._handle.seek(base + sum(sizes))      # the sink appends the EOF block behind the last rank's stream
+        if self.assoc:
+            self.assoc_counts = numpy.concatenate(counts)
         if index is not None:
             off = numpy.concatenate([numpy.zeros(1, numpy.uint64)] +
                                     [r[1:] + numpy.uint64(sum(int(q[-1]) for q in row_off[:g])) for g, r in enumerate(row_off)])
@@ -527,6 +570,9 @@ def parse_cmd_args(args):
     ap.add_argument("--bed", action="store_true",
                     help="also write population.bed / population.bim (PLINK 1 binary fileset beside population.fam, "
                          "A1 = ALT); every SNP must be biallelic")
+    ap.add_argument("--assoc", action="store_true",
+                    help="also write population.assoc (case/control allelic test of every SNP, counted on the GPU) and "
+                         "deleterious_assoc.txt (rank of every planted deleterious SNP); every SNP must be biallelic")
     return ap.parse_args(args)
 
 
@@ -539,7 +585,7 @@ def main(sys_args):
                                 deleterious_list_path=args.deleterious_file, sample_id_offset=args.offset,
                                 male_odds=args.male_odds, deleterious_config=args.deleterious_config,
                                 snps_path=args.snps_file, output_path=args.outdir, seed=args.seed, gpus=args.gpus,
-                                gpu_select=args.gpu_select, tbi=args.tbi, bed=args.bed)
+                                gpu_select=args.gpu_select, tbi=args.tbi, bed=args.bed, assoc=args.assoc)
     factory.generate_population(args.control_size, args.size, args.min_freq, args.max_snps, args.compression_level)
 
 

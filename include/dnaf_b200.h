@@ -208,6 +208,33 @@ int dnaf_generate_bed_fd_at(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end,
 /* Same work, output left in device memory: kernel-only timing. */
 int dnaf_generate_bed_device(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, dnaf_stats* stats);
 
+/*
+ * Case/control allele counts of rows [row_begin,row_end), the input of the 1-df allelic association test (plink
+ * --assoc): the same draws, forced minors and ploidy rules as the VCF and .bed rows of the same seed.  counts is
+ * [rows][4]: ALT alleles in cases, alleles observed in cases, ALT alleles in controls, alleles observed in controls
+ * (cases: is_control[i] == 0 in dnaf_set_samples).  Every allele the VCF text prints counts once: autosome rows count
+ * both slots of every sample; X rows slot 0 of males and both slots of females; Y rows slot 0 of males and nothing of
+ * females ('.'); MT rows slot 0 of every sample.  A forced minor counts as ALT on every counted slot of its cell.  Rows
+ * with more than 2 alleles: DNAF_E_INPUT before any GPU work, naming the row; K = 1 rows count ALT only where a minor
+ * is forced.  stats: rows, calls, kernel_launches, ms_sample (the counting kernel), ms_total; the other fields are 0.
+ */
+int dnaf_allele_counts(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* counts,
+                       dnaf_stats* stats);
+/* Same work, counts left in device memory: kernel-only timing. */
+int dnaf_allele_counts_device(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, dnaf_stats* stats);
+/*
+ * The .assoc body lines of n rows from their counts (host code, no context, no GPU; `labels` = 8 bytes per chromosome
+ * label, nts = [n][DNAF_KMAX]).  With a = ALT and b = REF alleles in cases, c / d the same in controls:
+ *   F_A = a/(a+b), F_U = c/(c+d), CHISQ = n(ad-bc)^2 / ((a+b)(c+d)(a+c)(b+d)) (no continuity correction),
+ *   P = erfc(sqrt(CHISQ/2)), OR = ad/(bc); "NA" where a denominator is 0; values printed with "%.4g" in double.
+ * Columns CHR SNP BP A1 F_A F_U A2 CHISQ P OR, right-aligned, one space apart; CHR is the label with X, Y, MT written
+ * 23, 24, 26; SNP is rs<id>; A1 = ALT ('0' for one-allele rows) and A2 = REF, as in the .bim.  `out` holds at least
+ * 192 bytes per row.  Returns the bytes written.
+ */
+uint64_t dnaf_format_assoc(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
+                           const int64_t* position, const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts,
+                           char* out);
+
 /* Parity gates. genotypes: out[(r*n_samples+i)*2+s] = allele index, 0xFF where the cell has no such
  * allele (second slot of a haploid cell, both slots of '.').  text: the uncompressed rows. */
 int dnaf_genotypes(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out,
