@@ -42,7 +42,8 @@ EXPORTS = ["dnaf_abi_version", "dnaf_device_count", "dnaf_last_error", "dnaf_cre
            "dnaf_text", "dnaf_bgzf_compress", "dnaf_bgzf_bound", "dnaf_bgzf_eof", "dnaf_bgzf_scan", "dnaf_block_log",
            "dnaf_block_log_get", "dnaf_select_snps", "dnaf_parse_snps_jsonl", "dnaf_format_prefixes",
            "dnaf_format_snps_jsonl", "dnaf_debug_lz_block", "dnaf_generate_bed", "dnaf_generate_bed_fd_at",
-           "dnaf_generate_bed_device", "dnaf_allele_counts", "dnaf_allele_counts_device", "dnaf_format_assoc"]
+           "dnaf_generate_bed_device", "dnaf_allele_counts", "dnaf_allele_counts_device", "dnaf_format_assoc",
+           "dnaf_genotype_counts", "dnaf_genotype_counts_device", "dnaf_hwe_exact", "dnaf_format_model", "dnaf_format_hardy"]
 
 _lib = None
 
@@ -88,6 +89,13 @@ def load():
         "dnaf_allele_counts_device": (i32, [vp, u64, u64, u64, sp]),
         "dnaf_format_assoc": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64),
                                     ctypes.POINTER(ctypes.c_int64), u8p, u8p, u32p, u8p]),
+        "dnaf_genotype_counts": (i32, [vp, u64, u64, u64, u32p, f64p, sp]),
+        "dnaf_genotype_counts_device": (i32, [vp, u64, u64, u64, i32, sp]),
+        "dnaf_hwe_exact": (i32, [vp, u64, u32p, f64p]),
+        "dnaf_format_model": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64),
+                                    u8p, u8p, u32p, u8p]),
+        "dnaf_format_hardy": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64),
+                                    u8p, u8p, u32p, f64p, u8p]),
         "dnaf_genotypes": (i32, [vp, u64, u64, u64, u8p, u64]),
         "dnaf_text": (i32, [vp, u64, u64, u64, u8p, u64, u64p]),
         "dnaf_bgzf_compress": (i32, [vp, u8p, u64, u8p, u64, sp]),
@@ -350,6 +358,39 @@ class Engine:
         self._check(self._lib.dnaf_allele_counts_device(self._h, row_begin, row_end, seed, ctypes.byref(st)))
         return st.as_dict()
 
+    # -- case/control genotype counts and Hardy-Weinberg exact tests (pop_factory --model / --hardy)
+    def genotype_counts(self, row_begin, row_end, seed, hwe=True):
+        """(uint32[rows, 10], float64[rows, 3] or None) of rows [row_begin,row_end): per row dip, het, hom, hap, hap_alt
+        of the cases, then of the controls, and the Hardy-Weinberg exact P of ALL, AFF, UNAFF (counting rule and test:
+        include/dnaf_b200.h, dnaf_genotype_counts)."""
+        return self.genotype_counts_stats(row_begin, row_end, seed, hwe)[:2]
+
+    def genotype_counts_stats(self, row_begin, row_end, seed, hwe=True):
+        """Same -> (counts, P or None, stats dict)."""
+        rows = max(row_end - row_begin, 0)
+        out = np.zeros((rows, 10), np.uint32)
+        p = np.zeros((rows, 3), np.float64) if hwe else None
+        st = Stats()
+        self._check(self._lib.dnaf_genotype_counts(
+            self._h, row_begin, row_end, seed, out.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
+            p.ctypes.data_as(ctypes.POINTER(ctypes.c_double)) if hwe else None, ctypes.byref(st)))
+        return out, p, st.as_dict()
+
+    def genotype_counts_device(self, row_begin, row_end, seed, hwe=True):
+        """Same work, results left on the device; returns stats dict."""
+        st = Stats()
+        self._check(self._lib.dnaf_genotype_counts_device(self._h, row_begin, row_end, seed, int(bool(hwe)), ctypes.byref(st)))
+        return st.as_dict()
+
+    def hwe_exact(self, geno):
+        """float64[n]: the Hardy-Weinberg exact P of every (n11, n12, n22) row of `geno`, computed by the device kernel
+        (dnaf_hwe_exact)."""
+        g = np.ascontiguousarray(geno, np.uint32).reshape(-1, 3)
+        p = np.zeros(len(g), np.float64)
+        self._check(self._lib.dnaf_hwe_exact(self._h, len(g), g.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
+                                             p.ctypes.data_as(ctypes.POINTER(ctypes.c_double))))
+        return p
+
     # -- parity gates
     def genotypes(self, row_begin, row_end, seed):
         rows = row_end - row_begin
@@ -483,6 +524,45 @@ def format_assoc(ids, chrom_idx, labels, position, n_alleles, nts, counts):
     used = lib.dnaf_format_assoc(n, ci.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), _label_block(labels),
                                  ids.ctypes.data_as(i64p), pos.ctypes.data_as(i64p), _u8(nt), _u8(k),
                                  cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)), _u8(out))
+    return out[:used].tobytes()
+
+
+def _geno_columns(ids, chrom_idx, labels, n_alleles, nts, counts):
+    n = len(ids)
+    return (np.ascontiguousarray(ids, np.int64), np.ascontiguousarray(chrom_idx, np.int32), _label_block(labels),
+            np.ascontiguousarray(n_alleles, np.uint8), np.ascontiguousarray(nts, np.uint8).reshape(n, KMAX),
+            np.ascontiguousarray(counts, np.uint32).reshape(n, 10))
+
+
+def format_model(ids, chrom_idx, labels, n_alleles, nts, counts):
+    """.model body lines (dnaf_format_model: GENO, TREND, ALLELIC, DOM, REC per SNP) of a column-form SNP table and its
+    uint32[rows, 10] genotype counts -> bytes."""
+    lib = load()
+    n = len(ids)
+    if n == 0:
+        return b""
+    ids, ci, lab, k, nt, cnt = _geno_columns(ids, chrom_idx, labels, n_alleles, nts, counts)
+    out = np.empty(n * 960 + 16, np.uint8)
+    used = lib.dnaf_format_model(n, ci.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), lab,
+                                 ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _u8(nt), _u8(k),
+                                 cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)), _u8(out))
+    return out[:used].tobytes()
+
+
+def format_hardy(ids, chrom_idx, labels, n_alleles, nts, counts, hwe_p):
+    """.hwe body lines (dnaf_format_hardy: ALL, AFF, UNAFF per SNP) of a column-form SNP table, its uint32[rows, 10]
+    genotype counts and float64[rows, 3] exact-test P -> bytes."""
+    lib = load()
+    n = len(ids)
+    if n == 0:
+        return b""
+    ids, ci, lab, k, nt, cnt = _geno_columns(ids, chrom_idx, labels, n_alleles, nts, counts)
+    p = np.ascontiguousarray(hwe_p, np.float64).reshape(n, 3)
+    out = np.empty(n * 576 + 16, np.uint8)
+    used = lib.dnaf_format_hardy(n, ci.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), lab,
+                                 ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _u8(nt), _u8(k),
+                                 cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
+                                 p.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), _u8(out))
     return out[:used].tobytes()
 
 

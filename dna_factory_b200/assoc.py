@@ -54,38 +54,56 @@ def _g(v):
     return "NA" if v is None else "%.4g" % v
 
 
+def planted_rows(table, groups, orow):
+    """(group name, SNP id, weight, row or None, forced) of every (group, planted SNP), in the groups' order.
+
+    groups: {name: DeleteriousGroup}.  orow: the global row of every override pair (host.override_pairs*), so `forced`
+    is the number of cases whose minor allele was forced on that row.  A key of a --deleterious_file replay is a string,
+    which forces nothing upstream either (SURVEY R8): it still finds its row through int(key), with forced 0.  row is
+    None for an id the table does not hold."""
+    S = len(table)
+    forced = np.bincount(np.asarray(orow, np.int64), minlength=S) if len(orow) else np.zeros(S, np.int64)
+    ids = np.asarray(table.ids, np.int64)
+    order = np.argsort(ids, kind="stable")
+    for name, group in groups.items():
+        for key, weight in group.deleterious.items():
+            snp_id = int(key)
+            j = int(np.searchsorted(ids[order], snp_id))
+            if j >= S or ids[order[j]] != snp_id:
+                yield name, snp_id, weight, None, 0
+            else:
+                r = int(order[j])
+                yield name, snp_id, weight, r, int(forced[r])
+
+
+def rank_of(tested, x):
+    """1 + the number of values of the sorted array `tested` above x; behind all of them when x is None (NA)."""
+    return len(tested) + 1 if x is None else 1 + len(tested) - int(np.searchsorted(tested, x, side="right"))
+
+
 def deleterious_report(table, groups, counts, orow):
     """deleterious_assoc.txt text and its one-line summary.
 
-    groups: {name: DeleteriousGroup}; every (group, planted SNP id) gives one line.  orow: the global row of every
-    override pair (host.override_pairs*), so FORCED is the number of cases whose minor allele was forced on that row.
-    A key of a --deleterious_file replay is a string, which forces nothing upstream either (SURVEY R8): the line still
-    finds its row through int(key) and shows FORCED 0.  RANK is 1 + the rows with a larger CHISQ (ranked by CHISQ, not
-    P, which underflows to 0 for strong effects); a row whose CHISQ is NA ranks behind every tested row.
+    One line per (group, planted SNP) (planted_rows): FORCED is the number of cases whose minor allele was forced on
+    that row.  RANK is 1 + the rows with a larger CHISQ (ranked by CHISQ, not P, which underflows to 0 for strong
+    effects); a row whose CHISQ is NA ranks behind every tested row.
     -> (text bytes, summary str)."""
     counts = np.asarray(counts, np.uint32).reshape(-1, 4)
     S = len(table)
     x2 = chisq(counts)
     tested = np.sort(x2[~np.isnan(x2)])
-    forced = np.bincount(np.asarray(orow, np.int64), minlength=S) if len(orow) else np.zeros(S, np.int64)
-    ids = np.asarray(table.ids, np.int64)
-    order = np.argsort(ids, kind="stable")
     lines = ["\t".join(REPORT_COLUMNS)]
     planted = hits = 0
     alpha = 0.05 / max(S, 1)
-    for name, group in groups.items():
-        for key, weight in group.deleterious.items():
-            planted += 1
-            snp_id = int(key)
-            j = int(np.searchsorted(ids[order], snp_id))
-            if j >= S or ids[order[j]] != snp_id:
-                lines.append("\t".join([name, "rs%d" % snp_id, "NA", "NA", "%g" % weight, "0"] + ["NA"] * 6))
-                continue
-            r = int(order[j])
-            f_a, f_u, x, p, odds = row_stats(*counts[r])
-            rank = len(tested) + 1 if x is None else 1 + len(tested) - int(np.searchsorted(tested, x, side="right"))
-            hits += p is not None and p < alpha
-            lines.append("\t".join([name, "rs%d" % snp_id, table.chrom_labels[table.chrom_idx[r]], "%d" % table.position[r],
-                                    "%g" % weight, "%d" % forced[r], _g(f_a), _g(f_u), _g(x), _g(p), _g(odds), "%d" % rank]))
+    for name, snp_id, weight, r, forced in planted_rows(table, groups, orow):
+        planted += 1
+        if r is None:
+            lines.append("\t".join([name, "rs%d" % snp_id, "NA", "NA", "%g" % weight, "0"] + ["NA"] * 6))
+            continue
+        f_a, f_u, x, p, odds = row_stats(*counts[r])
+        hits += p is not None and p < alpha
+        lines.append("\t".join([name, "rs%d" % snp_id, table.chrom_labels[table.chrom_idx[r]], "%d" % table.position[r],
+                                "%g" % weight, "%d" % forced, _g(f_a), _g(f_u), _g(x), _g(p), _g(odds),
+                                "%d" % rank_of(tested, x)]))
     summary = "%d of %d planted deleterious SNPs pass P < 0.05 / %d = %.3g" % (hits, planted, S, alpha)
     return ("\n".join(lines) + "\n").encode(), summary

@@ -8,7 +8,8 @@
 //   sample -> (overrides) -> format -> BGZF encode -> scan -> compact -> D2H -> sink      (generic path)
 // or the fused kernel (k_fused.cuh) followed by scan -> compact -> D2H -> sink.  The PLINK 1 .bed writer
 // (dnaf_generate_bed*) is one kernel per pass, k_bed -> D2H -> sink (host_bed.h); the case/control allele counts
-// (dnaf_allele_counts*) are one kernel per pass too, k_assoc -> D2H (host_assoc.h).
+// (dnaf_allele_counts*) are one kernel per pass too, k_assoc -> D2H (host_assoc.h), and the genotype counts
+// (dnaf_genotype_counts*) k_geno -> (k_hwe) -> D2H through the same pass driver (host_geno.h).
 #include <unistd.h>
 
 #include <algorithm>
@@ -30,6 +31,7 @@
 #include "k_deflate.cuh"
 #include "k_fused.cuh"
 #include "k_fused_text.cuh"
+#include "k_geno.cuh"
 #include "k_sample_format.cuh"
 #include "k_select.cuh"
 #include "snps_json.h"
@@ -46,6 +48,7 @@ using namespace dnaf;
 #include "host_passes.h"
 #include "host_bed.h"
 #include "host_assoc.h"
+#include "host_geno.h"
 
 
 // ================================================================================================ C ABI
@@ -614,6 +617,42 @@ uint64_t dnaf_format_assoc(uint64_t n, const int32_t* chrom_idx, const char* lab
                            const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, char* out) {
     if (!n || !chrom_idx || !labels || !ids || !position || !nts || !n_alleles || !counts || !out) return 0;
     return assocfmt::lines(n, chrom_idx, labels, ids, position, nts, n_alleles, counts, out);
+}
+
+int dnaf_genotype_counts(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* counts, double* hwe_p,
+                         dnaf_stats* stats) {
+    if (!c) return DNAF_E_ARG;
+    if (!counts && row_end > row_begin) return fail(c, DNAF_E_ARG, "counts is NULL");
+    return geno_impl(c, row_begin, row_end, seed, counts, hwe_p, hwe_p != nullptr, stats);
+}
+
+int dnaf_genotype_counts_device(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, int with_hwe,
+                                dnaf_stats* stats) {
+    return geno_impl(c, row_begin, row_end, seed, nullptr, nullptr, with_hwe != 0, stats);
+}
+
+int dnaf_hwe_exact(dnaf_ctx* c, uint64_t n, const uint32_t* geno, double* p) {
+    if (!c) return DNAF_E_ARG;
+    if (n && (!geno || !p)) return fail(c, DNAF_E_ARG, "geno / p is NULL");
+    const int rc = hwe_exact_impl(c, n, geno, p);
+    if (rc) quiesce(c);
+    return rc;
+}
+
+uint64_t dnaf_format_model(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const uint8_t* nts,
+                           const uint8_t* n_alleles, const uint32_t* counts, char* out) {
+    if (!n || !chrom_idx || !labels || !ids || !nts || !n_alleles || !counts || !out) return 0;
+    return assocfmt::sliced(n, modelfmt::kModelLineBytes, out, [&](uint64_t r0, uint64_t r1, char* o) {
+        return modelfmt::model_serial(r0, r1, chrom_idx, labels, ids, nts, n_alleles, counts, o);
+    });
+}
+
+uint64_t dnaf_format_hardy(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const uint8_t* nts,
+                           const uint8_t* n_alleles, const uint32_t* counts, const double* hwe_p, char* out) {
+    if (!n || !chrom_idx || !labels || !ids || !nts || !n_alleles || !counts || !hwe_p || !out) return 0;
+    return assocfmt::sliced(n, modelfmt::kHardyLineBytes, out, [&](uint64_t r0, uint64_t r1, char* o) {
+        return modelfmt::hardy_serial(r0, r1, chrom_idx, labels, ids, nts, n_alleles, counts, hwe_p, o);
+    });
 }
 
 int dnaf_genotypes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out, uint64_t cap) {

@@ -1,7 +1,8 @@
-// Host side of the case/control allele counts (k_assoc.cuh) and the .assoc text formatter.  Rows [row_begin,row_end)
-// go in passes bounded by the 2^31-CTA grid and by chunk_bytes of counts (16 bytes a row); every pass zeroes its
-// [rows][4] array, runs one k_assoc and, unless the call is device-only, ends with one copy of the array into the
-// caller's buffer.  Included by dnaf_api.cu after host_bed.h.
+// Host side of the case/control allele counts (k_assoc.cuh) and the .assoc text formatter, and the pass driver of
+// every per-row count kernel (k_assoc here, k_geno in host_geno.h).  Rows [row_begin,row_end) go in passes bounded by
+// the 2^31-CTA grid and by chunk_bytes of device output (16 bytes a row for k_assoc); every pass zeroes its
+// [rows][words] counters, runs its kernels and, unless the call is device-only, ends with the copies into the
+// caller's buffers.  Included by dnaf_api.cu after host_bed.h.
 #pragma once
 
 #include <cmath>
@@ -16,35 +17,30 @@ std::vector<uint32_t> assoc_case_masks(const uint8_t* is_control, uint32_t n) {
     return m;
 }
 
-int assoc_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* out, dnaf_stats* st) {
+// Refuses rows of more than 2 alleles before any launch (`test` names what counts them).
+int check_biallelic(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, const char* test) {
     if (!c->have_samples || !c->have_snps) return fail(c, DNAF_E_ARG, "set_samples and set_snps must be called first");
     if (row_begin > row_end || row_end > c->S) return fail(c, DNAF_E_ARG, "row range out of bounds");
     for (uint64_t r = row_begin; r < row_end; ++r)
         if (c->h_k[r] > 2)
-            return fail(c, DNAF_E_INPUT, "row %llu has %u alleles: the allelic test counts biallelic rows only",
-                        (unsigned long long)r, c->h_k[r]);
+            return fail(c, DNAF_E_INPUT, "row %llu has %u alleles: %s counts biallelic rows only", (unsigned long long)r,
+                        c->h_k[r], test);
+    return DNAF_OK;
+}
+
+// One count kernel over rows [row_begin,row_end) (checked by the caller): `tiles` CTAs a row, `words` uint32 counters a
+// row in c->d_counts (zeroed by every pass), `row_bytes` of device output a row (the pass-size bound).
+// launch(r0, r1) queues the pass's kernels and returns how many; fetch(r0, r1) queues the pass's copies to the host
+// (nothing for device-only calls).  stats: rows, calls, kernel_launches, ms_sample (the pass kernels), ms_total.
+template <class Launch, class Fetch>
+int count_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint32_t tiles, uint32_t words, uint64_t row_bytes,
+                 dnaf_stats* st, Launch launch, Fetch fetch) {
     CU(c, cudaSetDevice(c->dev));
     dnaf_stats local;
     memset(&local, 0, sizeof local);
-    AssocArgs a;
-    a.cls = c->d_cls.as<uint8_t>();
-    a.k = c->d_k.as<uint8_t>();
-    a.thr = c->d_thr.as<uint32_t>();
-    a.sexmask = c->d_sexmask.as<uint2>();
-    a.casemask = c->d_casemask.as<uint32_t>();
-    a.orow = c->d_orow.as<uint64_t>();
-    a.osamp = c->d_osamp.as<uint32_t>();
-    a.n_over = c->P;
-    a.row_base = c->row_base;
-    a.n = c->n;
-    a.groups = (c->n + 15u) / 16u;
-    a.tiles = std::max<uint32_t>(1u, (a.groups + kAssocThreads - 1u) / kAssocThreads);
-    a.k0 = (uint32_t)seed;
-    a.k1 = (uint32_t)(seed >> 32);
-    const uint64_t per_pass = std::max<uint64_t>(1, std::min<uint64_t>(c->chunk_bytes / 16u, 0x7FFFFFFFull / a.tiles));
+    const uint64_t per_pass = std::max<uint64_t>(1, std::min<uint64_t>(c->chunk_bytes / row_bytes, 0x7FFFFFFFull / tiles));
     const uint64_t rows = row_end - row_begin;
-    if (rows) CU(c, c->d_counts.reserve(std::min(rows, per_pass) * 16u));
-    a.counts = c->d_counts.as<uint32_t>();
+    if (rows) CU(c, c->d_counts.reserve(std::min(rows, per_pass) * 4u * words));
     bool timed[3] = {false, false, false};
     // the kernel time of the pass three back (its events are reused by this pass)
     auto retire = [&](int k) -> int {
@@ -63,17 +59,13 @@ int assoc_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t see
         const int k = npass % 3;
         int rc = retire(k);
         if (rc) return rc;
-        a.row0 = r0;
-        CU(c, cudaMemsetAsync(c->d_counts.p, 0, (r1 - r0) * 16u, c->stream));
+        CU(c, cudaMemsetAsync(c->d_counts.p, 0, (r1 - r0) * 4u * words, c->stream));
         CU(c, cudaEventRecord(c->ob[k].ev[0], c->stream));
-        k_assoc<<<(uint32_t)((r1 - r0) * a.tiles), kAssocThreads, 0, c->stream>>>(a);
+        local.kernel_launches += launch(r0, r1);
         CU(c, cudaGetLastError());
         CU(c, cudaEventRecord(c->ob[k].ev[1], c->stream));
         timed[k] = true;
-        local.kernel_launches += 1;
-        if (out)
-            CU(c, cudaMemcpyAsync(out + 4 * (r0 - row_begin), c->d_counts.p, (r1 - r0) * 16u, cudaMemcpyDeviceToHost,
-                                  c->stream));
+        CU(c, fetch(r0, r1));
         local.rows += r1 - r0;
         r0 = r1;
     }
@@ -87,6 +79,38 @@ int assoc_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t see
     local.calls = local.rows * c->n;
     if (st) *st = local;
     return DNAF_OK;
+}
+
+int assoc_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* out, dnaf_stats* st) {
+    int rc = check_biallelic(c, row_begin, row_end, "the allelic test");
+    if (rc) return rc;
+    AssocArgs a;
+    a.cls = c->d_cls.as<uint8_t>();
+    a.k = c->d_k.as<uint8_t>();
+    a.thr = c->d_thr.as<uint32_t>();
+    a.sexmask = c->d_sexmask.as<uint2>();
+    a.casemask = c->d_casemask.as<uint32_t>();
+    a.orow = c->d_orow.as<uint64_t>();
+    a.osamp = c->d_osamp.as<uint32_t>();
+    a.n_over = c->P;
+    a.row_base = c->row_base;
+    a.n = c->n;
+    a.groups = (c->n + 15u) / 16u;
+    a.tiles = std::max<uint32_t>(1u, (a.groups + kAssocThreads - 1u) / kAssocThreads);
+    a.k0 = (uint32_t)seed;
+    a.k1 = (uint32_t)(seed >> 32);
+    auto launch = [&](uint64_t r0, uint64_t r1) {
+        a.row0 = r0;
+        a.counts = c->d_counts.as<uint32_t>();
+        k_assoc<<<(uint32_t)((r1 - r0) * a.tiles), kAssocThreads, 0, c->stream>>>(a);
+        return 1u;
+    };
+    auto fetch = [&](uint64_t r0, uint64_t r1) {
+        return out ? cudaMemcpyAsync(out + 4 * (r0 - row_begin), c->d_counts.p, (r1 - r0) * 16u, cudaMemcpyDeviceToHost,
+                                     c->stream)
+                   : cudaSuccess;
+    };
+    return count_passes(c, row_begin, row_end, a.tiles, 4u, 16u, st, launch, fetch);
 }
 
 int assoc_impl(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* out, dnaf_stats* st) {
@@ -106,13 +130,18 @@ inline int num(char* p, size_t cap, double v) {
     return std::isnan(v) ? snprintf(p, cap, "NA") : snprintf(p, cap, "%.4g", v);
 }
 
+// PLINK's CHR column of label `idx` (8 bytes a label): X, Y and MT are written 23, 24 and 26; `lab` holds the label
+inline const char* chr_code(const char* labels, int32_t idx, char lab[8]) {
+    memcpy(lab, labels + 8 * (size_t)idx, 8);
+    lab[7] = 0;
+    return !strcmp(lab, "X") ? "23" : !strcmp(lab, "Y") ? "24" : !strcmp(lab, "MT") ? "26" : lab;
+}
+
 inline char* lines_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
                           const int64_t* position, const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, char* o) {
     for (uint64_t r = r0; r < r1; ++r) {
         char lab[8];
-        memcpy(lab, labels + 8 * (size_t)chrom_idx[r], 8);
-        lab[7] = 0;
-        const char* chr = !strcmp(lab, "X") ? "23" : !strcmp(lab, "Y") ? "24" : !strcmp(lab, "MT") ? "26" : lab;
+        const char* chr = chr_code(labels, chrom_idx[r], lab);
         const double a = counts[4 * r], ca = counts[4 * r + 1], c = counts[4 * r + 2], cu = counts[4 * r + 3];
         const double b = ca - a, d = cu - c;   // REF in cases, REF in controls
         const double nan = std::nan("");
@@ -137,20 +166,20 @@ inline char* lines_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, co
     return o;
 }
 
-// Rows in slices of 64 Ki over the host's cores (about 1.7 us of printf per row); every slice is written to its own
-// buffer and the slices are joined in order.
-inline uint64_t lines(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const int64_t* position,
-                      const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, char* out) {
-    constexpr uint64_t kSlice = 1ull << 16, kLine = 192;
+// Rows [0,n) in slices of 64 Ki over the host's cores: serial(r0, r1, o) writes the lines of rows [r0,r1) at o (at most
+// `line` bytes a row) and returns their end; every slice is written to its own buffer and the slices are joined in order.
+template <class Serial>
+uint64_t sliced(uint64_t n, uint64_t line, char* out, Serial serial) {
+    constexpr uint64_t kSlice = 1ull << 16;
     const uint64_t slices = (n + kSlice - 1) / kSlice;
-    if (slices <= 1) return (uint64_t)(lines_serial(0, n, chrom_idx, labels, ids, position, nts, n_alleles, counts, out) - out);
+    if (slices <= 1) return (uint64_t)(serial(0, n, out) - out);
     std::vector<std::vector<char>> buf(slices);
     std::atomic<uint64_t> next{0};
     auto work = [&]() {
         for (uint64_t k; (k = next.fetch_add(1)) < slices;) {
             const uint64_t r0 = k * kSlice, r1 = std::min(n, r0 + kSlice);
-            buf[k].resize((r1 - r0) * kLine);
-            char* e = lines_serial(r0, r1, chrom_idx, labels, ids, position, nts, n_alleles, counts, buf[k].data());
+            buf[k].resize((r1 - r0) * line);
+            char* e = serial(r0, r1, buf[k].data());
             buf[k].resize((size_t)(e - buf[k].data()));
         }
     };
@@ -165,6 +194,14 @@ inline uint64_t lines(uint64_t n, const int32_t* chrom_idx, const char* labels, 
         o += b.size();
     }
     return (uint64_t)(o - out);
+}
+
+// about 1.7 us of printf per row
+inline uint64_t lines(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const int64_t* position,
+                      const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, char* out) {
+    return sliced(n, 192, out, [&](uint64_t r0, uint64_t r1, char* o) {
+        return lines_serial(r0, r1, chrom_idx, labels, ids, position, nts, n_alleles, counts, o);
+    });
 }
 
 }  // namespace assocfmt

@@ -1,6 +1,6 @@
 // Host-side state of one GPU context (struct dnaf_ctx), error / trace helpers, uploads and the row layout.
 // Part of the single translation unit dnaf_api.cu (included there, in order: host_ctx.h, host_tables.h,
-// host_plan.h, host_sink.h, host_passes.h, host_bed.h, host_assoc.h).
+// host_plan.h, host_sink.h, host_passes.h, host_bed.h, host_assoc.h, host_geno.h).
 #pragma once
 
 namespace {
@@ -200,6 +200,8 @@ struct dnaf_ctx {
     std::vector<XSpan> h_xspans;
     DevBuf d_sexmask;                      // k_bed: per 16-sample group, bit pairs of the males (x) and females (y)
     DevBuf d_casemask, d_counts;           // k_assoc: per 16-sample group, bit pairs of the cases; a pass's [rows][4] counts
+                                           // (k_geno: [rows][10]; dnaf_hwe_exact: the uploaded triples)
+    DevBuf d_hwe;                          // k_hwe: a pass's [rows][3] P (dnaf_hwe_exact: [n])
     cudaEvent_t ev_bed[2] = {};            // k_bed calls: first launch, last kernel end
     std::vector<uint32_t> h_seg_crc_x;     // L(template body) per X segment
     std::vector<uint32_t> h_xoff;

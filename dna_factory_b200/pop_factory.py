@@ -26,7 +26,7 @@ from datetime import datetime
 
 import numpy
 
-from . import _native, assoc, partition, host
+from . import _native, assoc, model, partition, host
 from . import tabix
 from .tabix import TabixBuilder
 from .snp import (CHROMOSOME_LIST, CHROMOSOME_MAX_POSITION, CHROMOSOME_PROB, SNPTuples, SnpFactory, SnpTable,  # noqa: F401
@@ -57,10 +57,10 @@ def validate_assoc_table(table):
     validate_biallelic_table(table, "--assoc", "the allelic test counts biallelic SNPs only")
 
 
-def validate_assoc_population(control_size, test_size):
-    """--assoc compares cases with controls: both groups must be non-empty."""
+def validate_assoc_population(control_size, test_size, flag="--assoc"):
+    """--assoc and --model compare cases with controls: both groups must be non-empty."""
     if control_size <= 0 or test_size <= 0:
-        raise ValueError("--assoc needs cases and controls (-s %d, -c %d)" % (test_size, control_size))
+        raise ValueError("%s needs cases and controls (-s %d, -c %d)" % (flag, test_size, control_size))
 
 
 def gen_vcf_header(fam_data):
@@ -205,7 +205,8 @@ class DeleteriousGroup:
 class PopulationFactory:
     def __init__(self, num_processes=1, generate_snps=False, male_odds=0.5, deleterious_config=None,
                  deleterious_list_path=None, sample_id_offset=0, snps_path=None, output_path=None, seed=None,
-                 gpus=1, gpu_select=False, tbi=False, bed=False, assoc=False):
+                 gpus=1, gpu_select=False, tbi=False, bed=False, assoc=False, model=False,
+                 hardy=False):
         self.deleterious = {}
         self.ordered_snps = []
         self.snp_table = None
@@ -231,12 +232,18 @@ class PopulationFactory:
         self.assoc = bool(assoc)
         self.assoc_counts = None     # uint32[rows, 4] allele counts of the last write_vcf_snps (--assoc)
         self.override_rows = None    # global row of every override pair of the last write_vcf_snps
+        self.model = bool(model)
+        self.hardy = bool(hardy)
+        self.geno_counts = None      # uint32[rows, 10] genotype counts of the last write_vcf_snps (--model / --hardy)
+        self.hwe_p = None            # float64[rows, 3] Hardy-Weinberg exact P (ALL, AFF, UNAFF) of the same rows
 
     # ------------------------------------------------------------------------------------------ orchestration
     def generate_population(self, control_size, test_size, min_freq, max_snps, compression_level=6):
         t0 = time.time()
         if self.assoc:
             validate_assoc_population(control_size, test_size)
+        if self.model:
+            validate_assoc_population(control_size, test_size, "--model")
         clock_seed = int(datetime.now().strftime("%H%M%S"))
         numpy.random.seed(clock_seed)
         if self.seed is None:
@@ -334,6 +341,10 @@ class PopulationFactory:
             validate_bed_table(snps)
         if self.assoc:
             validate_assoc_table(snps)
+        if self.model:
+            validate_biallelic_table(snps, "--model", "the genotypic tests count biallelic SNPs only")
+        if self.hardy:
+            validate_biallelic_table(snps, "--hardy", "the Hardy-Weinberg tests count biallelic SNPs only")
         groups = PopulationFactory.pick_deleterious_groups(list(self.deleterious.values()), test_size)
         fam_data = self.generate_fam_file(control_size, test_size, male_odds, groups)
         main_file = self.population_dir + "population.vcf.gz"
@@ -362,6 +373,8 @@ class PopulationFactory:
                     b.write(snps.bim_bytes())
             if self.assoc:
                 self.output_assoc(snps)
+            if self.model or self.hardy:
+                self.output_model(snps)
         finally:
             engine.close()
             if bed_fd is not None:
@@ -378,12 +391,28 @@ class PopulationFactory:
             f.write(text)
         print(summary, flush=True)
 
+    def output_model(self, table):
+        """population.model and deleterious_model.txt (--model) and population.hwe (--hardy) from the genotype counts
+        and exact-test P write_vcf_snps took on the GPU."""
+        if self.model:
+            with open(self.population_dir + "population.model", "wb") as f:
+                f.write(model.model_bytes(table, self.geno_counts))
+            text, summary = model.deleterious_model_report(table, self.deleterious, self.geno_counts, self.hwe_p,
+                                                           self.override_rows)
+            with open(self.population_dir + "deleterious_model.txt", "wb") as f:
+                f.write(text)
+            print(summary, flush=True)
+        if self.hardy:
+            with open(self.population_dir + "population.hwe", "wb") as f:
+                f.write(model.hardy_bytes(table, self.geno_counts, self.hwe_p))
+
     # ------------------------------------------------------------------------------------------ the GPU seam
     def write_vcf_snps(self, fam_data, snps, file, engine=None, bed_fd=None):
         """Rows of `snps` (in order) for `fam_data`, appended to `file` -- the reference's seam
         (pop_factory.py:417-469).  `snps` is a list of SNPTuples or a SnpTable; `file` a BgzfSink.  With `bed_fd`
         (an open population.bed that holds the 3 magic bytes) the same rows also go there as PLINK 1 .bed rows.  With
-        --assoc the case/control allele counts of the same rows land in self.assoc_counts."""
+        --assoc the case/control allele counts of the same rows land in self.assoc_counts, with --model / --hardy their
+        genotype counts and exact-test P in self.geno_counts / self.hwe_p."""
         t0 = time.time()
         level = getattr(file, "compresslevel", getattr(self, "_level", 6))
         seed = self.seed if self.seed is not None else int(datetime.now().strftime("%H%M%S"))
@@ -423,6 +452,8 @@ class PopulationFactory:
                     self.bed_stats.append(eng.generate_bed_fd_at(0, n_rows, seed, bed_fd, len(BED_MAGIC)))
                 if self.assoc:
                     self.assoc_counts = eng.allele_counts(0, n_rows, seed)
+                if self.model or self.hardy:
+                    self.geno_counts, self.hwe_p = eng.genotype_counts(0, n_rows, seed)
             finally:
                 if own:
                     eng.close()
@@ -439,13 +470,13 @@ class PopulationFactory:
         nothing is spooled or copied twice.  Every rank holds only its own slice of the SNP table; the Philox row
         counter of its local row r is bounds[g] + r (dnaf_set_row_base).  .bed rows have a fixed size, so rank g
         pwrite()s its rows at 3 + bounds[g] * ceil(N/4) of population.bed without a sizing pass.  With --assoc every
-        rank counts its own rows after its VCF write; the slices are joined in rank order."""
+        rank counts its own rows after its VCF write; the slices are joined in rank order (so do --model / --hardy)."""
         bounds = partition.row_bounds(n_rows, gpus)
         n_dev = max(1, _native.device_count())      # more ranks than devices: ranks share devices round-robin
         errors = []
         index = getattr(file, "index", None)
         blocks, row_off, sizes, engines = [None] * gpus, [None] * gpus, [0] * gpus, [None] * gpus
-        counts = [None] * gpus
+        counts, geno = [None] * gpus, [None] * gpus
         barrier = threading.Barrier(gpus)
         file.flush()   # the header blocks must be in the file: the ranks write behind them
         base = file._handle.tell()
@@ -485,6 +516,8 @@ class PopulationFactory:
                     blocks[g] = eng.block_log_get()
                 if self.assoc:
                     counts[g] = eng.allele_counts(0, hi - lo, seed)
+                if self.model or self.hardy:
+                    geno[g] = eng.genotype_counts(0, hi - lo, seed)
             except BaseException as e:  # noqa
                 errors.append(e)
 
@@ -501,6 +534,9 @@ class PopulationFactory:
         file._handle.seek(base + sum(sizes))      # the sink appends the EOF block behind the last rank's stream
         if self.assoc:
             self.assoc_counts = numpy.concatenate(counts)
+        if self.model or self.hardy:
+            self.geno_counts = numpy.concatenate([q[0] for q in geno])
+            self.hwe_p = numpy.concatenate([q[1] for q in geno])
         if index is not None:
             off = numpy.concatenate([numpy.zeros(1, numpy.uint64)] +
                                     [r[1:] + numpy.uint64(sum(int(q[-1]) for q in row_off[:g])) for g, r in enumerate(row_off)])
@@ -573,6 +609,13 @@ def parse_cmd_args(args):
     ap.add_argument("--assoc", action="store_true",
                     help="also write population.assoc (case/control allelic test of every SNP, counted on the GPU) and "
                          "deleterious_assoc.txt (rank of every planted deleterious SNP); every SNP must be biallelic")
+    ap.add_argument("--model", action="store_true",
+                    help="also write population.model (GENO, TREND, ALLELIC, DOM, REC case/control tests of every SNP, "
+                         "genotypes counted on the GPU) and deleterious_model.txt (how every planted deleterious SNP "
+                         "fares under them); every SNP must be biallelic")
+    ap.add_argument("--hardy", action="store_true",
+                    help="also write population.hwe (Hardy-Weinberg exact tests of every SNP in all samples, cases and "
+                         "controls, on the GPU); every SNP must be biallelic")
     return ap.parse_args(args)
 
 
@@ -585,7 +628,8 @@ def main(sys_args):
                                 deleterious_list_path=args.deleterious_file, sample_id_offset=args.offset,
                                 male_odds=args.male_odds, deleterious_config=args.deleterious_config,
                                 snps_path=args.snps_file, output_path=args.outdir, seed=args.seed, gpus=args.gpus,
-                                gpu_select=args.gpu_select, tbi=args.tbi, bed=args.bed, assoc=args.assoc)
+                                gpu_select=args.gpu_select, tbi=args.tbi, bed=args.bed, assoc=args.assoc,
+                                model=args.model, hardy=args.hardy)
     factory.generate_population(args.control_size, args.size, args.min_freq, args.max_snps, args.compression_level)
 
 

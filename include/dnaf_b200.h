@@ -235,6 +235,54 @@ uint64_t dnaf_format_assoc(uint64_t n, const int32_t* chrom_idx, const char* lab
                            const int64_t* position, const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts,
                            char* out);
 
+/*
+ * Case/control genotype counts of rows [row_begin,row_end), the input of the genotypic tests (plink --model) and of
+ * the Hardy-Weinberg exact tests (plink --hardy): the same draws, forced minors and ploidy rules as the VCF and .bed
+ * rows of the same seed.  counts is [rows][10]: for the cases (is_control[i] == 0 in dnaf_set_samples) dip (diploid
+ * cells), het (diploid 0/1), hom (diploid 1/1, ALT/ALT), hap (haploid cells printed), hap_alt (haploid cells printed
+ * as ALT); then the same five for the controls.  Diploid cells: every sample on autosome rows, females on X rows;
+ * haploid cells: males on X and Y rows, every sample on MT rows; female Y cells ('.') count nothing.  A forced minor
+ * makes its cell 1/1 (ALT on a haploid cell).  So 2 hom + het + hap_alt and 2 dip + hap are the ALT and observed
+ * allele counts of dnaf_allele_counts.  hwe_p (NULL: not computed) is [rows][3]: the two-sided Hardy-Weinberg exact P
+ * (dnaf_hwe_exact) of the diploid genotypes of ALL samples, the cases (AFF) and the controls (UNAFF); NaN where the
+ * group has no diploid cell (Y and MT rows, empty groups).  Rows with more than 2 alleles: DNAF_E_INPUT before any GPU
+ * work, naming the row.  stats: rows, calls, kernel_launches, ms_sample (the counting and exact-test kernels),
+ * ms_total; the other fields are 0.
+ */
+int dnaf_genotype_counts(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* counts,
+                         double* hwe_p, dnaf_stats* stats);
+/* Same work, counts (and, with with_hwe != 0, the exact tests) left in device memory: kernel-only timing. */
+int dnaf_genotype_counts_device(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, int with_hwe,
+                                dnaf_stats* stats);
+/*
+ * Two-sided Hardy-Weinberg exact P of n genotype triples geno[i] = (n11, n12, n22) (ALT/ALT, het, REF/REF), computed
+ * on the device by the kernel dnaf_genotype_counts uses: Wigginton, Cutler & Abecasis (2005), the SNPHWE definition
+ * of plink --hardy.  P is the sum of the probabilities of every het count whose probability is <= (1 + 1e-7) times
+ * that of the observed one (the relative tolerance makes ties independent of rounding), over the sum of all of them,
+ * in double precision; 0 where P < 1e-290, NaN where n11 + n12 + n22 = 0.  Synchronous.
+ */
+int dnaf_hwe_exact(dnaf_ctx* ctx, uint64_t n, const uint32_t* geno, double* p);
+/*
+ * The .model body lines of n rows from their genotype counts (host code, no context, no GPU; labels and nts as in
+ * dnaf_format_assoc): five lines a row, GENO, TREND, ALLELIC, DOM, REC, with columns CHR SNP A1 A2 TEST AFF UNAFF
+ * CHISQ DF P.  With n11 / n12 / n22 the diploid ALT/ALT, het and REF/REF counts of a group, AFF and UNAFF are
+ * n11/n12/n22 (GENO, TREND), ALT/REF alleles with haploid cells (ALLELIC), n11+n12/n22 (DOM), n11/n12+n22 (REC).
+ * ALLELIC is the .assoc statistic; TREND the Cochran-Armitage trend test on diploid cells; GENO the 2x3 Pearson
+ * test (2 df), DOM and REC 2x2 Pearson tests (1 df); no continuity correction, P the chi-square survival in double.
+ * GENO, DOM and REC are NA when any of the six genotype cells is below 5 (PLINK's --cell 5); any zero denominator is
+ * NA; an NA test prints NA for CHISQ, DF and P.  `out` holds at least 960 bytes per row.  Returns the bytes written.
+ */
+uint64_t dnaf_format_model(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const uint8_t* nts,
+                           const uint8_t* n_alleles, const uint32_t* counts, char* out);
+/*
+ * The .hwe body lines of n rows from their genotype counts and hwe_p (dnaf_genotype_counts): three lines a row, ALL,
+ * AFF, UNAFF, with columns CHR SNP TEST A1 A2 GENO O(HET) E(HET) P; GENO is n11/n12/n22 of the diploid cells (females
+ * only on X rows, 0/0/0 on Y and MT rows), O(HET) = n12 / n and E(HET) = 2 f (1 - f) with f = (2 n11 + n12) / 2n;
+ * NA where n = 0.  `out` holds at least 576 bytes per row.  Returns the bytes written.
+ */
+uint64_t dnaf_format_hardy(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const uint8_t* nts,
+                           const uint8_t* n_alleles, const uint32_t* counts, const double* hwe_p, char* out);
+
 /* Parity gates. genotypes: out[(r*n_samples+i)*2+s] = allele index, 0xFF where the cell has no such
  * allele (second slot of a haploid cell, both slots of '.').  text: the uncompressed rows. */
 int dnaf_genotypes(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out,
