@@ -43,7 +43,9 @@ EXPORTS = ["dnaf_abi_version", "dnaf_device_count", "dnaf_last_error", "dnaf_cre
            "dnaf_block_log_get", "dnaf_select_snps", "dnaf_parse_snps_jsonl", "dnaf_format_prefixes",
            "dnaf_format_snps_jsonl", "dnaf_debug_lz_block", "dnaf_generate_bed", "dnaf_generate_bed_fd_at",
            "dnaf_generate_bed_device", "dnaf_allele_counts", "dnaf_allele_counts_device", "dnaf_format_assoc",
-           "dnaf_genotype_counts", "dnaf_genotype_counts_device", "dnaf_hwe_exact", "dnaf_format_model", "dnaf_format_hardy"]
+           "dnaf_genotype_counts", "dnaf_genotype_counts_device", "dnaf_hwe_exact", "dnaf_format_model", "dnaf_format_hardy",
+           "dnaf_genotype_tests", "dnaf_genotype_tests_device", "dnaf_fisher_exact", "dnaf_format_assoc_fisher",
+           "dnaf_format_model_fisher"]
 
 _lib = None
 
@@ -96,6 +98,13 @@ def load():
                                     u8p, u8p, u32p, u8p]),
         "dnaf_format_hardy": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64),
                                     u8p, u8p, u32p, f64p, u8p]),
+        "dnaf_genotype_tests": (i32, [vp, u64, u64, u64, u32p, f64p, f64p, sp]),
+        "dnaf_genotype_tests_device": (i32, [vp, u64, u64, u64, i32, i32, sp]),
+        "dnaf_fisher_exact": (i32, [vp, u64, u32p, f64p]),
+        "dnaf_format_assoc_fisher": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64),
+                                           ctypes.POINTER(ctypes.c_int64), u8p, u8p, u32p, f64p, u8p]),
+        "dnaf_format_model_fisher": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64),
+                                           u8p, u8p, u32p, f64p, u8p]),
         "dnaf_genotypes": (i32, [vp, u64, u64, u64, u8p, u64]),
         "dnaf_text": (i32, [vp, u64, u64, u64, u8p, u64, u64p]),
         "dnaf_bgzf_compress": (i32, [vp, u8p, u64, u8p, u64, sp]),
@@ -391,6 +400,42 @@ class Engine:
                                              p.ctypes.data_as(ctypes.POINTER(ctypes.c_double))))
         return p
 
+    # -- counts, Hardy-Weinberg and Fisher exact tests in one pass (pop_factory --fisher / --model / --hardy)
+    def genotype_tests(self, row_begin, row_end, seed, hwe=True, fisher=True):
+        """(uint32[rows, 10], float64[rows, 3] or None, float64[rows, 4] or None) of rows [row_begin,row_end): the
+        genotype counts, the Hardy-Weinberg exact P of ALL, AFF, UNAFF and log10 of the Fisher exact P of GENO, ALLELIC,
+        DOM, REC (include/dnaf_b200.h, dnaf_genotype_tests)."""
+        return self.genotype_tests_stats(row_begin, row_end, seed, hwe, fisher)[:3]
+
+    def genotype_tests_stats(self, row_begin, row_end, seed, hwe=True, fisher=True):
+        """Same -> (counts, P or None, log10 P or None, stats dict)."""
+        rows = max(row_end - row_begin, 0)
+        out = np.zeros((rows, 10), np.uint32)
+        p = np.zeros((rows, 3), np.float64) if hwe else None
+        l = np.zeros((rows, 4), np.float64) if fisher else None
+        f64p = ctypes.POINTER(ctypes.c_double)
+        st = Stats()
+        self._check(self._lib.dnaf_genotype_tests(
+            self._h, row_begin, row_end, seed, out.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
+            p.ctypes.data_as(f64p) if hwe else None, l.ctypes.data_as(f64p) if fisher else None, ctypes.byref(st)))
+        return out, p, l, st.as_dict()
+
+    def genotype_tests_device(self, row_begin, row_end, seed, hwe=True, fisher=True):
+        """Same work, results left on the device; returns stats dict."""
+        st = Stats()
+        self._check(self._lib.dnaf_genotype_tests_device(self._h, row_begin, row_end, seed, int(bool(hwe)), int(bool(fisher)),
+                                                         ctypes.byref(st)))
+        return st.as_dict()
+
+    def fisher_exact(self, tables):
+        """float64[n]: log10 of the two-sided Fisher exact P of every (x1, x2, x3, y1, y2, y3) row of `tables` (case row,
+        control row), computed by the device kernel (dnaf_fisher_exact); NaN where there is no test."""
+        t = np.ascontiguousarray(tables, np.uint32).reshape(-1, 6)
+        l = np.zeros(len(t), np.float64)
+        self._check(self._lib.dnaf_fisher_exact(self._h, len(t), t.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
+                                                l.ctypes.data_as(ctypes.POINTER(ctypes.c_double))))
+        return l
+
     # -- parity gates
     def genotypes(self, row_begin, row_end, seed):
         rows = row_end - row_begin
@@ -563,6 +608,42 @@ def format_hardy(ids, chrom_idx, labels, n_alleles, nts, counts, hwe_p):
                                  ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _u8(nt), _u8(k),
                                  cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
                                  p.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), _u8(out))
+    return out[:used].tobytes()
+
+
+def format_assoc_fisher(ids, chrom_idx, labels, position, n_alleles, nts, counts, log10p):
+    """.assoc.fisher body lines (dnaf_format_assoc_fisher: F_A, F_U, P of Fisher ALLELIC, OR) of a column-form SNP
+    table, its uint32[rows, 10] genotype counts and float64[rows, 4] Fisher log10 P -> bytes."""
+    lib = load()
+    n = len(ids)
+    if n == 0:
+        return b""
+    ids, ci, lab, k, nt, cnt = _geno_columns(ids, chrom_idx, labels, n_alleles, nts, counts)
+    pos = np.ascontiguousarray(position, np.int64)
+    l = np.ascontiguousarray(log10p, np.float64).reshape(n, 4)
+    out = np.empty(n * 192 + 16, np.uint8)
+    i64p = ctypes.POINTER(ctypes.c_int64)
+    used = lib.dnaf_format_assoc_fisher(n, ci.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), lab, ids.ctypes.data_as(i64p),
+                                        pos.ctypes.data_as(i64p), _u8(nt), _u8(k),
+                                        cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
+                                        l.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), _u8(out))
+    return out[:used].tobytes()
+
+
+def format_model_fisher(ids, chrom_idx, labels, n_alleles, nts, counts, log10p):
+    """Fisher .model body lines (dnaf_format_model_fisher: GENO, TREND, ALLELIC, DOM, REC per SNP) of a column-form SNP
+    table, its uint32[rows, 10] genotype counts and float64[rows, 4] Fisher log10 P -> bytes."""
+    lib = load()
+    n = len(ids)
+    if n == 0:
+        return b""
+    ids, ci, lab, k, nt, cnt = _geno_columns(ids, chrom_idx, labels, n_alleles, nts, counts)
+    l = np.ascontiguousarray(log10p, np.float64).reshape(n, 4)
+    out = np.empty(n * 960 + 16, np.uint8)
+    used = lib.dnaf_format_model_fisher(n, ci.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), lab,
+                                        ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _u8(nt), _u8(k),
+                                        cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
+                                        l.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), _u8(out))
     return out[:used].tobytes()
 
 

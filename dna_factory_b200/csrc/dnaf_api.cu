@@ -29,6 +29,7 @@
 #include "k_assoc.cuh"
 #include "k_bed.cuh"
 #include "k_deflate.cuh"
+#include "k_fisher.cuh"
 #include "k_fused.cuh"
 #include "k_fused_text.cuh"
 #include "k_geno.cuh"
@@ -619,22 +620,41 @@ uint64_t dnaf_format_assoc(uint64_t n, const int32_t* chrom_idx, const char* lab
     return assocfmt::lines(n, chrom_idx, labels, ids, position, nts, n_alleles, counts, out);
 }
 
-int dnaf_genotype_counts(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* counts, double* hwe_p,
-                         dnaf_stats* stats) {
+int dnaf_genotype_tests(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* counts, double* hwe_p,
+                        double* fisher_log10p, dnaf_stats* stats) {
     if (!c) return DNAF_E_ARG;
     if (!counts && row_end > row_begin) return fail(c, DNAF_E_ARG, "counts is NULL");
-    return geno_impl(c, row_begin, row_end, seed, counts, hwe_p, hwe_p != nullptr, stats);
+    return geno_impl(c, row_begin, row_end, seed, counts, hwe_p, hwe_p != nullptr, fisher_log10p, fisher_log10p != nullptr,
+                     stats);
+}
+
+int dnaf_genotype_tests_device(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, int with_hwe,
+                               int with_fisher, dnaf_stats* stats) {
+    return geno_impl(c, row_begin, row_end, seed, nullptr, nullptr, with_hwe != 0, nullptr, with_fisher != 0, stats);
+}
+
+int dnaf_genotype_counts(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* counts, double* hwe_p,
+                         dnaf_stats* stats) {
+    return dnaf_genotype_tests(c, row_begin, row_end, seed, counts, hwe_p, nullptr, stats);
 }
 
 int dnaf_genotype_counts_device(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, int with_hwe,
                                 dnaf_stats* stats) {
-    return geno_impl(c, row_begin, row_end, seed, nullptr, nullptr, with_hwe != 0, stats);
+    return dnaf_genotype_tests_device(c, row_begin, row_end, seed, with_hwe, 0, stats);
 }
 
 int dnaf_hwe_exact(dnaf_ctx* c, uint64_t n, const uint32_t* geno, double* p) {
     if (!c) return DNAF_E_ARG;
     if (n && (!geno || !p)) return fail(c, DNAF_E_ARG, "geno / p is NULL");
     const int rc = hwe_exact_impl(c, n, geno, p);
+    if (rc) quiesce(c);
+    return rc;
+}
+
+int dnaf_fisher_exact(dnaf_ctx* c, uint64_t n, const uint32_t* tables, double* log10p) {
+    if (!c) return DNAF_E_ARG;
+    if (n && (!tables || !log10p)) return fail(c, DNAF_E_ARG, "tables / log10p is NULL");
+    const int rc = fisher_exact_impl(c, n, tables, log10p);
     if (rc) quiesce(c);
     return rc;
 }
@@ -652,6 +672,24 @@ uint64_t dnaf_format_hardy(uint64_t n, const int32_t* chrom_idx, const char* lab
     if (!n || !chrom_idx || !labels || !ids || !nts || !n_alleles || !counts || !hwe_p || !out) return 0;
     return assocfmt::sliced(n, modelfmt::kHardyLineBytes, out, [&](uint64_t r0, uint64_t r1, char* o) {
         return modelfmt::hardy_serial(r0, r1, chrom_idx, labels, ids, nts, n_alleles, counts, hwe_p, o);
+    });
+}
+
+uint64_t dnaf_format_assoc_fisher(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
+                                  const int64_t* position, const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts,
+                                  const double* log10p, char* out) {
+    if (!n || !chrom_idx || !labels || !ids || !position || !nts || !n_alleles || !counts || !log10p || !out) return 0;
+    return assocfmt::sliced(n, modelfmt::kAssocLineBytes, out, [&](uint64_t r0, uint64_t r1, char* o) {
+        return modelfmt::assoc_fisher_serial(r0, r1, chrom_idx, labels, ids, position, nts, n_alleles, counts, log10p, o);
+    });
+}
+
+uint64_t dnaf_format_model_fisher(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
+                                  const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, const double* log10p,
+                                  char* out) {
+    if (!n || !chrom_idx || !labels || !ids || !nts || !n_alleles || !counts || !log10p || !out) return 0;
+    return assocfmt::sliced(n, modelfmt::kModelLineBytes, out, [&](uint64_t r0, uint64_t r1, char* o) {
+        return modelfmt::model_fisher_serial(r0, r1, chrom_idx, labels, ids, nts, n_alleles, counts, log10p, o);
     });
 }
 

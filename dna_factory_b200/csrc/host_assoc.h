@@ -137,25 +137,33 @@ inline const char* chr_code(const char* labels, int32_t idx, char lab[8]) {
     return !strcmp(lab, "X") ? "23" : !strcmp(lab, "Y") ? "24" : !strcmp(lab, "MT") ? "26" : lab;
 }
 
+// The allelic statistics of a row from a = ALT and ca = observed alleles in cases, c / cu the same in controls; NaN = NA
+struct AlleleStats {
+    double f_a, f_u, chisq, p, odds;
+    AlleleStats(double a, double ca, double c, double cu) {
+        const double b = ca - a, d = cu - c;   // REF in cases, REF in controls
+        const double nan = std::nan("");
+        f_a = ca > 0 ? a / ca : nan;
+        f_u = cu > 0 ? c / cu : nan;
+        const double den = ca * cu * (a + c) * (b + d);
+        chisq = den > 0 ? (a + b + c + d) * (a * d - b * c) * (a * d - b * c) / den : nan;
+        p = std::isnan(chisq) ? nan : std::erfc(std::sqrt(chisq / 2.0));
+        odds = b * c > 0 ? a * d / (b * c) : nan;
+    }
+};
+
 inline char* lines_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
                           const int64_t* position, const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, char* o) {
     for (uint64_t r = r0; r < r1; ++r) {
         char lab[8];
         const char* chr = chr_code(labels, chrom_idx[r], lab);
-        const double a = counts[4 * r], ca = counts[4 * r + 1], c = counts[4 * r + 2], cu = counts[4 * r + 3];
-        const double b = ca - a, d = cu - c;   // REF in cases, REF in controls
-        const double nan = std::nan("");
-        const double f_a = ca > 0 ? a / ca : nan, f_u = cu > 0 ? c / cu : nan;
-        const double den = ca * cu * (a + c) * (b + d);
-        const double chisq = den > 0 ? (a + b + c + d) * (a * d - b * c) * (a * d - b * c) / den : nan;
-        const double p = std::isnan(chisq) ? nan : std::erfc(std::sqrt(chisq / 2.0));
-        const double odds = b * c > 0 ? a * d / (b * c) : nan;
+        const AlleleStats s(counts[4 * r], counts[4 * r + 1], counts[4 * r + 2], counts[4 * r + 3]);
         char v[5][32];
-        num(v[0], 32, f_a);
-        num(v[1], 32, f_u);
-        num(v[2], 32, chisq);
-        num(v[3], 32, p);
-        num(v[4], 32, odds);
+        num(v[0], 32, s.f_a);
+        num(v[1], 32, s.f_u);
+        num(v[2], 32, s.chisq);
+        num(v[3], 32, s.p);
+        num(v[4], 32, s.odds);
         char snp[32];
         snprintf(snp, sizeof snp, "rs%lld", (long long)ids[r]);
         const char a1 = n_alleles[r] >= 2 ? (char)nts[4 * r + 1] : '0';   // A1 = ALT ('0' when the row has none), as in the .bim

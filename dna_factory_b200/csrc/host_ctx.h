@@ -202,6 +202,7 @@ struct dnaf_ctx {
     DevBuf d_casemask, d_counts;           // k_assoc: per 16-sample group, bit pairs of the cases; a pass's [rows][4] counts
                                            // (k_geno: [rows][10]; dnaf_hwe_exact: the uploaded triples)
     DevBuf d_hwe;                          // k_hwe: a pass's [rows][3] P (dnaf_hwe_exact: [n])
+    DevBuf d_fisher;                       // k_fisher: a pass's [rows][4] log10 P (dnaf_fisher_exact: [n])
     cudaEvent_t ev_bed[2] = {};            // k_bed calls: first launch, last kernel end
     std::vector<uint32_t> h_seg_crc_x;     // L(template body) per X segment
     std::vector<uint32_t> h_xoff;

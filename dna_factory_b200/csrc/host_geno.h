@@ -1,13 +1,14 @@
-// Host side of the case/control genotype counts (k_geno) and the Hardy-Weinberg exact tests (k_hwe), and the .model
-// and .hwe text formatters.  The counts run through count_passes (host_assoc.h): 40 bytes of counters a row, plus 24
-// bytes of P a row when the call also runs k_hwe over the pass's counters (three tests a row: ALL, AFF, UNAFF).
-// Included by dnaf_api.cu after host_assoc.h.
+// Host side of the case/control genotype counts (k_geno), the Hardy-Weinberg exact tests (k_hwe) and Fisher's exact
+// tests (k_fisher), and the .model, .hwe and Fisher text formatters.  The counts run through count_passes
+// (host_assoc.h): 40 bytes of counters a row, plus 24 bytes of P a row when the call also runs k_hwe over the pass's
+// counters (three tests a row: ALL, AFF, UNAFF), plus 32 bytes of log10 P a row when it also runs k_fisher (four tests
+// a row: GENO, ALLELIC, DOM, REC).  Included by dnaf_api.cu after host_assoc.h.
 #pragma once
 
 namespace {
 
 int geno_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* out, double* hwe_out,
-                bool with_hwe, dnaf_stats* st) {
+                bool with_hwe, double* fisher_out, bool with_fisher, dnaf_stats* st) {
     int rc = check_biallelic(c, row_begin, row_end, "the genotype count");
     if (rc) return rc;
     GenoArgs a;
@@ -25,24 +26,38 @@ int geno_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed
     a.tiles = std::max<uint32_t>(1u, (a.groups + kGenoThreads - 1u) / kGenoThreads);
     a.k0 = (uint32_t)seed;
     a.k1 = (uint32_t)(seed >> 32);
-    constexpr uint64_t kCountBytes = 4u * kGenoWords;
-    const uint64_t row_bytes = kCountBytes + (with_hwe ? 3u * sizeof(double) : 0u);
-    if (with_hwe && row_end > row_begin) {
+    constexpr uint64_t kCountBytes = 4u * kGenoWords, kFisherBytes = kFisherTests * sizeof(double);
+    const uint64_t row_bytes = kCountBytes + (with_hwe ? 3u * sizeof(double) : 0u) + (with_fisher ? kFisherBytes : 0u);
+    if ((with_hwe || with_fisher) && row_end > row_begin) {
         const uint64_t per_pass = std::max<uint64_t>(1, std::min<uint64_t>(c->chunk_bytes / row_bytes, 0x7FFFFFFFull / a.tiles));
-        CU(c, c->d_hwe.reserve(std::min(row_end - row_begin, per_pass) * 3u * sizeof(double)));
+        const uint64_t rows = std::min(row_end - row_begin, per_pass);
+        if (with_hwe) CU(c, c->d_hwe.reserve(rows * 3u * sizeof(double)));
+        if (with_fisher) CU(c, c->d_fisher.reserve(rows * kFisherBytes));
     }
     auto launch = [&](uint64_t r0, uint64_t r1) {
         a.row0 = r0;
         a.counts = c->d_counts.as<uint32_t>();
         k_geno<<<(uint32_t)((r1 - r0) * a.tiles), kGenoThreads, 0, c->stream>>>(a);
-        if (!with_hwe) return 1u;
-        HweArgs h;
-        h.counts = a.counts;
-        h.items = 3 * (r1 - r0);
-        h.rows = 1;
-        h.p = c->d_hwe.as<double>();
-        k_hwe<<<(uint32_t)((h.items + 255) / 256), 256, 0, c->stream>>>(h);
-        return 2u;
+        uint32_t n = 1;
+        if (with_hwe) {
+            HweArgs h;
+            h.counts = a.counts;
+            h.items = 3 * (r1 - r0);
+            h.rows = 1;
+            h.p = c->d_hwe.as<double>();
+            k_hwe<<<(uint32_t)((h.items + 255) / 256), 256, 0, c->stream>>>(h);
+            ++n;
+        }
+        if (with_fisher) {
+            FisherArgs f;
+            f.counts = a.counts;
+            f.items = kFisherTests * (r1 - r0);
+            f.rows = 1;
+            f.log10p = c->d_fisher.as<double>();
+            k_fisher<<<(uint32_t)((f.items + kFisherThreads - 1) / kFisherThreads), kFisherThreads, 0, c->stream>>>(f);
+            ++n;
+        }
+        return n;
     };
     auto fetch = [&](uint64_t r0, uint64_t r1) {
         cudaError_t e = cudaSuccess;
@@ -52,15 +67,18 @@ int geno_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed
         if (e == cudaSuccess && with_hwe && hwe_out)
             e = cudaMemcpyAsync(hwe_out + 3 * (r0 - row_begin), c->d_hwe.p, (r1 - r0) * 3u * sizeof(double),
                                 cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess && with_fisher && fisher_out)
+            e = cudaMemcpyAsync(fisher_out + kFisherTests * (r0 - row_begin), c->d_fisher.p, (r1 - r0) * kFisherBytes,
+                                cudaMemcpyDeviceToHost, c->stream);
         return e;
     };
     return count_passes(c, row_begin, row_end, a.tiles, kGenoWords, row_bytes, st, launch, fetch);
 }
 
 int geno_impl(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* out, double* hwe_out,
-              bool with_hwe, dnaf_stats* st) {
+              bool with_hwe, double* fisher_out, bool with_fisher, dnaf_stats* st) {
     if (!c) return DNAF_E_ARG;
-    const int rc = geno_passes(c, row_begin, row_end, seed, out, hwe_out, with_hwe, st);
+    const int rc = geno_passes(c, row_begin, row_end, seed, out, hwe_out, with_hwe, fisher_out, with_fisher, st);
     if (rc) quiesce(c);
     return rc;
 }
@@ -80,6 +98,25 @@ int hwe_exact_impl(dnaf_ctx* c, uint64_t n, const uint32_t* geno, double* p) {
     k_hwe<<<(uint32_t)((n + 255) / 256), 256, 0, c->stream>>>(h);
     CU(c, cudaGetLastError());
     CU(c, cudaMemcpyAsync(p, c->d_hwe.p, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    return DNAF_OK;
+}
+
+int fisher_exact_impl(dnaf_ctx* c, uint64_t n, const uint32_t* tables, double* log10p) {
+    if (n == 0) return DNAF_OK;
+    if (n > 0x7FFFFFFFull * kFisherThreads) return fail(c, DNAF_E_ARG, "too many tables for one grid");
+    CU(c, cudaSetDevice(c->dev));
+    int rc = upload(c, c->d_counts, tables, 6 * n, false);
+    if (rc) return rc;
+    CU(c, c->d_fisher.reserve(n * sizeof(double)));
+    FisherArgs f;
+    f.counts = c->d_counts.as<uint32_t>();
+    f.items = n;
+    f.rows = 0;
+    f.log10p = c->d_fisher.as<double>();
+    k_fisher<<<(uint32_t)((n + kFisherThreads - 1) / kFisherThreads), kFisherThreads, 0, c->stream>>>(f);
+    CU(c, cudaGetLastError());
+    CU(c, cudaMemcpyAsync(log10p, c->d_fisher.p, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
     return DNAF_OK;
 }
@@ -153,22 +190,19 @@ inline char a1_of(const uint8_t* nts, const uint8_t* n_alleles, uint64_t r) {
     return n_alleles[r] >= 2 ? (char)nts[4 * r + 1] : '0';   // A1 = ALT ('0' when the row has none), as in the .bim
 }
 
-inline char* model_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
-                          const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, char* o) {
-    static const char* const kTest[5] = {"GENO", "TREND", "ALLELIC", "DOM", "REC"};
-    static const int kDf[5] = {2, 1, 1, 1, 1};
-    for (uint64_t r = r0; r < r1; ++r) {
-        const uint32_t* c = counts + (uint64_t)kGenoWords * r;
-        char lab[8];
-        const char* chr = assocfmt::chr_code(labels, chrom_idx[r], lab);
-        char snp[32];
+// The columns a .model line and a Fisher .model line share: CHR, SNP, A1, A2 and the AFF / UNAFF cells of GENO, TREND,
+// ALLELIC, DOM, REC
+struct ModelFields {
+    char lab[8], snp[32], aff[5][40], unaff[5][40];
+    const char* chr;
+    char a1, a2;
+    ModelFields(uint64_t r, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const uint8_t* nts,
+                const uint8_t* n_alleles, const uint32_t* c, const RowCounts& g) {
+        chr = assocfmt::chr_code(labels, chrom_idx[r], lab);
         snprintf(snp, sizeof snp, "rs%lld", (long long)ids[r]);
-        const char a1 = a1_of(nts, n_alleles, r), a2 = (char)nts[4 * r];
-        const RowCounts g(c);
-        double x[5];
-        model_chisq(c, x);
+        a1 = a1_of(nts, n_alleles, r);
+        a2 = (char)nts[4 * r];
         const unsigned A11 = c[2], A12 = c[1], A22 = c[0] - c[1] - c[2], U11 = c[7], U12 = c[6], U22 = c[5] - c[6] - c[7];
-        char aff[5][40], unaff[5][40];
         snprintf(aff[0], 40, "%u/%u/%u", A11, A12, A22);
         snprintf(unaff[0], 40, "%u/%u/%u", U11, U12, U22);
         memcpy(aff[1], aff[0], 40);
@@ -179,15 +213,77 @@ inline char* model_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, co
         snprintf(unaff[3], 40, "%u/%u", U11 + U12, U22);
         snprintf(aff[4], 40, "%u/%u", A11, A12 + A22);
         snprintf(unaff[4], 40, "%u/%u", U11, U12 + U22);
+    }
+};
+
+static const char* const kModelTest[5] = {"GENO", "TREND", "ALLELIC", "DOM", "REC"};
+
+inline char* model_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
+                          const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, char* o) {
+    static const int kDf[5] = {2, 1, 1, 1, 1};
+    for (uint64_t r = r0; r < r1; ++r) {
+        const uint32_t* c = counts + (uint64_t)kGenoWords * r;
+        const RowCounts g(c);
+        const ModelFields f(r, chrom_idx, labels, ids, nts, n_alleles, c, g);
+        double x[5];
+        model_chisq(c, x);
         for (int t = 0; t < 5; ++t) {
             const bool na = std::isnan(x[t]);
             char vx[32], vp[32], df[8];
             assocfmt::num(vx, 32, x[t]);
             assocfmt::num(vp, 32, na ? x[t] : chi2_sf(x[t], kDf[t]));
             snprintf(df, sizeof df, na ? "NA" : "%d", kDf[t]);
-            o += sprintf(o, "%4s %12s %4c %4c %8s %14s %14s %12s %4s %12s\n", chr, snp, a1, a2, kTest[t], aff[t], unaff[t], vx,
-                         df, vp);
+            o += sprintf(o, "%4s %12s %4c %4c %8s %14s %14s %12s %4s %12s\n", f.chr, f.snp, f.a1, f.a2, kModelTest[t], f.aff[t],
+                         f.unaff[t], vx, df, vp);
         }
+    }
+    return o;
+}
+
+// "%.4g" of the P whose log10 is l: 0 where 10^l underflows, NA for NaN
+inline int fisher_p(char* p, size_t cap, double l) { return assocfmt::num(p, cap, std::isnan(l) ? l : std::pow(10.0, l)); }
+
+// Fisher .model lines: GENO, TREND, ALLELIC, DOM, REC; TREND keeps its asymptotic P, the others print the Fisher P of
+// `log10p` ([rows][4]: GENO, ALLELIC, DOM, REC)
+inline char* model_fisher_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
+                                 const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, const double* log10p,
+                                 char* o) {
+    for (uint64_t r = r0; r < r1; ++r) {
+        const uint32_t* c = counts + (uint64_t)kGenoWords * r;
+        const RowCounts g(c);
+        const ModelFields f(r, chrom_idx, labels, ids, nts, n_alleles, c, g);
+        const double* l = log10p + 4 * r;
+        for (int t = 0; t < 5; ++t) {
+            char vp[32];
+            if (t == 1) {
+                const double x = chi2_trend(g);
+                assocfmt::num(vp, 32, std::isnan(x) ? x : chi2_sf(x, 1));
+            } else {
+                fisher_p(vp, 32, l[t == 0 ? 0 : t - 1]);
+            }
+            o += sprintf(o, "%4s %12s %4c %4c %8s %14s %14s %12s\n", f.chr, f.snp, f.a1, f.a2, kModelTest[t], f.aff[t],
+                         f.unaff[t], vp);
+        }
+    }
+    return o;
+}
+
+// .assoc.fisher lines: F_A, F_U and OR of the allele counts (haploid cells included), as in .assoc; P = Fisher ALLELIC
+inline char* assoc_fisher_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
+                                 const int64_t* position, const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts,
+                                 const double* log10p, char* o) {
+    for (uint64_t r = r0; r < r1; ++r) {
+        const RowCounts g(counts + (uint64_t)kGenoWords * r);
+        const assocfmt::AlleleStats s(g.alt_a, g.alt_a + g.ref_a, g.alt_u, g.alt_u + g.ref_u);
+        char lab[8], snp[32], v[4][32];
+        const char* chr = assocfmt::chr_code(labels, chrom_idx[r], lab);
+        snprintf(snp, sizeof snp, "rs%lld", (long long)ids[r]);
+        assocfmt::num(v[0], 32, s.f_a);
+        assocfmt::num(v[1], 32, s.f_u);
+        fisher_p(v[2], 32, log10p[4 * r + 1]);
+        assocfmt::num(v[3], 32, s.odds);
+        o += sprintf(o, "%4s %12s %10lld %4c %8s %8s %4c %12s %12s\n", chr, snp, (long long)position[r], a1_of(nts, n_alleles, r),
+                     v[0], v[1], (char)nts[4 * r], v[2], v[3]);
     }
     return o;
 }
@@ -219,6 +315,6 @@ inline char* hardy_serial(uint64_t r0, uint64_t r1, const int32_t* chrom_idx, co
     return o;
 }
 
-constexpr uint64_t kModelLineBytes = 5 * 192, kHardyLineBytes = 3 * 192;   // output room a row
+constexpr uint64_t kModelLineBytes = 5 * 192, kHardyLineBytes = 3 * 192, kAssocLineBytes = 192;   // output room a row
 
 }  // namespace modelfmt

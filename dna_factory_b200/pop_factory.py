@@ -26,7 +26,7 @@ from datetime import datetime
 
 import numpy
 
-from . import _native, assoc, model, partition, host
+from . import _native, assoc, fisher, model, partition, host
 from . import tabix
 from .tabix import TabixBuilder
 from .snp import (CHROMOSOME_LIST, CHROMOSOME_MAX_POSITION, CHROMOSOME_PROB, SNPTuples, SnpFactory, SnpTable,  # noqa: F401
@@ -58,7 +58,7 @@ def validate_assoc_table(table):
 
 
 def validate_assoc_population(control_size, test_size, flag="--assoc"):
-    """--assoc and --model compare cases with controls: both groups must be non-empty."""
+    """--assoc, --model and --fisher compare cases with controls: both groups must be non-empty."""
     if control_size <= 0 or test_size <= 0:
         raise ValueError("%s needs cases and controls (-s %d, -c %d)" % (flag, test_size, control_size))
 
@@ -206,7 +206,7 @@ class PopulationFactory:
     def __init__(self, num_processes=1, generate_snps=False, male_odds=0.5, deleterious_config=None,
                  deleterious_list_path=None, sample_id_offset=0, snps_path=None, output_path=None, seed=None,
                  gpus=1, gpu_select=False, tbi=False, bed=False, assoc=False, model=False,
-                 hardy=False):
+                 hardy=False, fisher=False):
         self.deleterious = {}
         self.ordered_snps = []
         self.snp_table = None
@@ -236,6 +236,8 @@ class PopulationFactory:
         self.hardy = bool(hardy)
         self.geno_counts = None      # uint32[rows, 10] genotype counts of the last write_vcf_snps (--model / --hardy)
         self.hwe_p = None            # float64[rows, 3] Hardy-Weinberg exact P (ALL, AFF, UNAFF) of the same rows
+        self.fisher = bool(fisher)
+        self.fisher_log10p = None    # float64[rows, 4] Fisher log10 P (GENO, ALLELIC, DOM, REC) of the same rows (--fisher)
 
     # ------------------------------------------------------------------------------------------ orchestration
     def generate_population(self, control_size, test_size, min_freq, max_snps, compression_level=6):
@@ -244,6 +246,8 @@ class PopulationFactory:
             validate_assoc_population(control_size, test_size)
         if self.model:
             validate_assoc_population(control_size, test_size, "--model")
+        if self.fisher:
+            validate_assoc_population(control_size, test_size, "--fisher")
         clock_seed = int(datetime.now().strftime("%H%M%S"))
         numpy.random.seed(clock_seed)
         if self.seed is None:
@@ -345,6 +349,8 @@ class PopulationFactory:
             validate_biallelic_table(snps, "--model", "the genotypic tests count biallelic SNPs only")
         if self.hardy:
             validate_biallelic_table(snps, "--hardy", "the Hardy-Weinberg tests count biallelic SNPs only")
+        if self.fisher:
+            validate_biallelic_table(snps, "--fisher", "the Fisher exact tests count biallelic SNPs only")
         groups = PopulationFactory.pick_deleterious_groups(list(self.deleterious.values()), test_size)
         fam_data = self.generate_fam_file(control_size, test_size, male_odds, groups)
         main_file = self.population_dir + "population.vcf.gz"
@@ -375,6 +381,8 @@ class PopulationFactory:
                 self.output_assoc(snps)
             if self.model or self.hardy:
                 self.output_model(snps)
+            if self.fisher:
+                self.output_fisher(snps)
         finally:
             engine.close()
             if bed_fd is not None:
@@ -406,13 +414,33 @@ class PopulationFactory:
             with open(self.population_dir + "population.hwe", "wb") as f:
                 f.write(model.hardy_bytes(table, self.geno_counts, self.hwe_p))
 
+    def output_fisher(self, table):
+        """population.assoc.fisher, population.model.fisher and deleterious_fisher.txt (--fisher) from the genotype
+        counts and Fisher log10 P write_vcf_snps took on the GPU."""
+        with open(self.population_dir + "population.assoc.fisher", "wb") as f:
+            f.write(fisher.assoc_fisher_bytes(table, self.geno_counts, self.fisher_log10p))
+        with open(self.population_dir + "population.model.fisher", "wb") as f:
+            f.write(fisher.model_fisher_bytes(table, self.geno_counts, self.fisher_log10p))
+        text, summary = fisher.deleterious_fisher_report(table, self.deleterious, self.geno_counts, self.fisher_log10p,
+                                                         self.override_rows)
+        with open(self.population_dir + "deleterious_fisher.txt", "wb") as f:
+            f.write(text)
+        print(summary, flush=True)
+
+    def _geno_tests(self):
+        return self.model or self.hardy or self.fisher
+
+    def _genotype_tests(self, eng, rows, seed):
+        """One dnaf_genotype_tests call for --model / --hardy / --fisher: (counts, HWE P or None, log10 P or None)."""
+        return eng.genotype_tests(0, rows, seed, hwe=self.model or self.hardy, fisher=self.fisher)
+
     # ------------------------------------------------------------------------------------------ the GPU seam
     def write_vcf_snps(self, fam_data, snps, file, engine=None, bed_fd=None):
         """Rows of `snps` (in order) for `fam_data`, appended to `file` -- the reference's seam
         (pop_factory.py:417-469).  `snps` is a list of SNPTuples or a SnpTable; `file` a BgzfSink.  With `bed_fd`
         (an open population.bed that holds the 3 magic bytes) the same rows also go there as PLINK 1 .bed rows.  With
-        --assoc the case/control allele counts of the same rows land in self.assoc_counts, with --model / --hardy their
-        genotype counts and exact-test P in self.geno_counts / self.hwe_p."""
+        --assoc the case/control allele counts of the same rows land in self.assoc_counts, with --model / --hardy /
+        --fisher their genotype counts and exact-test P in self.geno_counts / self.hwe_p / self.fisher_log10p."""
         t0 = time.time()
         level = getattr(file, "compresslevel", getattr(self, "_level", 6))
         seed = self.seed if self.seed is not None else int(datetime.now().strftime("%H%M%S"))
@@ -452,8 +480,8 @@ class PopulationFactory:
                     self.bed_stats.append(eng.generate_bed_fd_at(0, n_rows, seed, bed_fd, len(BED_MAGIC)))
                 if self.assoc:
                     self.assoc_counts = eng.allele_counts(0, n_rows, seed)
-                if self.model or self.hardy:
-                    self.geno_counts, self.hwe_p = eng.genotype_counts(0, n_rows, seed)
+                if self._geno_tests():
+                    self.geno_counts, self.hwe_p, self.fisher_log10p = self._genotype_tests(eng, n_rows, seed)
             finally:
                 if own:
                     eng.close()
@@ -470,7 +498,8 @@ class PopulationFactory:
         nothing is spooled or copied twice.  Every rank holds only its own slice of the SNP table; the Philox row
         counter of its local row r is bounds[g] + r (dnaf_set_row_base).  .bed rows have a fixed size, so rank g
         pwrite()s its rows at 3 + bounds[g] * ceil(N/4) of population.bed without a sizing pass.  With --assoc every
-        rank counts its own rows after its VCF write; the slices are joined in rank order (so do --model / --hardy)."""
+        rank counts its own rows after its VCF write; the slices are joined in rank order (so do --model / --hardy /
+        --fisher)."""
         bounds = partition.row_bounds(n_rows, gpus)
         n_dev = max(1, _native.device_count())      # more ranks than devices: ranks share devices round-robin
         errors = []
@@ -516,8 +545,8 @@ class PopulationFactory:
                     blocks[g] = eng.block_log_get()
                 if self.assoc:
                     counts[g] = eng.allele_counts(0, hi - lo, seed)
-                if self.model or self.hardy:
-                    geno[g] = eng.genotype_counts(0, hi - lo, seed)
+                if self._geno_tests():
+                    geno[g] = self._genotype_tests(eng, hi - lo, seed)
             except BaseException as e:  # noqa
                 errors.append(e)
 
@@ -534,9 +563,12 @@ class PopulationFactory:
         file._handle.seek(base + sum(sizes))      # the sink appends the EOF block behind the last rank's stream
         if self.assoc:
             self.assoc_counts = numpy.concatenate(counts)
-        if self.model or self.hardy:
+        if self._geno_tests():
             self.geno_counts = numpy.concatenate([q[0] for q in geno])
-            self.hwe_p = numpy.concatenate([q[1] for q in geno])
+            if self.model or self.hardy:
+                self.hwe_p = numpy.concatenate([q[1] for q in geno])
+            if self.fisher:
+                self.fisher_log10p = numpy.concatenate([q[2] for q in geno])
         if index is not None:
             off = numpy.concatenate([numpy.zeros(1, numpy.uint64)] +
                                     [r[1:] + numpy.uint64(sum(int(q[-1]) for q in row_off[:g])) for g, r in enumerate(row_off)])
@@ -616,6 +648,10 @@ def parse_cmd_args(args):
     ap.add_argument("--hardy", action="store_true",
                     help="also write population.hwe (Hardy-Weinberg exact tests of every SNP in all samples, cases and "
                          "controls, on the GPU); every SNP must be biallelic")
+    ap.add_argument("--fisher", action="store_true",
+                    help="also write population.assoc.fisher and population.model.fisher (Fisher's exact case/control "
+                         "tests of every SNP: ALLELIC, GENO, DOM, REC, no cell rule, on the GPU) and deleterious_fisher.txt "
+                         "(how every planted deleterious SNP fares under them); every SNP must be biallelic")
     return ap.parse_args(args)
 
 
@@ -629,7 +665,7 @@ def main(sys_args):
                                 male_odds=args.male_odds, deleterious_config=args.deleterious_config,
                                 snps_path=args.snps_file, output_path=args.outdir, seed=args.seed, gpus=args.gpus,
                                 gpu_select=args.gpu_select, tbi=args.tbi, bed=args.bed, assoc=args.assoc,
-                                model=args.model, hardy=args.hardy)
+                                model=args.model, hardy=args.hardy, fisher=args.fisher)
     factory.generate_population(args.control_size, args.size, args.min_freq, args.max_snps, args.compression_level)
 
 

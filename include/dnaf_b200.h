@@ -263,6 +263,47 @@ int dnaf_genotype_counts_device(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_
  */
 int dnaf_hwe_exact(dnaf_ctx* ctx, uint64_t n, const uint32_t* geno, double* p);
 /*
+ * The counts, Hardy-Weinberg P and Fisher exact tests of rows [row_begin,row_end) in one call: counts and hwe_p as in
+ * dnaf_genotype_counts; fisher_log10p (NULL: not computed) is [rows][4], log10 of the two-sided Fisher exact P
+ * (dnaf_fisher_exact) of GENO (the diploid 2x3 table n11 / n12 / n22 of cases and controls), ALLELIC (ALT / REF
+ * alleles, haploid cells included, as in .assoc), DOM (n11 + n12 / n22) and REC (n11 / n12 + n22), each computed on
+ * the device from the pass's counts.  Y and MT rows have no diploid cell, so only their ALLELIC test is defined (the
+ * others are NaN).  A NULL hwe_p or fisher_log10p is not computed.  dnaf_genotype_counts is this call with
+ * fisher_log10p = NULL.  Rows with more than 2 alleles: DNAF_E_INPUT before any GPU work, naming the row.
+ */
+int dnaf_genotype_tests(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* counts,
+                        double* hwe_p, double* fisher_log10p, dnaf_stats* stats);
+/* Same work, results left in device memory (the exact tests only where with_hwe / with_fisher != 0). */
+int dnaf_genotype_tests_device(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, int with_hwe,
+                               int with_fisher, dnaf_stats* stats);
+/*
+ * log10 of the two-sided Fisher exact P of n case/control tables, tables[i] = (x1, x2, x3, y1, y2, y3) (case row, then
+ * control row), computed on the device by the kernel dnaf_genotype_tests uses.  With both margins fixed a table has
+ * probability prod_j C(x_j + y_j, x_j) / C(N, R); P is the sum of the probabilities of every table whose probability
+ * is <= (1 + 1e-7) times the observed one's (the tie rule of dnaf_hwe_exact).  A table with one empty column is the 2x2
+ * test over the other two.  Double precision, with the scale of P kept in a separate exponent, so log10 P stays exact
+ * far below the double range; NaN where a row margin is 0 or fewer than two columns are non-empty.  Synchronous.
+ */
+int dnaf_fisher_exact(dnaf_ctx* ctx, uint64_t n, const uint32_t* tables, double* log10p);
+/*
+ * The .assoc.fisher body lines of n rows from their genotype counts and Fisher log10 P (dnaf_genotype_tests; labels
+ * and nts as in dnaf_format_assoc): columns CHR SNP BP A1 F_A F_U A2 P OR (PLINK 1.9's plink.assoc.fisher), F_A, F_U
+ * and OR from the allele counts as in .assoc, P the Fisher ALLELIC P printed "%.4g" (0 where 10^log10P underflows, NA
+ * for NaN).  `out` holds at least 192 bytes per row.  Returns the bytes written.
+ */
+uint64_t dnaf_format_assoc_fisher(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
+                                  const int64_t* position, const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts,
+                                  const double* log10p, char* out);
+/*
+ * The Fisher .model body lines (plink --model fisher): five lines a row, GENO, TREND, ALLELIC, DOM, REC, with columns
+ * CHR SNP A1 A2 TEST AFF UNAFF P; AFF and UNAFF as in dnaf_format_model.  TREND prints its asymptotic chi-square P; the
+ * others print the Fisher P of log10p, with no cell rule, as in dnaf_format_assoc_fisher.  `out` holds at least 960
+ * bytes per row.  Returns the bytes written.
+ */
+uint64_t dnaf_format_model_fisher(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids,
+                                  const uint8_t* nts, const uint8_t* n_alleles, const uint32_t* counts, const double* log10p,
+                                  char* out);
+/*
  * The .model body lines of n rows from their genotype counts (host code, no context, no GPU; labels and nts as in
  * dnaf_format_assoc): five lines a row, GENO, TREND, ALLELIC, DOM, REC, with columns CHR SNP A1 A2 TEST AFF UNAFF
  * CHISQ DF P.  With n11 / n12 / n22 the diploid ALT/ALT, het and REF/REF counts of a group, AFF and UNAFF are
