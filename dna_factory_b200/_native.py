@@ -45,7 +45,7 @@ EXPORTS = ["dnaf_abi_version", "dnaf_device_count", "dnaf_last_error", "dnaf_cre
            "dnaf_generate_bed_device", "dnaf_allele_counts", "dnaf_allele_counts_device", "dnaf_format_assoc",
            "dnaf_genotype_counts", "dnaf_genotype_counts_device", "dnaf_hwe_exact", "dnaf_format_model", "dnaf_format_hardy",
            "dnaf_genotype_tests", "dnaf_genotype_tests_device", "dnaf_fisher_exact", "dnaf_format_assoc_fisher",
-           "dnaf_format_model_fisher"]
+           "dnaf_format_model_fisher", "dnaf_perm_case_masks", "dnaf_mperm", "dnaf_mperm_device", "dnaf_format_mperm"]
 
 _lib = None
 
@@ -105,6 +105,11 @@ def load():
                                            ctypes.POINTER(ctypes.c_int64), u8p, u8p, u32p, f64p, u8p]),
         "dnaf_format_model_fisher": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64),
                                            u8p, u8p, u32p, f64p, u8p]),
+        "dnaf_perm_case_masks": (i32, [vp, u64, u64, ctypes.c_uint32, u32p, u32p]),
+        "dnaf_mperm": (i32, [vp, u64, u64, u64, ctypes.c_uint32, f64p, u32p, f64p, sp]),
+        "dnaf_mperm_device": (i32, [vp, u64, u64, u64, ctypes.c_uint32, sp]),
+        "dnaf_format_mperm": (u64, [u64, ctypes.POINTER(ctypes.c_int32), ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64), f64p,
+                                    u8p]),
         "dnaf_genotypes": (i32, [vp, u64, u64, u64, u8p, u64]),
         "dnaf_text": (i32, [vp, u64, u64, u64, u8p, u64, u64p]),
         "dnaf_bgzf_compress": (i32, [vp, u8p, u64, u8p, u64, sp]),
@@ -436,6 +441,43 @@ class Engine:
                                                 l.ctypes.data_as(ctypes.POINTER(ctypes.c_double))))
         return l
 
+    # -- max(T) permutation tests of ALLELIC and REC (pop_factory --mperm)
+    def perm_case_masks(self, seed, first_perm, n_perm):
+        """(uint32[n_perm, ceil(N/32)], uint32[n_perm, 2]): the case masks of permutations first_perm ..
+        first_perm + n_perm - 1 (bit i & 31 of word i >> 5 = sample i is a case) and their (male, female) cases
+        (include/dnaf_b200.h, dnaf_perm_case_masks)."""
+        masks = np.zeros((n_perm, (self.n_samples + 31) // 32), np.uint32)
+        sexc = np.zeros((n_perm, 2), np.uint32)
+        u32p = ctypes.POINTER(ctypes.c_uint32)
+        self._check(self._lib.dnaf_perm_case_masks(self._h, seed, first_perm, n_perm, masks.ctypes.data_as(u32p),
+                                                   sexc.ctypes.data_as(u32p)))
+        return masks, sexc
+
+    def mperm(self, row_begin, row_end, seed, n_perm):
+        """(float64[rows, 2], uint32[rows, 2], float64[n_perm, 2]) of rows [row_begin,row_end) under n_perm permutations:
+        the observed ALLELIC and REC statistics (NaN: no test), how many permutations reach them, and every
+        permutation's maximum over the rows (include/dnaf_b200.h, dnaf_mperm)."""
+        return self.mperm_stats(row_begin, row_end, seed, n_perm)[:3]
+
+    def mperm_stats(self, row_begin, row_end, seed, n_perm):
+        """Same -> (t_obs, exceed, max_t, stats dict)."""
+        rows = max(row_end - row_begin, 0)
+        t_obs = np.zeros((rows, 2), np.float64)
+        exceed = np.zeros((rows, 2), np.uint32)
+        max_t = np.zeros((n_perm, 2), np.float64)
+        f64p = ctypes.POINTER(ctypes.c_double)
+        st = Stats()
+        self._check(self._lib.dnaf_mperm(self._h, row_begin, row_end, seed, n_perm, t_obs.ctypes.data_as(f64p),
+                                         exceed.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)), max_t.ctypes.data_as(f64p),
+                                         ctypes.byref(st)))
+        return t_obs, exceed, max_t, st.as_dict()
+
+    def mperm_device(self, row_begin, row_end, seed, n_perm):
+        """Same work, results left on the device; returns stats dict."""
+        st = Stats()
+        self._check(self._lib.dnaf_mperm_device(self._h, row_begin, row_end, seed, n_perm, ctypes.byref(st)))
+        return st.as_dict()
+
     # -- parity gates
     def genotypes(self, row_begin, row_end, seed):
         rows = row_end - row_begin
@@ -644,6 +686,23 @@ def format_model_fisher(ids, chrom_idx, labels, n_alleles, nts, counts, log10p):
                                         ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _u8(nt), _u8(k),
                                         cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)),
                                         l.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), _u8(out))
+    return out[:used].tobytes()
+
+
+def format_mperm(ids, chrom_idx, labels, emp):
+    """.mperm body lines (dnaf_format_mperm: CHR SNP EMP1 EMP2, "%.4g", NA for NaN) of a column-form SNP table and its
+    float64[rows, 2] (EMP1, EMP2) -> bytes."""
+    lib = load()
+    n = len(ids)
+    if n == 0:
+        return b""
+    ids = np.ascontiguousarray(ids, np.int64)
+    ci = np.ascontiguousarray(chrom_idx, np.int32)
+    e = np.ascontiguousarray(emp, np.float64).reshape(n, 2)
+    out = np.empty(n * 96 + 16, np.uint8)
+    used = lib.dnaf_format_mperm(n, ci.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), _label_block(labels),
+                                 ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), e.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+                                 _u8(out))
     return out[:used].tobytes()
 
 

@@ -9,7 +9,8 @@
 // or the fused kernel (k_fused.cuh) followed by scan -> compact -> D2H -> sink.  The PLINK 1 .bed writer
 // (dnaf_generate_bed*) is one kernel per pass, k_bed -> D2H -> sink (host_bed.h); the case/control allele counts
 // (dnaf_allele_counts*) are one kernel per pass too, k_assoc -> D2H (host_assoc.h), and the genotype counts
-// (dnaf_genotype_counts*) k_geno -> (k_hwe) -> D2H through the same pass driver (host_geno.h).
+// (dnaf_genotype_counts*) k_geno -> (k_hwe) -> D2H through the same pass driver (host_geno.h), and the permutation
+// tests (dnaf_mperm*) k_geno -> k_mperm_planes -> k_mperm through it too (host_mperm.h).
 #include <unistd.h>
 
 #include <algorithm>
@@ -33,6 +34,7 @@
 #include "k_fused.cuh"
 #include "k_fused_text.cuh"
 #include "k_geno.cuh"
+#include "k_mperm.cuh"
 #include "k_sample_format.cuh"
 #include "k_select.cuh"
 #include "snps_json.h"
@@ -50,6 +52,7 @@ using namespace dnaf;
 #include "host_bed.h"
 #include "host_assoc.h"
 #include "host_geno.h"
+#include "host_mperm.h"
 
 
 // ================================================================================================ C ABI
@@ -206,6 +209,8 @@ int dnaf_set_samples(dnaf_ctx* c, uint32_t n, const uint8_t* sex, const uint8_t*
     xoff[n] = acc;
     c->n = n;
     c->males = males;
+    c->ncase = 0;
+    for (uint32_t i = 0; i < n; ++i) c->ncase += !is_control[i];
     // body bytes incl. the '\n' that replaces the last '\t' ("\t".join(...) + "\n", pop_factory.py:508)
     c->body[kAuto] = n ? 4u * n : 1u;
     c->body[kX] = n ? acc : 1u;
@@ -690,6 +695,34 @@ uint64_t dnaf_format_model_fisher(uint64_t n, const int32_t* chrom_idx, const ch
     if (!n || !chrom_idx || !labels || !ids || !nts || !n_alleles || !counts || !log10p || !out) return 0;
     return assocfmt::sliced(n, modelfmt::kModelLineBytes, out, [&](uint64_t r0, uint64_t r1, char* o) {
         return modelfmt::model_fisher_serial(r0, r1, chrom_idx, labels, ids, nts, n_alleles, counts, log10p, o);
+    });
+}
+
+int dnaf_perm_case_masks(dnaf_ctx* c, uint64_t seed, uint64_t first_perm, uint32_t n_perm, uint32_t* masks,
+                         uint32_t* sex_counts) {
+    if (!c) return DNAF_E_ARG;
+    const int rc = perm_masks_impl(c, seed, first_perm, n_perm, masks, sex_counts);
+    if (rc) quiesce(c);
+    return rc;
+}
+
+int dnaf_mperm(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t n_perm, double* t_obs,
+               uint32_t* exceed, double* max_t, dnaf_stats* stats) {
+    if (!c) return DNAF_E_ARG;
+    if ((!t_obs || !exceed) && row_end > row_begin) return fail(c, DNAF_E_ARG, "t_obs / exceed is NULL");
+    if (!max_t && n_perm) return fail(c, DNAF_E_ARG, "max_t is NULL");
+    return mperm_impl(c, row_begin, row_end, seed, n_perm, t_obs, exceed, max_t, stats);
+}
+
+int dnaf_mperm_device(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t n_perm, dnaf_stats* stats) {
+    return mperm_impl(c, row_begin, row_end, seed, n_perm, nullptr, nullptr, nullptr, stats);
+}
+
+uint64_t dnaf_format_mperm(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const double* emp,
+                           char* out) {
+    if (!n || !chrom_idx || !labels || !ids || !emp || !out) return 0;
+    return assocfmt::sliced(n, mpermfmt::kLineBytes, out, [&](uint64_t r0, uint64_t r1, char* o) {
+        return mpermfmt::lines_serial(r0, r1, chrom_idx, labels, ids, emp, o);
     });
 }
 

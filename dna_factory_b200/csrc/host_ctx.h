@@ -203,6 +203,11 @@ struct dnaf_ctx {
                                            // (k_geno: [rows][10]; dnaf_hwe_exact: the uploaded triples)
     DevBuf d_hwe;                          // k_hwe: a pass's [rows][3] P (dnaf_hwe_exact: [n])
     DevBuf d_fisher;                       // k_fisher: a pass's [rows][4] log10 P (dnaf_fisher_exact: [n])
+    uint32_t ncase = 0;                    // samples with is_control == 0
+    DevBuf d_pmask;                        // k_perm_masks: case masks [perms][pitch], then (male, female) cases [perms][2]
+    DevBuf d_planes;                       // k_mperm_planes: a pass's A and B planes, [rows][pitch] each
+    DevBuf d_mrow;                         // k_mperm: a pass's T_obs [rows][2] (double), then exceedances [rows][2]
+    DevBuf d_maxt;                         // k_mperm: [perms][2] maxima, zeroed once per call
     cudaEvent_t ev_bed[2] = {};            // k_bed calls: first launch, last kernel end
     std::vector<uint32_t> h_seg_crc_x;     // L(template body) per X segment
     std::vector<uint32_t> h_xoff;

@@ -7,10 +7,8 @@
 
 namespace {
 
-int geno_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* out, double* hwe_out,
-                bool with_hwe, double* fisher_out, bool with_fisher, dnaf_stats* st) {
-    int rc = check_biallelic(c, row_begin, row_end, "the genotype count");
-    if (rc) return rc;
+// k_geno's arguments for the context's samples, SNPs and forced minors (row0 and counts are set per pass)
+GenoArgs geno_args(const dnaf_ctx* c, uint64_t seed) {
     GenoArgs a;
     a.cls = c->d_cls.as<uint8_t>();
     a.k = c->d_k.as<uint8_t>();
@@ -26,6 +24,14 @@ int geno_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed
     a.tiles = std::max<uint32_t>(1u, (a.groups + kGenoThreads - 1u) / kGenoThreads);
     a.k0 = (uint32_t)seed;
     a.k1 = (uint32_t)(seed >> 32);
+    return a;
+}
+
+int geno_passes(dnaf_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t* out, double* hwe_out,
+                bool with_hwe, double* fisher_out, bool with_fisher, dnaf_stats* st) {
+    int rc = check_biallelic(c, row_begin, row_end, "the genotype count");
+    if (rc) return rc;
+    GenoArgs a = geno_args(c, seed);
     constexpr uint64_t kCountBytes = 4u * kGenoWords, kFisherBytes = kFisherTests * sizeof(double);
     const uint64_t row_bytes = kCountBytes + (with_hwe ? 3u * sizeof(double) : 0u) + (with_fisher ? kFisherBytes : 0u);
     if ((with_hwe || with_fisher) && row_end > row_begin) {
@@ -143,11 +149,7 @@ struct RowCounts {
 
 inline double nan_() { return std::nan(""); }
 
-// Pearson 2x2 (cases a, b / controls c, d), no continuity correction; the .assoc expression
-inline double chi2_2x2(double a, double b, double c, double d) {
-    const double den = (a + b) * (c + d) * (a + c) * (b + d);
-    return den > 0 ? (a + b + c + d) * (a * d - b * c) * (a * d - b * c) / den : nan_();
-}
+// chi2_2x2, the Pearson 2x2 of .assoc, ALLELIC, DOM and REC: k_mperm.cuh (shared with the permutation kernel)
 
 // Pearson 2x3 over the genotype cells
 inline double chi2_geno(const RowCounts& g) {

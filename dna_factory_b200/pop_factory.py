@@ -26,7 +26,7 @@ from datetime import datetime
 
 import numpy
 
-from . import _native, assoc, fisher, model, partition, host
+from . import _native, assoc, fisher, model, mperm, partition, host
 from . import tabix
 from .tabix import TabixBuilder
 from .snp import (CHROMOSOME_LIST, CHROMOSOME_MAX_POSITION, CHROMOSOME_PROB, SNPTuples, SnpFactory, SnpTable,  # noqa: F401
@@ -58,7 +58,7 @@ def validate_assoc_table(table):
 
 
 def validate_assoc_population(control_size, test_size, flag="--assoc"):
-    """--assoc, --model and --fisher compare cases with controls: both groups must be non-empty."""
+    """--assoc, --model, --fisher and --mperm compare cases with controls: both groups must be non-empty."""
     if control_size <= 0 or test_size <= 0:
         raise ValueError("%s needs cases and controls (-s %d, -c %d)" % (flag, test_size, control_size))
 
@@ -206,7 +206,7 @@ class PopulationFactory:
     def __init__(self, num_processes=1, generate_snps=False, male_odds=0.5, deleterious_config=None,
                  deleterious_list_path=None, sample_id_offset=0, snps_path=None, output_path=None, seed=None,
                  gpus=1, gpu_select=False, tbi=False, bed=False, assoc=False, model=False,
-                 hardy=False, fisher=False):
+                 hardy=False, fisher=False, mperm=None):
         self.deleterious = {}
         self.ordered_snps = []
         self.snp_table = None
@@ -238,6 +238,8 @@ class PopulationFactory:
         self.hwe_p = None            # float64[rows, 3] Hardy-Weinberg exact P (ALL, AFF, UNAFF) of the same rows
         self.fisher = bool(fisher)
         self.fisher_log10p = None    # float64[rows, 4] Fisher log10 P (GENO, ALLELIC, DOM, REC) of the same rows (--fisher)
+        self.mperm = mperm           # permutations of --mperm (None: no permutation tests)
+        self.mperm_result = None     # (T_obs [rows, 2], exceedances [rows, 2], maxima [N, 2]) of ALLELIC and REC (--mperm)
 
     # ------------------------------------------------------------------------------------------ orchestration
     def generate_population(self, control_size, test_size, min_freq, max_snps, compression_level=6):
@@ -248,6 +250,10 @@ class PopulationFactory:
             validate_assoc_population(control_size, test_size, "--model")
         if self.fisher:
             validate_assoc_population(control_size, test_size, "--fisher")
+        if self.mperm is not None:
+            if self.mperm < 1:
+                raise ValueError("--mperm needs at least 1 permutation (got %d)" % self.mperm)
+            validate_assoc_population(control_size, test_size, "--mperm")
         clock_seed = int(datetime.now().strftime("%H%M%S"))
         numpy.random.seed(clock_seed)
         if self.seed is None:
@@ -351,6 +357,8 @@ class PopulationFactory:
             validate_biallelic_table(snps, "--hardy", "the Hardy-Weinberg tests count biallelic SNPs only")
         if self.fisher:
             validate_biallelic_table(snps, "--fisher", "the Fisher exact tests count biallelic SNPs only")
+        if self.mperm:
+            validate_biallelic_table(snps, "--mperm", "the permutation tests count biallelic SNPs only")
         groups = PopulationFactory.pick_deleterious_groups(list(self.deleterious.values()), test_size)
         fam_data = self.generate_fam_file(control_size, test_size, male_odds, groups)
         main_file = self.population_dir + "population.vcf.gz"
@@ -383,6 +391,8 @@ class PopulationFactory:
                 self.output_model(snps)
             if self.fisher:
                 self.output_fisher(snps)
+            if self.mperm:
+                self.output_mperm(snps)
         finally:
             engine.close()
             if bed_fd is not None:
@@ -427,6 +437,20 @@ class PopulationFactory:
             f.write(text)
         print(summary, flush=True)
 
+    def output_mperm(self, table):
+        """population.assoc.mperm, population.model.rec.mperm and deleterious_mperm.txt (--mperm) from the permutation
+        results write_vcf_snps took on the GPU."""
+        t_obs, exceed, max_t = self.mperm_result
+        emp1, emp2 = mperm.empirical(t_obs, exceed, max_t)
+        with open(self.population_dir + "population.assoc.mperm", "wb") as f:
+            f.write(mperm.mperm_bytes(table, emp1, emp2, 0))
+        with open(self.population_dir + "population.model.rec.mperm", "wb") as f:
+            f.write(mperm.mperm_bytes(table, emp1, emp2, 1))
+        text, summary = mperm.deleterious_mperm_report(table, self.deleterious, t_obs, exceed, max_t, self.override_rows)
+        with open(self.population_dir + "deleterious_mperm.txt", "wb") as f:
+            f.write(text)
+        print(summary, flush=True)
+
     def _geno_tests(self):
         return self.model or self.hardy or self.fisher
 
@@ -440,7 +464,8 @@ class PopulationFactory:
         (pop_factory.py:417-469).  `snps` is a list of SNPTuples or a SnpTable; `file` a BgzfSink.  With `bed_fd`
         (an open population.bed that holds the 3 magic bytes) the same rows also go there as PLINK 1 .bed rows.  With
         --assoc the case/control allele counts of the same rows land in self.assoc_counts, with --model / --hardy /
-        --fisher their genotype counts and exact-test P in self.geno_counts / self.hwe_p / self.fisher_log10p."""
+        --fisher their genotype counts and exact-test P in self.geno_counts / self.hwe_p / self.fisher_log10p, with
+        --mperm the permutation results in self.mperm_result."""
         t0 = time.time()
         level = getattr(file, "compresslevel", getattr(self, "_level", 6))
         seed = self.seed if self.seed is not None else int(datetime.now().strftime("%H%M%S"))
@@ -482,6 +507,8 @@ class PopulationFactory:
                     self.assoc_counts = eng.allele_counts(0, n_rows, seed)
                 if self._geno_tests():
                     self.geno_counts, self.hwe_p, self.fisher_log10p = self._genotype_tests(eng, n_rows, seed)
+                if self.mperm:
+                    self.mperm_result = eng.mperm(0, n_rows, seed, self.mperm)
             finally:
                 if own:
                     eng.close()
@@ -499,13 +526,14 @@ class PopulationFactory:
         counter of its local row r is bounds[g] + r (dnaf_set_row_base).  .bed rows have a fixed size, so rank g
         pwrite()s its rows at 3 + bounds[g] * ceil(N/4) of population.bed without a sizing pass.  With --assoc every
         rank counts its own rows after its VCF write; the slices are joined in rank order (so do --model / --hardy /
-        --fisher)."""
+        --fisher / --mperm; the --mperm maxima of the ranks join by elementwise max: a maximum composes over row
+        ranges)."""
         bounds = partition.row_bounds(n_rows, gpus)
         n_dev = max(1, _native.device_count())      # more ranks than devices: ranks share devices round-robin
         errors = []
         index = getattr(file, "index", None)
         blocks, row_off, sizes, engines = [None] * gpus, [None] * gpus, [0] * gpus, [None] * gpus
-        counts, geno = [None] * gpus, [None] * gpus
+        counts, geno, perm = [None] * gpus, [None] * gpus, [None] * gpus
         barrier = threading.Barrier(gpus)
         file.flush()   # the header blocks must be in the file: the ranks write behind them
         base = file._handle.tell()
@@ -547,6 +575,8 @@ class PopulationFactory:
                     counts[g] = eng.allele_counts(0, hi - lo, seed)
                 if self._geno_tests():
                     geno[g] = self._genotype_tests(eng, hi - lo, seed)
+                if self.mperm:
+                    perm[g] = eng.mperm(0, hi - lo, seed, self.mperm)
             except BaseException as e:  # noqa
                 errors.append(e)
 
@@ -569,6 +599,9 @@ class PopulationFactory:
                 self.hwe_p = numpy.concatenate([q[1] for q in geno])
             if self.fisher:
                 self.fisher_log10p = numpy.concatenate([q[2] for q in geno])
+        if self.mperm:
+            self.mperm_result = (numpy.concatenate([q[0] for q in perm]), numpy.concatenate([q[1] for q in perm]),
+                                 numpy.maximum.reduce([q[2] for q in perm]))
         if index is not None:
             off = numpy.concatenate([numpy.zeros(1, numpy.uint64)] +
                                     [r[1:] + numpy.uint64(sum(int(q[-1]) for q in row_off[:g])) for g, r in enumerate(row_off)])
@@ -652,6 +685,11 @@ def parse_cmd_args(args):
                     help="also write population.assoc.fisher and population.model.fisher (Fisher's exact case/control "
                          "tests of every SNP: ALLELIC, GENO, DOM, REC, no cell rule, on the GPU) and deleterious_fisher.txt "
                          "(how every planted deleterious SNP fares under them); every SNP must be biallelic")
+    ap.add_argument("--mperm", type=int, default=None, metavar="N",
+                    help="also write population.assoc.mperm and population.model.rec.mperm (max(T) permutation tests of "
+                         "ALLELIC and REC over N case/control permutations, on the GPU: EMP1 pointwise, EMP2 family-wise "
+                         "empirical P) and deleterious_mperm.txt (how every planted deleterious SNP fares under them); "
+                         "every SNP must be biallelic")
     return ap.parse_args(args)
 
 
@@ -665,7 +703,7 @@ def main(sys_args):
                                 male_odds=args.male_odds, deleterious_config=args.deleterious_config,
                                 snps_path=args.snps_file, output_path=args.outdir, seed=args.seed, gpus=args.gpus,
                                 gpu_select=args.gpu_select, tbi=args.tbi, bed=args.bed, assoc=args.assoc,
-                                model=args.model, hardy=args.hardy, fisher=args.fisher)
+                                model=args.model, hardy=args.hardy, fisher=args.fisher, mperm=args.mperm)
     factory.generate_population(args.control_size, args.size, args.min_freq, args.max_snps, args.compression_level)
 
 

@@ -324,6 +324,43 @@ uint64_t dnaf_format_model(uint64_t n, const int32_t* chrom_idx, const char* lab
 uint64_t dnaf_format_hardy(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const uint8_t* nts,
                            const uint8_t* n_alleles, const uint32_t* counts, const double* hwe_p, char* out);
 
+/*
+ * Case/control permutations of the samples of dnaf_set_samples (max(T) permutation tests).  Permutation p is a
+ * uniformly random subset of exactly ncase of the N samples (ncase = samples with is_control == 0), by selection
+ * sampling: for i = 0..N-1, with `need` starting at ncase, sample i is a case iff
+ *   (uint64)U(p,i) * (N - i) < (uint64)need << 32   (then need -= 1),
+ *   U(p,i) = philox4x32_10(ctr = (i >> 2, p, 0x4D505200, 0xFFFFFFFF), key = (seed_lo, seed_hi))[i & 3].
+ * This call writes permutations first_perm .. first_perm + n_perm - 1 (indices below 2^32): masks is
+ * [n_perm][ceil(N/32)], bit i & 31 of word i >> 5 set where sample i is a case; sex_counts is [n_perm][2], the male
+ * (sex == 1) and female cases.  Any ncase from 0 to N is drawn; n_perm == 0: DNAF_E_ARG.  Synchronous.
+ */
+int dnaf_perm_case_masks(dnaf_ctx* ctx, uint64_t seed, uint64_t first_perm, uint32_t n_perm, uint32_t* masks,
+                         uint32_t* sex_counts);
+/*
+ * max(T) permutation tests of rows [row_begin,row_end) under permutations 0 .. n_perm - 1: t_obs is [rows][2], the
+ * observed ALLELIC (the .assoc CHISQ, haploid cells included) and REC (2x2 Pearson n11 / n12 + n22 over the diploid
+ * cells, no cell rule) statistics, NaN where a denominator is 0 (no test; Y and MT rows have no REC).  exceed is
+ * [rows][2], the permutations whose statistic T_p >= T_obs (1 - 1e-7); max_t is [n_perm][2], the maximum of T_p over
+ * the rows with a test (0 where none has one).  Under permutation p the case margins follow from the row class and
+ * p's male and female cases (m, f): case alleles 2(m + f), 2f + m, m, m + f and case diploid cells m + f, f, 0, 0 on
+ * autosome, X, Y, MT rows; the row totals are those of dnaf_genotype_counts.  EMP1 = (exceed + 1) / (n_perm + 1),
+ * EMP2 = (#{p : max_t[p] >= T_obs (1 - 1e-7)} + 1) / (n_perm + 1).  max_t composes over row ranges by elementwise max.
+ * Rows with more than 2 alleles: DNAF_E_INPUT before any GPU work, naming the row; no cases, no controls or
+ * n_perm == 0: DNAF_E_ARG.
+ */
+int dnaf_mperm(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t n_perm, double* t_obs,
+               uint32_t* exceed, double* max_t, dnaf_stats* stats);
+/* Same work, results left in device memory. */
+int dnaf_mperm_device(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint32_t n_perm,
+                      dnaf_stats* stats);
+/*
+ * The .mperm body lines of n rows (PLINK 1.9's plink.assoc.mperm: CHR SNP EMP1 EMP2; labels as in dnaf_format_assoc):
+ * emp is [n][2] (EMP1, EMP2), printed "%.4g", NA for NaN.  `out` holds at least 96 bytes per row.  Returns the bytes
+ * written.
+ */
+uint64_t dnaf_format_mperm(uint64_t n, const int32_t* chrom_idx, const char* labels, const int64_t* ids, const double* emp,
+                           char* out);
+
 /* Parity gates. genotypes: out[(r*n_samples+i)*2+s] = allele index, 0xFF where the cell has no such
  * allele (second slot of a haploid cell, both slots of '.').  text: the uncompressed rows. */
 int dnaf_genotypes(dnaf_ctx* ctx, uint64_t row_begin, uint64_t row_end, uint64_t seed, uint8_t* out,
