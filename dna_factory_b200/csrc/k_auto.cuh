@@ -350,25 +350,38 @@ __device__ __forceinline__ void auto_draw_span(const AutoArgs& a, const FusedDes
         for (uint32_t q = 0; q < 2; ++q)
 #pragma unroll
             for (int w = 0; w < 4; ++w) cmp_words(philox4x32_10(g0 + w, q, r_lo, r_hi, a.k0, a.k1), thr, 4u * q, eq[w], lt[w]);
-        // residual: one (group, call) per trip, whichever group of this thread still has an undecided lane
-        uint32_t qn = 0x02020202u;   // next call index per group, one byte each
+        // residual: one call per trip on the first group of this thread that still has an undecided lane, groups in
+        // order, calls q = 2..7 in order.  That group is rotated into slot 0 (decided groups go to the back), so that
+        // no array is indexed by a runtime group number: such an index puts eq / lt in local memory.
+        uint32_t rot = 0, q = 2;   // slot 0 holds group g0 + rot; q: its next call
         for (;;) {
-            const int w = eq[0] ? 0 : (eq[1] ? 1 : (eq[2] ? 2 : (eq[3] ? 3 : 4)));
-            if (w == 4) break;
-            const uint32_t q = (qn >> (8 * w)) & 0xFFu;
-            uint32_t e = pick4(eq, w), l = pick4(lt, w);
-            cmp_words(philox4x32_10(g0 + w, q, r_lo, r_hi, a.k0, a.k1), thr, 4u * q, e, l);
-            if (q == 7u) {   // all 32 bits compared: lanes still equal have U == T, i.e. U <= T
-                l |= e;
-                e = 0;
+            if (!(eq[0] | eq[1])) {
+                uint32_t t = eq[0]; eq[0] = eq[2]; eq[2] = t; t = eq[1]; eq[1] = eq[3]; eq[3] = t;
+                t = lt[0]; lt[0] = lt[2]; lt[2] = t; t = lt[1]; lt[1] = lt[3]; lt[3] = t;
+                rot += 2; q = 2;
             }
-            qn += 1u << (8 * w);
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-                if (k == w) { eq[k] = e; lt[k] = l; }
+            if (!eq[0]) {
+                uint32_t t = eq[0]; eq[0] = eq[1]; eq[1] = eq[2]; eq[2] = eq[3]; eq[3] = t;
+                t = lt[0]; lt[0] = lt[1]; lt[1] = lt[2]; lt[2] = lt[3]; lt[3] = t;
+                rot += 1; q = 2;
+            }
+            if (!eq[0]) break;   // every group decided
+            cmp_words(philox4x32_10(g0 + rot, q, r_lo, r_hi, a.k0, a.k1), thr, 4u * q, eq[0], lt[0]);
+            if (q == 7u) {   // all 32 bits compared: lanes still equal have U == T, i.e. U <= T
+                lt[0] |= eq[0];
+                eq[0] = 0;
+            }
+            ++q;
+        }
+        // every eq is 0 now; rotate lt back by rot (mod 4)
+        if (rot & 2u) {
+            uint32_t t = lt[0]; lt[0] = lt[2]; lt[2] = t; t = lt[1]; lt[1] = lt[3]; lt[3] = t;
+        }
+        if (rot & 1u) {
+            const uint32_t t = lt[3]; lt[3] = lt[2]; lt[2] = lt[1]; lt[1] = lt[0]; lt[0] = t;
         }
 #pragma unroll
-        for (int w = 0; w < 4; ++w) m[w] = ~(lt[w] | eq[w]);   // U <= T -> reference allele
+        for (int w = 0; w < 4; ++w) m[w] = ~lt[w];   // U <= T -> reference allele
     }
     // forced-minor cells (pop_factory.py:495-499)
     if (nc > 0) {
@@ -377,19 +390,26 @@ __device__ __forceinline__ void auto_draw_span(const AutoArgs& a, const FusedDes
             if (i >= cs && i < cs + (uint32_t)nc) {
                 const uint32_t j = 2u * (i - cs);
                 const uint32_t bit = 3u << (j & 31u);
+                // selects, not m[j >> 5]: an indexed m lives in local memory for the whole kernel
 #pragma unroll
-                for (int w = 0; w < 4; ++w)
-                    if ((j >> 5) == (uint32_t)w) m[w] |= bit;
+                for (int w = 0; w < 4; ++w) m[w] |= (j >> 5) == (uint32_t)w ? bit : 0u;
             }
         }
     }
 }
 
 // CRC32 share of one span: the span-local linear CRC of its allele mask, moved to the end of the block's cells.
-__device__ __forceinline__ uint32_t auto_span_crc(const AutoArgs& a, const FusedDesc& d, const uint32_t m[4], int nc, uint32_t tid,
-                                                  uint32_t nspans) {
+// Two halves, so that a caller can issue the loads early and consume them late: _gather reads the E table and issues
+// the four lookups of the multiply table (1 MB, from L2), _finish XORs them and applies the short-last-span move.
+struct SpanCrc {
+    uint32_t t[4];   // mtab lookups of the span-local CRC's bytes; all 0 when the span has no share
+    bool tail;       // the span's share still moves across the block's short last span
+};
+
+__device__ __forceinline__ SpanCrc auto_span_crc_gather(const AutoArgs& a, const FusedDesc& d, const uint32_t m[4], int nc,
+                                                        uint32_t tid, uint32_t nspans) {
     // ---- CRC32 share of this span: template ^ delta (affine); delta's span-local CRC moved to the block end
-    uint32_t crc = 0;
+    SpanCrc c{{0u, 0u, 0u, 0u}, false};
     const bool partial_tail = (d.ncells & 63u) != 0u;   // the block's last span is short
     if (nc > 0 && (m[0] | m[1] | m[2] | m[3])) {
         uint32_t mm[4] = {m[0], m[1], m[2], m[3]};
@@ -409,16 +429,26 @@ __device__ __forceinline__ uint32_t auto_span_crc(const AutoArgs& a, const Fused
         for (int w = 0; w < 4; ++w)
 #pragma unroll
             for (int k = 0; k < 4; ++k) sp ^= __ldg(&a.etab[(4 * w + k) * 256 + ((mm[w] >> (8 * k)) & 0xFFu)]);
-        // whole spans between the end of this span's cells and the end of the block's cells, then the short last span
+        // whole spans between the end of this span's cells and the end of the block's cells (mtab + 0 multiplies by
+        // 1: the last span's share, and the one before a short last span, are sp itself), then the short last span
         const uint32_t last = nspans - 1u;
-        if (tid == last) crc = sp;                                   // ends where the cells end
-        else {
-            const uint32_t j = partial_tail ? last - 1u - tid : last - tid;
-            crc = j ? mul_tab(a.mtab + (size_t)j * 1024u, sp) : sp;
-            if (partial_tail) crc = mul_tab(a.mtail, crc);
-        }
+        const uint32_t j = tid == last ? 0u : (partial_tail ? last - 1u - tid : last - tid);
+        const uint32_t* t = a.mtab + (size_t)j * 1024u;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) c.t[k] = __ldg(&t[256 * k + ((sp >> (8 * k)) & 0xFFu)]);
+        c.tail = partial_tail && tid != last;
     }
-    return crc;
+    return c;
+}
+
+__device__ __forceinline__ uint32_t auto_span_crc_finish(const AutoArgs& a, const SpanCrc& c) {
+    const uint32_t crc = c.t[0] ^ c.t[1] ^ c.t[2] ^ c.t[3];
+    return c.tail ? mul_tab(a.mtail, crc) : crc;
+}
+
+__device__ __forceinline__ uint32_t auto_span_crc(const AutoArgs& a, const FusedDesc& d, const uint32_t m[4], int nc, uint32_t tid,
+                                                  uint32_t nspans) {
+    return auto_span_crc_finish(a, auto_span_crc_gather(a, d, m, nc, tid, nspans));
 }
 
 #ifndef DNAF_AUTO_REGS
@@ -465,12 +495,6 @@ __global__ void __maxnreg__(DNAF_AUTO_REGS) k_auto(const AutoArgs a) {
     }
     if (tid == 6) { s_misc[16] = 0; s_misc[17] = 0; }
     const bool starts_row = d.flags & 1u, ends_row = (d.flags >> 1) & 1u;
-    const uint64_t pb = a.nv.pre_off[d.row];
-    const uint32_t plen = starts_row ? (uint32_t)(a.nv.pre_off[d.row + 1] - pb) : 0u;
-    // text bytes of this block: [prefix | the separator that ended the previous segment] cells, minus the last
-    // separator unless the row ends here
-    const uint32_t lead = starts_row ? plen : 1u;
-    const uint32_t n = lead + 4u * d.ncells - (ends_row ? 0u : 1u);
     const uint32_t nspans = (d.ncells + 63u) / 64u;
 
     // ---- draw this span's 128 allele bits (replay RNG spec: dnaf_device.cuh)
@@ -479,7 +503,14 @@ __global__ void __maxnreg__(DNAF_AUTO_REGS) k_auto(const AutoArgs a) {
     if (tid < nspans) nc = (int)min(64u, d.ncells - 64u * tid);
     uint32_t m[4] = {0, 0, 0, 0};
     auto_draw_span(a, d, cs, nc, m);
-    uint32_t crc = auto_span_crc(a, d, m, nc, tid, nspans);
+    const SpanCrc crc_part = auto_span_crc_gather(a, d, m, nc, tid, nspans);
+    // the prefix is read after the draws: live across them, its offsets pushed the draw loop into spills
+    const uint64_t pb = a.nv.pre_off[d.row];
+    const uint32_t plen = starts_row ? (uint32_t)(a.nv.pre_off[d.row + 1] - pb) : 0u;
+    // text bytes of this block: [prefix | the separator that ended the previous segment] cells, minus the last
+    // separator unless the row ends here
+    const uint32_t lead = starts_row ? plen : 1u;
+    const uint32_t n = lead + 4u * d.ncells - (ends_row ? 0u : 1u);
     // prefix literal of this thread (blocks that start a row)
     uint32_t pre_tok = 0;
     if (tid < plen) pre_tok = __ldg(&tb->pre_lit[a.nv.prefix[pb + tid]]);
@@ -488,7 +519,6 @@ __global__ void __maxnreg__(DNAF_AUTO_REGS) k_auto(const AutoArgs a) {
         if (starts_row) c0 ^= mul_tab(ends_row ? a.mpre + 1024 : a.mpre, __ldg(&a.pre_crc[d.row]));
         s_misc[10] = c0;
     }
-    crc = warp_xor(crc);
 
     // ---- m' = (m << 2) | carry in shared memory, mismatch bytes
     // slots past the span's last cell repeat that cell, so that they never mismatch
@@ -507,7 +537,6 @@ __global__ void __maxnreg__(DNAF_AUTO_REGS) k_auto(const AutoArgs a) {
     s_last2[tid] = mp[3] >> 30;
     __syncthreads();        // also orders the mbarrier's initialisation before the waits
     mbar_wait(mbar, 0u);    // the code tables have landed
-    if (lane == 0 && crc) atomicXor(&s_misc[16], crc);
     const uint32_t carry = tid ? s_last2[tid - 1] : (mp[0] & 3u);
     uint32_t nz = 0;
     if (nc > 0) {
@@ -534,6 +563,10 @@ __global__ void __maxnreg__(DNAF_AUTO_REGS) k_auto(const AutoArgs a) {
         emit_span(st, s_lut, s_len, s_lits, eob, s_mp + 20u * tid, nz, mp[0], mlast_bit, tid == 0, starts_row, nc, p_end, p_last);
         if (st.bits() > 32u * kAStage) s_misc[17] = 1;
     }
+    // the CRC share is consumed only now: its mtab lookups (L2), issued before the first barrier, land under the token
+    // pass instead of holding the CTA at that barrier; XOR is order-free and the trailer reads s_misc[16] two barriers on
+    const uint32_t crc = warp_xor(auto_span_crc_finish(a, crc_part));
+    if (lane == 0 && crc) atomicXor(&s_misc[16], crc);
     // ---- exclusive scans over the CTA: prefix literal bits (warps 0-1) and span bits
     const uint32_t pre_bits = pre_tok >> 24;
     const uint32_t my_bits = worker ? st.bits() : 0u;
@@ -665,9 +698,9 @@ __global__ void __maxnreg__(DNAF_AUTO_REGS) k_auto(const AutoArgs a) {
         if (ends_row) delta = __ldg(&a.crctab[delta & 0xFFu]) ^ (delta >> 8);
         const uint32_t crc32 = ~(delta ^ s_misc[10]);
         const uint32_t bsize = out_payload + 25u;
-        if (tid < 16) {
-            const uint8_t head[16] = {0x1f, 0x8b, 0x08, 0x04, 0, 0, 0, 0, 0, 0xff, 0x06, 0x00, 0x42, 0x43, 0x02, 0x00};
-            blk[tid] = head[tid];
+        if (tid < 16) {   // 1f 8b 08 04 | 00 00 00 00 | 00 ff 06 00 | 42 43 02 00, from words (an indexed byte array is local memory)
+            const uint32_t hw = tid < 4u ? 0x04088b1fu : (tid < 8u ? 0u : (tid < 12u ? 0x0006ff00u : 0x00024342u));
+            blk[tid] = (uint8_t)(hw >> (8u * (tid & 3u)));
         } else if (tid < 18) {
             blk[tid] = (uint8_t)(bsize >> (8 * (tid - 16)));
         } else if (tid < 22) {

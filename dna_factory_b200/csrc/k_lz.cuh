@@ -297,7 +297,8 @@ __host__ __device__ inline uint32_t lz_smem_bytes(uint32_t nthr, uint32_t hbits,
            (with_chains ? (nthr / 32u) * (4u << hbits) + nthr * 256u : 0u);   // heads + prev[] come last
 }
 
-__global__ void __launch_bounds__(256) k_lz(const LzArgs la) {
+// 64 registers, as before the shared draw lost its stack frame (left free, ptxas takes 80 for the register-only draw)
+__global__ void __launch_bounds__(256, 4) k_lz(const LzArgs la) {
     const AutoArgs& a = la.a;
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const uint32_t tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31u, wid = tid >> 5;
